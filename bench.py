@@ -44,6 +44,12 @@ through b200rt_multi_render_rgb8 — the single-process entry a Rust `render_sce
 
 `--impl reference` times the reference's own CPU path (the oracle port — the Rust crate
 cannot be built in this image) on the same config with all host threads.
+
+`--dump-outputs DIR` writes what the last timed step computed, as float32 .npy files: at N = 1 the
+accumulation buffer a caller of b200rt_render_device receives (DIR/accum.npy, [H, W, 4]: RGB sums and
+the sample count), at N > 1 the RGB8 frame on rank 0 (DIR/frame.npy, [H, W, 3]).  Scene and seeds are
+fixed, so two builds run with the same arguments can be compared output for output.  An output over
+64 MiB is replaced by a fixed, seeded sample of its pixels, whose flat indices go to DIR/<name>_pixels.npy.
 """
 import argparse
 import ctypes as C
@@ -62,6 +68,7 @@ WORKLOAD = "weekend_final_scene_1200x800_500spp_depth50"
 # ncu --set full of the C4 launches (scripts/profile_c4.py; profiles/r02_c4_metrics.md): bytes per 64-spp launch
 C4_NCU = {"lts_1e6": 267870144256, "dram_1e6": 172336384, "lts_1e5": 178832932832, "dram_1e5": 110871296}
 METRIC = "Mrays/s, Weekend final scene 1200x800 500spp (ms/frame in ms_per_step)"
+DUMP_BYTES = 64 << 20          # --dump-outputs: at most this much per run
 
 
 # stdout carries exactly ONE JSON line: anything else a library prints there (NCCL's version banner,
@@ -184,6 +191,22 @@ def algorithmic_bytes_per_ray(node_visits, prim_tests, rays):
     return 64.0 * (node_visits / rays) + 16.0 * (prim_tests / rays) + 32.0
 
 
+def dump_output(out_dir, name, t, limit=DUMP_BYTES):
+    """Writes tensor t ([H, W, C] on the device) as out_dir/<name>.npy in float32; over `limit` bytes, a fixed
+    seeded sample of its pixels instead, with their flat indices in out_dir/<name>_pixels.npy (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    a = t.float().cpu().numpy()
+    if a.nbytes > limit:
+        px = a.reshape(-1, a.shape[-1])
+        n = (limit - 4096) // (px.shape[1] * 4 + 8)
+        idx = np.sort(np.random.default_rng(0).choice(len(px), n, replace=False))
+        np.save(os.path.join(out_dir, f"{name}_pixels.npy"), idx.astype(np.float64))
+        a = px[idx]
+    np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    log(f"dumped {name} {list(a.shape)} float32 to {out_dir}")
+
+
 def workload_config(W, H, spp, world, scaling):
     name = WORKLOAD if (spp == SPP and W == WIDTH and scaling == "strong") else (
         f"weekend_{W}x{H}_{spp}spp_depth{DEPTH}" if scaling == "strong" else f"weekend_{W}x{H}_{spp * world}spp_depth{DEPTH}_weak_{spp}spp_per_gpu")
@@ -243,7 +266,10 @@ def main():
                     help="--combine peer: order the ranks with flags in peer memory (default) or a one-element NCCL all_reduce")
     ap.add_argument("--combine", default="peer", choices=["peer", "nccl"],
                     help="N > 1: fused peer-memory reduce+resolve kernel over NVLink (default) or NCCL reduce then resolve on rank 0")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -411,6 +437,14 @@ def main():
     wall = time.perf_counter() - wall0
     clocks = sampler.stop()
     total_ms = float(sum(step_ms))
+    if args.dump_outputs:
+        # before the e2e leg, which renders into the same buffers at N > 1
+        if world == 1:
+            dump_output(args.dump_outputs, "accum", accum)
+        elif rank == 0:
+            dump_output(args.dump_outputs, "frame", frame_on_rank0())
+        if world > 1:
+            dist.barrier()
 
     # ---- e2e: the reference-facing call with host buffers -----------------------------------------
     rgb = np.empty((H, W, 3), dtype=np.uint8)                      # pageable, like a Rust Vec<u8>

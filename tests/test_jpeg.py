@@ -1,6 +1,7 @@
 """Host-side JPEG decoder (baseline and progressive) (shirley_raytracing_rs_b200/host/jpeg_decoder.cpp) — what
 `image::open` / `image::load_from_memory` do for the reference's image textures
 (material/texture/image_texture.rs:18-31).  Checked against PIL (libjpeg): identical bytes."""
+import hashlib
 import io
 import os
 
@@ -141,10 +142,12 @@ def test_image_path_texture_is_decoded_at_finalize(rt, tmp_path):
         b2.finalize()
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/assets/earthmap.jpg"), reason="reference asset not present on this machine")
 def test_reference_earthmap(rt):
-    """The asset the reference embeds (image_texture.rs:11): 1024x512, baseline, 4:4:4."""
-    data = open("/root/reference/assets/earthmap.jpg", "rb").read()
+    """The asset the reference embeds (image_texture.rs:11): 1024x512, baseline, 4:4:4.  The package ships the same
+    file (assets/README.md); the hashes pin it and its decoded texels to the reference's copy."""
+    data = open(os.path.join(os.path.dirname(rt.__file__), "assets", "earthmap.jpg"), "rb").read()
+    assert hashlib.sha256(data).hexdigest() == "e7c5a0062719708d0943dcc13bb48af677c46de8686e3940062f6a70285695d4"
     got = rt.decode_jpeg(data)
     assert got.shape == (512, 1024, 3)
+    assert hashlib.sha256(got.tobytes()).hexdigest() == "a8cdc92a168d554ddc693785d31f5e251063724f44099571d7fbce3b43d44c45"
     assert np.array_equal(got, _pil_decode(data))
