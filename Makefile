@@ -6,10 +6,6 @@ NVCC      ?= nvcc
 HOSTCXX   ?= /usr/bin/g++
 ARCH      := -gencode arch=compute_100a,code=sm_100a
 NVFLAGS   := $(ARCH) -O3 -std=c++17 -lineinfo -Xcompiler -fPIC,-fopenmp -Xptxas -v --expt-relaxed-constexpr $(EXTRA_NVFLAGS)
-# make DEV=1: compile only the default render-kernel variant (fast iteration)
-ifdef DEV
-NVFLAGS   += -DB200RT_DEV_BUILD
-endif
 CXXFLAGS  := -O2 -std=c++17 -fPIC -Wall -Wno-unused-function
 PKG       := shirley_raytracing_rs_b200
 CSRC      := $(PKG)/csrc
@@ -30,15 +26,15 @@ cli: ray-cli
 ray-cli: $(PKG)/cli/ray_cli.cpp $(LIB) $(HOST_HDRS)
 	$(HOSTCXX) $(CXXFLAGS) -o $@ $< -L$(PKG) -lb200rt -Wl,-rpath,'$$ORIGIN/$(PKG)'
 
-# The build mode (full / DEV) is recorded in build/.mode, rewritten only when it changes, and is a prerequisite of
-# the CUDA object: switching between `make DEV=1` and `make` always recompiles, so a stale DEV library never ships.
-MODE := $(if $(DEV),dev,full) $(EXTRA_NVFLAGS)
+# EXTRA_NVFLAGS is recorded in build/.mode, rewritten only when it changes, and is a prerequisite of the CUDA
+# object: changing the flags always recompiles, so a library built with other flags never ships.
+MODE := nvflags: $(EXTRA_NVFLAGS)
 build/.mode: FORCE
 	@mkdir -p build
 	@if [ "$$(cat $@ 2>/dev/null)" != "$(MODE)" ]; then echo "$(MODE)" > $@; fi
 FORCE:
 
-build/b200rt.o: build/.mode $(CSRC)/b200rt.cu $(wildcard $(CSRC)/*.cuh) $(CSRC)/bvh_build.hpp include/b200rt.h
+build/b200rt.o: build/.mode $(CSRC)/b200rt.cu $(wildcard $(CSRC)/*.cuh) $(CSRC)/bvh_build.hpp $(CSRC)/launch_plan.hpp include/b200rt.h
 	@mkdir -p build
 	$(NVCC) $(NVFLAGS) -c $(CSRC)/b200rt.cu -o $@ 2> build/ptxas_b200rt.log || (cat build/ptxas_b200rt.log; false)
 	@grep -E "error|warning: .*spill|bytes spill" build/ptxas_b200rt.log | grep -v "0 bytes spill" | head -20 || true

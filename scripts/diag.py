@@ -9,12 +9,7 @@ rt.render(scene, cam, samples=8, seed=1)
 _, st0 = rt.render(scene, cam, samples=spp, seed=1)
 acc, st = rt.render(scene, cam, samples=spp, seed=1, count_traversal=True)
 d = list(st.diag)
-kv = os.environ.get("B200RT_KERNEL", "2")
 envs = {k: v for k, v in os.environ.items() if k.startswith("B200RT_")}
 print(f"{envs}  kernel {st0.kernel_ms:.1f} ms -> {st0.rays / st0.kernel_ms / 1e3:.0f} Mrays/s  rays {st.rays} paths {st.paths}")
-if kv == "3":
-    print(f"   policy iterations {d[0]}  shade batches {d[1]} lanes/shade batch {d[5]/max(d[1],1):.2f} kinds/batch {d[2]/max(d[1],1):.2f}  fetch batches {d[7]} lanes/fetch {st.rays/max(d[7],1):.2f}")
-    print(f"   inner warp-steps {d[3]}  lanes per inner warp-step {d[4]/max(d[3],1):.2f}  node visits/ray {st.node_visits/st.rays:.2f} prim tests/ray {st.prim_tests/st.rays:.2f}")
-else:
-    print(f"   outer iterations {d[0]}  alive lanes/iter {d[1]/max(d[0],1):.2f}  out-of-work lanes/iter {d[2]/max(d[0],1):.2f}  regenerated/iter {d[6]/max(d[0],1):.2f}  shaded/iter {d[5]/max(d[0],1):.2f}")
-    print(f"   traversal rounds {d[3]}  traversing lanes/round {d[4]/max(d[3],1):.2f}  inner warp-steps {d[7]}  lanes per inner warp-step {st.node_visits/max(d[7],1):.2f}")
+print(f"   outer iterations {d[0]}  alive lanes/iter {d[1]/max(d[0],1):.2f}  out-of-work lanes/iter {d[2]/max(d[0],1):.2f}  regenerated/iter {d[6]/max(d[0],1):.2f}  shaded/iter {d[5]/max(d[0],1):.2f}")
+print(f"   traversal rounds {d[3]}  traversing lanes/round {d[4]/max(d[3],1):.2f}  inner warp-steps {d[7]}  lanes per inner warp-step {st.node_visits/max(d[7],1):.2f}")

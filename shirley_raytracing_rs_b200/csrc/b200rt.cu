@@ -8,6 +8,7 @@
 //                        K4 scatter / camera_rays / texture_value / aabb_hit / rng parity hooks, FFMA-chain microbenchmark
 //   lbvh.cuh             K5 linear BVH built on the device                         (bvh/bbox_tree/constructor.rs:9-212)
 //   bvh_build.hpp        host binned-SAH builder
+//   launch_plan.hpp      CTA size, shared-memory plan, sample-range schedule and grid of a launch (pure host arithmetic)
 // No tensor cores: nothing on this path is a dense contraction.  No CPU fallback.
 #include <cuda_runtime.h>
 
@@ -26,6 +27,7 @@
 #include <vector>
 
 #include "bvh_build.hpp"
+#include "launch_plan.hpp"
 #include "lbvh.cuh"
 #include "rt_device.cuh"
 
@@ -67,9 +69,9 @@ struct Scratch {                     // per in-flight render: counters, events, 
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev2 = nullptr, ev3 = nullptr;
     cudaStream_t own_stream = nullptr;
     cudaStream_t launch_stream = nullptr; bool launched = false;   // where the render in flight was enqueued (scene_destroy waits for it)
-    float4* d_accum = nullptr; size_t accum_px = 0;
+    float4* d_accum = nullptr; size_t accum_bytes = 0;
     uint8_t* d_rgb = nullptr; size_t rgb_bytes = 0;
-    long long* d_fix = nullptr; size_t fix_px = 0;     // fixed-point sums of a launch whose tiles are split into sample chunks
+    long long* d_fix = nullptr; size_t fix_bytes = 0;  // fixed-point sums of a launch whose tiles are split into sample chunks
     uint32_t launches = 0;
 };
 
@@ -96,8 +98,8 @@ struct B200rtScene {
     size_t smem_optin = 0;
     DeviceScene ds{};
     B200rtSceneInfo info{};
-    std::vector<void*> allocs;
-    size_t arena_bytes = 0;       // capacity of allocs[0] (may exceed what this scene uses: pooled arenas are reused)
+    void* arena = nullptr;        // the one device allocation that holds every scene array
+    size_t arena_bytes = 0;       // its capacity (may exceed what this scene uses: pooled arenas are reused)
     std::mutex mu;
     std::map<void*, Scratch*> inflight;   // keyed by stream
     float box_pad = 0.f;          // how far every BVH box was grown
@@ -111,6 +113,34 @@ struct DeviceGuard {
     explicit DeviceGuard(int dev) { if (cudaGetDevice(&prev) == cudaSuccess && cudaSetDevice(dev) == cudaSuccess) ok = true; }
     ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
+
+struct DevBuf {   // RAII device buffer for one call
+    void* p = nullptr;
+    ~DevBuf() { if (p) cudaFree(p); }
+    int alloc(size_t bytes) { CU(cudaMalloc(&p, bytes ? bytes : 16)); return B200RT_OK; }
+    template <class T> T* as() { return reinterpret_cast<T*>(p); }
+};
+
+// Buffers kept across calls only grow: when `cap` bytes are too few the old buffer is freed and `bytes` allocated
+// (on failure p is null and cap 0).
+template <class T> cudaError_t grow(T*& p, size_t& cap, size_t bytes) {
+    if (cap >= bytes) return cudaSuccess;
+    cudaFree(p); p = nullptr; cap = 0;
+    cudaError_t e = cudaMalloc(&p, bytes);
+    if (e == cudaSuccess) cap = bytes;
+    return e;
+}
+
+// an integer knob from the environment (README.md lists them); unset or empty: the default, the measured best
+int env_int(const char* name, int dflt) { const char* v = getenv(name); return v && *v ? atoi(v) : dflt; }
+
+SceneSize scene_size(const B200rtScene* sc) { return {sc->ds.n_nodes, sc->ds.n_prims, sc->ds.n_tex, sc->ds.bvh_depth}; }
+
+// The centre-form (one-FMA) slab planes are conservative only while |origin| * eps stays below the box padding;
+// `max_origin` is the largest |coordinate| of a ray origin.  B200RT_FAST_SLAB=0 forces the exact Aabb::hit2 arithmetic.
+bool use_fast_slab(const B200rtScene* sc, float max_origin) {
+    return sc->box_pad >= 4.0f * 1.1920929e-7f * std::max(sc->max_abs_coord, max_origin) && env_int("B200RT_FAST_SLAB", 1) != 0;
+}
 
 int resolve_device(int device, int* out) {
     int n = 0;
@@ -169,30 +199,6 @@ int validate(const B200rtSceneDesc* d) {
         if (!d->images[i].rgb8 || d->images[i].width == 0 || d->images[i].height == 0) return fail(B200RT_EINVAL, "image %u: empty", i);
     if (d->skybox.kind > B200RT_SKY_NONE) return fail(B200RT_EINVAL, "bad skybox kind %u", d->skybox.kind);
     return B200RT_OK;
-}
-
-// shared-memory budget: stage the whole scene when it fits, else nothing (the L1 cache does better)
-SmemPlan make_plan(const B200rtScene* sc, uint32_t blocks_per_sm_target, uint32_t block_threads = BLOCK, size_t extra_bytes = 0) {
-    SmemPlan p{};
-    const DeviceScene& s = sc->ds;
-    size_t budget = sc->smem_optin / blocks_per_sm_target;
-    if (budget > sc->smem_optin) budget = sc->smem_optin;
-    budget = budget > 2048 ? budget - 1024 : budget;   // per-CTA reserved shared memory
-    p.stack_depth = s.bvh_depth + 3;   // + the sentinel entry of the v2 kernel
-    // per-thread stack columns + whatever else the kernel keeps per CTA (v3: the path pools)
-    size_t stack_bytes = (size_t)p.stack_depth * block_threads * sizeof(int) + extra_bytes;
-    size_t scene_bytes = (size_t)s.n_nodes * (16 * SMEM_NODE_QUADS) + (size_t)s.n_prims * 64 + (size_t)s.n_tex * 32;
-    if (scene_bytes + stack_bytes <= budget) {
-        p.all_in_smem = 1; p.n_top = s.n_nodes;
-        p.bytes = (uint32_t)(scene_bytes + stack_bytes);
-    } else {
-        // Scenes that do not fit: nothing is staged, every array is read through __ldg and the shared memory
-        // left over is L1 cache (a staged prefix of the tree was measured slower — rt_device.cuh: GmemAcc).
-        p.all_in_smem = 0;
-        p.n_top = 0;
-        p.bytes = (uint32_t)stack_bytes;
-    }
-    return p;
 }
 
 DeviceCamera make_camera(const B200rtCamera& c) {
@@ -260,6 +266,27 @@ template <class K> int set_smem(K kernel, const B200rtScene* sc, uint32_t bytes)
     return B200RT_OK;
 }
 
+// The shipped instantiations: {fast, fast + counters, exact + counters} per accessor (and CTA size).  The exact-slab fallback
+// always counts: it is the rare path and one variant fewer to compile.  A combination without a kernel is an error.
+using RenderKernel = void (*)(RenderArgs);
+using HitKernel = void (*)(HitArgs);
+template <class Acc, int BLK> RenderKernel render_variant(bool fast, bool count) {
+    return !fast ? path_trace_kernel_v2<Acc, true, false, BLK> : count ? path_trace_kernel_v2<Acc, true, true, BLK> : path_trace_kernel_v2<Acc, false, true, BLK>;
+}
+RenderKernel render_kernel(bool all_in_smem, uint32_t block_threads, bool fast, bool count) {
+    if (all_in_smem) return block_threads == 768 ? render_variant<SmemAcc, 768>(fast, count) : nullptr;
+    switch (block_threads) {
+        case 256: return render_variant<GmemAcc, 256>(fast, count);
+        case 512: return render_variant<GmemAcc, 512>(fast, count);
+        case 768: return render_variant<GmemAcc, 768>(fast, count);
+        default: return nullptr;
+    }
+}
+template <class Acc> HitKernel hit_variant(bool fast, bool count) {
+    return !fast ? closest_hit_kernel<Acc, true, false> : count ? closest_hit_kernel<Acc, true, true> : closest_hit_kernel<Acc, false, true>;
+}
+HitKernel hit_kernel(bool all_in_smem, bool fast, bool count) { return all_in_smem ? hit_variant<SmemAcc>(fast, count) : hit_variant<GmemAcc>(fast, count); }
+
 int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderParams* prm, float* d_accum, cudaStream_t stream, Scratch* scr) {
     if (cam->image_width == 0 || cam->image_height == 0) return fail(B200RT_EINVAL, "camera image dimensions are zero");
     if ((uint64_t)cam->image_width * cam->image_height > 0xFFFFFFFFull) return fail(B200RT_EINVAL, "image too large");
@@ -285,41 +312,15 @@ int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderPa
     a.accum = reinterpret_cast<float4*>(d_accum);
     a.counters = scr->d_counters;
     bool count = (prm->flags & B200RT_FLAG_COUNT_TRAVERSAL) != 0;
-
-    // Tunables (defaults are the measured best; env vars exist for A/B runs under ncu):
-    //   B200RT_BLOCK=256|512|768   B200RT_TRAV_THRESHOLD=1..32   B200RT_REGEN_MIN=1..32   B200RT_FAST_SLAB=0|1
-    auto env_int = [](const char* name, int dflt) { const char* v = getenv(name); return v && *v ? atoi(v) : dflt; };
-    int block_threads = env_int("B200RT_BLOCK", 768);
-    if (block_threads != 256 && block_threads != 512 && block_threads != 768) block_threads = 768;
-#ifdef B200RT_DEV_BUILD
-#ifndef B200RT_DEV_BLK
-#define B200RT_DEV_BLK 768
-#endif
-    block_threads = B200RT_DEV_BLK;      // `make DEV=1 [EXTRA_NVFLAGS=-DB200RT_DEV_BLK=640]`: the one CTA size compiled
-#endif
     a.trav_threshold = (uint32_t)std::min(32, std::max(1, env_int("B200RT_TRAV_THRESHOLD", 8)));
     // New paths are handed out only when >= 6 lanes are free (the hand-out block then runs at >= 6 lanes instead of ~5 every
     // iteration): 14.66 -> 15.0 Grays/s on the bench frame, +5 % on the earth frame, 4..8 within 0.5 % of each other.
     a.regen_min = (uint32_t)std::min(32, std::max(1, env_int("B200RT_REGEN_MIN", 6)));
-    // the centre-form slab planes are conservative only while |origin| * eps stays below the box padding
-    float max_origin = std::max(sc->max_abs_coord, std::max(std::fabs((float)cam->origin[0]), std::max(std::fabs((float)cam->origin[1]), std::fabs((float)cam->origin[2]))));
-    bool fast_ok = sc->box_pad >= 4.0f * 1.1920929e-7f * max_origin;
-    bool fast = fast_ok && env_int("B200RT_FAST_SLAB", 1) != 0;
-
-    // per warp: the fixed-point tile sums and the primary-ray ring; per thread: 7 words of path state (attenuation, emitted, pixel)
-    auto extra_for = [](int threads) { return (size_t)(threads / 32) * (96 * sizeof(long long) + RAYQ_FIELDS * RAYQ_SLOTS * sizeof(uint32_t)) + (size_t)threads * 7 * sizeof(float); };
-    SmemPlan plan = make_plan(sc, 1, block_threads, extra_for(block_threads));
-#ifndef B200RT_DEV_BUILD
-    // A deep tree (the device-built linear BVH can reach 40-50 levels) needs more stack per thread than
-    // 768 threads leave room for: fall back to smaller CTAs rather than fail.  (Only scenes that live in
-    // global memory get that deep; a scene that fits in shared memory always runs 768-thread CTAs.)
-    if (plan.all_in_smem) block_threads = 768, plan = make_plan(sc, 1, 768, extra_for(768));
-    while (!plan.all_in_smem && plan.bytes + 1024 > sc->smem_optin && block_threads > 256) {
-        block_threads = block_threads > 512 ? 512 : 256;
-        plan = make_plan(sc, 1, block_threads, extra_for(block_threads));
-    }
-#endif
+    const bool fast = use_fast_slab(sc, std::max(std::fabs((float)cam->origin[0]), std::max(std::fabs((float)cam->origin[1]), std::fabs((float)cam->origin[2]))));
+    const auto [block_threads, plan] = render_shape(scene_size(sc), sc->smem_optin);
     a.plan = plan;
+    RenderKernel kernel = render_kernel(plan.all_in_smem, block_threads, fast, count);
+    if (!kernel) return fail(B200RT_ECUDA, "no path-tracing kernel is built for %u-thread CTAs with the scene %s", block_threads, plan.all_in_smem ? "in shared memory" : "read through L1");
 
     scr->launches = 0;
     scr->launch_stream = stream; scr->launched = true;
@@ -329,104 +330,36 @@ int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderPa
     // ("pixels outside the selected rows/tiles are written as zeros", include/b200rt.h).
     const bool covers_frame = a.shard_count == 1 && a.row_begin == 0 && a.row_end == H;
     if (!a.accumulate && !covers_frame) CU(cudaMemsetAsync(d_accum, 0, (size_t)W * H * sizeof(float4), stream));
+    int rc = set_smem(kernel, sc, plan.bytes); if (rc) return rc;
     int blocks_per_sm = 0;
-    auto go = [&](auto kernel) -> int {
-        int rc = set_smem(kernel, sc, plan.bytes); if (rc) return rc;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kernel, block_threads, plan.bytes));
-        if (blocks_per_sm < 1) return fail(B200RT_ECUDA, "path-tracing kernel does not fit on an SM (smem %u B, %d threads)", plan.bytes, block_threads);
-        const uint32_t warps_per_block = (uint32_t)block_threads / 32;
-        const uint32_t my_tiles = a.n_tiles > a.shard_index ? (a.n_tiles - a.shard_index + a.shard_count - 1) / a.shard_count : 0u;   // tiles t with t % shard_count == shard_index
-        const uint32_t full_grid = (uint32_t)(sc->sm_count * blocks_per_sm);
-        // Work granularity (profiles/r02_experiments.md §2, §9, §17).  A tile's samples are split into sample ranges that SHRINK:
-        // the launch ends when the last item ends, so the last items must be small (a whole-tile item of the 1200x800 frame is
-        // ~1 ms: 5 % of a 63-spp launch, which is what one of 8 GPUs renders), while big items are cheaper per sample (a warp
-        // drains once per item).  Guided schedule: each range takes 70 % of what is left — at most `cap` samples, 7 % of a warp's
-        // share of the launch, so that frames with few tiles per warp (tile shards, small images) still balance — until the rest is
-        // below ~1.5x the target size of the last range, 0.2 % of a warp's share of the launch (2 % for scenes read through L1,
-        // where every extra item costs L1 locality and atomics: whole tiles on the config-4 frames).  Items are handed out
-        // range by range, bottom rows first within each.  Measured against uniform ranges: +2.9 % at 500 spp, +5.8 % at 63 spp,
-        // +4.7 % at 16 spp on the bench frame.  B200RT_CHUNKS=n forces n ranges (geometric, last / first = B200RT_TAPER %).
-        const uint32_t S = a.samples;
-        const double tiles_per_warp = (double)my_tiles / ((double)full_grid * warps_per_block);
-        const double share = std::max((double)S * tiles_per_warp, 1e-9);                  // samples x tiles a resident warp renders
-        const double last_target = std::max(1.0, (plan.all_in_smem ? 0.002 : 0.02) * share);
-        // no item above ~7 % of a warp's share (a heavy tile costs ~3x the average one) — but not below 8 samples (256 paths) either
-        // when that share is small (tiny frames): an item drains the warp once whatever its size
-        const double cap = std::max(std::max(1.0, 0.07 * share), std::min(8.0, 0.5 * share));
-        uint32_t sizes[MAX_CHUNKS]; uint32_t C = 0;
-        const int forced = env_int("B200RT_CHUNKS", 0);
-        if (forced > 0) {
-            C = (uint32_t)std::min<int64_t>(std::min<int64_t>(forced, MAX_CHUNKS), S);
-            const double w = std::min(100, std::max(1, std::abs(env_int("B200RT_TAPER", 3)))) / 100.0;
-            const double r = C > 1 ? std::pow(w, 1.0 / (C - 1)) : 1.0;
-            uint32_t prev = 0;
-            for (uint32_t k = 1; k <= C; ++k) {
-                const double F = r < 0.999999 ? (1.0 - std::pow(r, (double)k)) / (1.0 - std::pow(r, (double)C)) : (double)k / C;
-                uint32_t b = k == C ? S : (uint32_t)std::llround(F * S);
-                b = std::min(std::max(b, prev + 1u), S - (C - k));            // every range non-empty
-                sizes[k - 1] = b - prev; prev = b;
-            }
-        } else {
-            uint32_t rem = S;
-            double cap_now = cap;
-            while (rem > 0) {
-                uint32_t s = (uint32_t)std::llround(std::min(cap_now, 0.7 * rem));
-                s = std::min(std::max(s, 1u), rem);
-                if (rem <= (uint32_t)std::ceil(1.5 * last_target) || C + 1 == MAX_CHUNKS) s = (C + 1 == MAX_CHUNKS || rem <= cap_now * 1.5) ? rem : s;
-                sizes[C++] = s; rem -= s;
-                if (C + 8 >= MAX_CHUNKS) cap_now = std::max(cap_now, (double)rem / 6.0);      // running out of table entries: bigger ranges
-            }
-        }
-        if (C == 0) { sizes[0] = S; C = 1; }
-        if ((uint64_t)my_tiles * C > 0xFFFFFFF0ull) { sizes[0] = S; C = 1; }      // the 32-bit work counter
-        a.chunks = C;
-        a.my_tiles = my_tiles ? my_tiles : 1u;
-        a.chunk_begin[0] = 0;
-        for (uint32_t k = 0; k < MAX_CHUNKS; ++k) a.chunk_begin[k + 1] = k < C ? a.chunk_begin[k] + sizes[k] : S;
-        a.fix = nullptr;
-        if (a.chunks > 1u) {
-            const size_t px = (size_t)W * H;
-            if (scr->fix_px < px) {
-                cudaFree(scr->d_fix); scr->d_fix = nullptr; scr->fix_px = 0;
-                cudaError_t e = cudaMalloc(&scr->d_fix, px * 3 * sizeof(long long));
-                if (e != cudaSuccess) return fail(B200RT_ENOMEM, "fixed-point accumulation buffer (%zu px): %s", px, cudaGetErrorString(e));
-                scr->fix_px = px;
-            }
-            a.fix = scr->d_fix;
-            CU(cudaMemsetAsync(scr->d_fix, 0, px * 3 * sizeof(long long), stream));
-        }
-        const uint64_t warps_needed = (uint64_t)my_tiles * a.chunks;
-        uint32_t grid = full_grid;
-        const uint64_t grid_needed = (warps_needed + warps_per_block - 1) / warps_per_block;
-        if (grid_needed < grid) grid = grid_needed ? (uint32_t)grid_needed : 1;
-        CU(cudaEventRecord(scr->ev1, stream));
-        kernel<<<grid, block_threads, plan.bytes, stream>>>(a);
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kernel, block_threads, plan.bytes));
+    if (blocks_per_sm < 1) return fail(B200RT_ECUDA, "path-tracing kernel does not fit on an SM (smem %u B, %u threads)", plan.bytes, block_threads);
+    const uint32_t warps_per_block = block_threads / 32;
+    const uint32_t my_tiles = a.n_tiles > a.shard_index ? (a.n_tiles - a.shard_index + a.shard_count - 1) / a.shard_count : 0u;   // tiles t with t % shard_count == shard_index
+    const uint32_t full_grid = (uint32_t)(sc->sm_count * blocks_per_sm);
+    const SampleSchedule sched = sample_schedule(a.samples, my_tiles, full_grid * warps_per_block, plan.all_in_smem, env_int("B200RT_CHUNKS", 0));
+    a.chunks = sched.chunks;
+    a.my_tiles = my_tiles ? my_tiles : 1u;
+    std::copy(sched.chunk_begin, sched.chunk_begin + MAX_CHUNKS + 1, a.chunk_begin);
+    a.fix = nullptr;
+    if (a.chunks > 1u) {
+        const size_t px = (size_t)W * H;
+        cudaError_t e = grow(scr->d_fix, scr->fix_bytes, px * 3 * sizeof(long long));
+        if (e != cudaSuccess) return fail(B200RT_ENOMEM, "fixed-point accumulation buffer (%zu px): %s", px, cudaGetErrorString(e));
+        a.fix = scr->d_fix;
+        CU(cudaMemsetAsync(scr->d_fix, 0, px * 3 * sizeof(long long), stream));
+    }
+    CU(cudaEventRecord(scr->ev1, stream));
+    kernel<<<render_grid(full_grid, my_tiles, a.chunks, warps_per_block), block_threads, plan.bytes, stream>>>(a);
+    CU(cudaGetLastError());
+    scr->launches += 1;
+    if (a.chunks > 1u && a.row_end > a.row_begin) {
+        dim3 fb(128, 1), fg((W + 127) / 128, a.row_end - a.row_begin);
+        finalize_kernel<<<fg, fb, 0, stream>>>(a);
         CU(cudaGetLastError());
         scr->launches += 1;
-        if (a.chunks > 1u && a.row_end > a.row_begin) {
-            dim3 fb(128, 1), fg((W + 127) / 128, a.row_end - a.row_begin);
-            finalize_kernel<<<fg, fb, 0, stream>>>(a);
-            CU(cudaGetLastError());
-            scr->launches += 1;
-        }
-        CU(cudaEventRecord(scr->ev2, stream));
-        return B200RT_OK;
-    };
-    int rc;
-    // Instantiations shipped: {fast, fast + counters, exact + counters} per accessor and CTA size (the exact-slab
-    // fallback always counts: it is the rare path and one variant fewer to compile).
-#ifdef B200RT_DEV_BUILD
-#define B200RT_GO(ACC, CNT, FST) go(path_trace_kernel_v2<ACC, CNT, FST, B200RT_DEV_BLK, 1>)
-    if (plan.all_in_smem) rc = !fast ? B200RT_GO(SmemAcc, true, false) : (count ? B200RT_GO(SmemAcc, true, true) : B200RT_GO(SmemAcc, false, true));
-    else rc = !fast ? B200RT_GO(GmemAcc, true, false) : (count ? B200RT_GO(GmemAcc, true, true) : B200RT_GO(GmemAcc, false, true));
-#undef B200RT_GO
-#else
-#define B200RT_GO(ACC, BLK) (!fast ? go(path_trace_kernel_v2<ACC, true, false, BLK, 1>) : (count ? go(path_trace_kernel_v2<ACC, true, true, BLK, 1>) : go(path_trace_kernel_v2<ACC, false, true, BLK, 1>)))
-    if (plan.all_in_smem) rc = B200RT_GO(SmemAcc, 768);
-    else rc = block_threads == 256 ? B200RT_GO(GmemAcc, 256) : (block_threads == 512 ? B200RT_GO(GmemAcc, 512) : B200RT_GO(GmemAcc, 768));
-#undef B200RT_GO
-#endif
-    if (rc) return rc;
+    }
+    CU(cudaEventRecord(scr->ev2, stream));
     CU(cudaMemcpyAsync(scr->h_counters, scr->d_counters, sizeof(Counters), cudaMemcpyDeviceToHost, stream));
     return B200RT_OK;
 }
@@ -665,7 +598,7 @@ int b200rt_scene_create(const B200rtSceneDesc* d, int device, B200rtScene** out)
         cudaError_t e = cudaSuccess;
         if (!dbase) { e = cudaMalloc(&dbase, arena.total); capacity = arena.total; }
         if (e != cudaSuccess) return bail(fail(B200RT_ENOMEM, "scene arena (%zu B): %s", arena.total, cudaGetErrorString(e)));
-        sc->allocs.push_back(dbase); sc->arena_bytes = capacity;
+        sc->arena = dbase; sc->arena_bytes = capacity;
         for (uint32_t i = 0; i < d->n_images; ++i) images[i].texels = reinterpret_cast<const uchar4*>(dbase + off_img[i]);
         e = arena.upload(dbase);
         if (e != cudaSuccess) return bail(fail(B200RT_ECUDA, "scene upload: %s", cudaGetErrorString(e)));
@@ -713,9 +646,7 @@ int b200rt_scene_create(const B200rtSceneDesc* d, int device, B200rtScene** out)
     bool flat = d->skybox.kind == B200RT_SKY_FLAT;
     sc->ds.sky_r = flat ? d->skybox.rgb[0] : 0.f; sc->ds.sky_g = flat ? d->skybox.rgb[1] : 0.f; sc->ds.sky_b = flat ? d->skybox.rgb[2] : 0.f;
     sc->info.n_prims = d->n_prims; sc->info.n_bvh_nodes = sc->ds.n_nodes; sc->info.bvh_depth = bvh.depth;
-    SmemPlan plan = make_plan(sc, 2);
-    if (!plan.all_in_smem) { SmemPlan p1 = make_plan(sc, 1); if (p1.all_in_smem) plan = p1; }
-    sc->info.bvh_nodes_in_smem = plan.n_top;
+    sc->info.bvh_nodes_in_smem = hook_plan(scene_size(sc), sc->smem_optin).n_top;
     *out = sc;
     return B200RT_OK;
 }
@@ -732,14 +663,14 @@ void b200rt_scene_destroy(B200rtScene* sc) {
             g_scratch_pool[sc->device].push_back(kv.second);
         }
     }
-    if (!sc->allocs.empty()) {   // one arena holds every scene array: back to the pool (every render on it has been waited for above)
+    if (sc->arena) {   // one arena holds every scene array: back to the pool (every render on it has been waited for above)
         bool pooled = false;
         {
             std::lock_guard<std::mutex> gl(g_scratch_mu);
             auto& pool = g_arena_pool[sc->device];
-            if (pool.size() < ARENA_POOL_MAX) { pool.push_back({sc->allocs[0], sc->arena_bytes}); pooled = true; }
+            if (pool.size() < ARENA_POOL_MAX) { pool.push_back({sc->arena, sc->arena_bytes}); pooled = true; }
         }
-        if (!pooled) cudaFree(sc->allocs[0]);
+        if (!pooled) cudaFree(sc->arena);
     }
     delete sc;
 }
@@ -781,17 +712,10 @@ static int render_host_impl(const B200rtScene* csc, const B200rtCamera* cam, con
     Scratch* scr; int rc = get_scratch(sc, key, &scr); if (rc) return rc;
     size_t px = (size_t)cam->image_width * cam->image_height;
     auto done = [&](int code) { put_scratch(sc, key); return code; };
-    if (scr->accum_px < px) {
-        cudaFree(scr->d_accum); scr->d_accum = nullptr; scr->accum_px = 0;
-        cudaError_t e = cudaMalloc(&scr->d_accum, px * sizeof(float4));
-        if (e != cudaSuccess) return done(fail(B200RT_ENOMEM, "accumulation buffer (%zu px): %s", px, cudaGetErrorString(e)));
-        scr->accum_px = px;
-    }
-    if (out_rgb8 && scr->rgb_bytes < px * 3) {
-        cudaFree(scr->d_rgb); scr->d_rgb = nullptr; scr->rgb_bytes = 0;
-        cudaError_t e = cudaMalloc(&scr->d_rgb, px * 3);
-        if (e != cudaSuccess) return done(fail(B200RT_ENOMEM, "rgb8 buffer: %s", cudaGetErrorString(e)));
-        scr->rgb_bytes = px * 3;
+    if (cudaError_t e = grow(scr->d_accum, scr->accum_bytes, px * sizeof(float4)))
+        return done(fail(B200RT_ENOMEM, "accumulation buffer (%zu px): %s", px, cudaGetErrorString(e)));
+    if (out_rgb8) {
+        if (cudaError_t e = grow(scr->d_rgb, scr->rgb_bytes, px * 3)) return done(fail(B200RT_ENOMEM, "rgb8 buffer: %s", cudaGetErrorString(e)));
     }
     // Progressive rendering with host buffers: with B200RT_FLAG_ACCUMULATE the caller's float4 sums
     // (an earlier call's output, or a checkpoint) are uploaded first and the new samples are added.
@@ -842,7 +766,7 @@ struct B200rtMulti {
     struct Dev {
         int id = 0;
         cudaStream_t stream = nullptr; cudaEvent_t done = nullptr;
-        float* accum = nullptr; size_t accum_px = 0;
+        float* accum = nullptr; size_t accum_bytes = 0;
         B200rtScene* scene = nullptr;
         int rc = 0; std::string err; bool ran = false;
         std::thread th;
@@ -868,11 +792,8 @@ void multi_device_job(B200rtMulti* m, uint32_t k) {
     const uint32_t total = m->prm->samples == 0 ? 1 : m->prm->samples;   // src/main.rs:75-80
     const size_t px = (size_t)m->cam->image_width * m->cam->image_height;
     if (int rc = b200rt_scene_create(m->desc, d.id, &d.scene)) return bad(rc);
-    if (d.accum_px < px) {
-        cudaFree(d.accum); d.accum = nullptr; d.accum_px = 0;
-        cudaError_t e = cudaMalloc(&d.accum, px * sizeof(float4));
-        if (e != cudaSuccess) { fail(B200RT_ENOMEM, "device %d: accumulation buffer: %s", d.id, cudaGetErrorString(e)); return bad(B200RT_ENOMEM); }
-        d.accum_px = px;
+    if (cudaError_t e = grow(d.accum, d.accum_bytes, px * sizeof(float4))) {
+        fail(B200RT_ENOMEM, "device %d: accumulation buffer: %s", d.id, cudaGetErrorString(e)); return bad(B200RT_ENOMEM);
     }
     B200rtRenderParams p = *m->prm;
     const uint32_t s0 = (uint32_t)((uint64_t)total * k / n), s1 = (uint32_t)((uint64_t)total * (k + 1) / n);
@@ -981,10 +902,7 @@ int b200rt_multi_render_rgb8(B200rtMulti* m, const B200rtSceneDesc* desc, const 
     // phase 2 on the first device: stream-ordered wait for everyone, fused sum + resolve over peer access, frame copy-back
     B200rtMulti::Dev& d0 = m->dv[0];
     if (rc == B200RT_OK && cudaSetDevice(d0.id) != cudaSuccess) rc = fail(B200RT_ECUDA, "cudaSetDevice(%d) failed", d0.id);
-    if (rc == B200RT_OK && m->rgb_bytes < px * 3) {
-        cudaFree(m->d_rgb); m->d_rgb = nullptr; m->rgb_bytes = 0;
-        if (cudaMalloc(&m->d_rgb, px * 3) != cudaSuccess) rc = fail(B200RT_ENOMEM, "rgb8 buffer"); else m->rgb_bytes = px * 3;
-    }
+    if (rc == B200RT_OK && grow(m->d_rgb, m->rgb_bytes, px * 3) != cudaSuccess) rc = fail(B200RT_ENOMEM, "rgb8 buffer");
     if (rc == B200RT_OK) {
         const float* ptrs[MAX_PEERS];
         for (uint32_t k = 0; k < n; ++k) {
@@ -1142,15 +1060,11 @@ int b200rt_resolve_rgb8(const float* accum, uint32_t W, uint32_t H, uint32_t sam
     int rc = resolve_device(device, &device); if (rc) return rc;
     DeviceGuard guard(device);
     size_t px = (size_t)W * H;
-    float* d_acc = nullptr; uint8_t* d_out = nullptr;
-    CU(cudaMalloc(&d_acc, px * 16));
-    cudaError_t e = cudaMalloc(&d_out, px * 3);
-    if (e != cudaSuccess) { cudaFree(d_acc); return fail(B200RT_ENOMEM, "resolve buffers: %s", cudaGetErrorString(e)); }
-    auto cleanup = [&]() { cudaFree(d_acc); cudaFree(d_out); };
-    e = cudaMemcpy(d_acc, accum, px * 16, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) { rc = b200rt_resolve_rgb8_device(d_acc, W, H, samples, d_out, nullptr); if (rc) { cleanup(); return rc; } }
-    if (e == cudaSuccess) e = cudaMemcpy(out, d_out, px * 3, cudaMemcpyDeviceToHost);
-    cleanup();
+    DevBuf d_acc, d_out;
+    if ((rc = d_acc.alloc(px * 16)) || (rc = d_out.alloc(px * 3))) return rc;
+    cudaError_t e = cudaMemcpy(d_acc.p, accum, px * 16, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) { rc = b200rt_resolve_rgb8_device(d_acc.as<float>(), W, H, samples, d_out.as<uint8_t>(), nullptr); if (rc) return rc; }
+    if (e == cudaSuccess) e = cudaMemcpy(out, d_out.p, px * 3, cudaMemcpyDeviceToHost);
     if (e != cudaSuccess) return fail(B200RT_ECUDA, "resolve: %s", cudaGetErrorString(e));
     return B200RT_OK;
 }
@@ -1158,15 +1072,6 @@ int b200rt_resolve_rgb8(const float* accum, uint32_t W, uint32_t H, uint32_t sam
 }  // extern "C"
 
 // ---- parity hooks ---------------------------------------------------------------------------
-namespace {
-struct DevBuf {   // RAII device buffer for the hooks
-    void* p = nullptr;
-    ~DevBuf() { if (p) cudaFree(p); }
-    int alloc(size_t bytes) { CU(cudaMalloc(&p, bytes ? bytes : 16)); return B200RT_OK; }
-    template <class T> T* as() { return reinterpret_cast<T*>(p); }
-};
-}  // namespace
-
 extern "C" {
 
 int b200rt_closest_hit(const B200rtScene* csc, const B200rtRay* rays, size_t n, float t_min, float t_max, int32_t* ids, B200rtHit* hits, B200rtStats* stats) {
@@ -1185,38 +1090,25 @@ int b200rt_closest_hit(const B200rtScene* csc, const B200rtRay* rays, size_t n, 
     a.scene = sc->ds; a.rays = d_rays.as<B200rtRay>(); a.n = n; a.t_min = t_min; a.t_max = t_max;
     a.ids = d_ids.as<int32_t>(); a.hits = hits ? d_hits.as<B200rtHit>() : nullptr; a.counters = d_ctr.as<Counters>();
     a.next_ray = &d_ctr.as<Counters>()->diag[0];     // zeroed with the counters
-    SmemPlan plan = make_plan(sc, 2);
-    if (!plan.all_in_smem) { SmemPlan p1 = make_plan(sc, 1); if (p1.all_in_smem) plan = p1; }
+    const SmemPlan plan = hook_plan(scene_size(sc), sc->smem_optin);
     a.plan = plan;
-    cudaEvent_t e0, e1; CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));
-    auto go = [&](auto kernel) -> int {
-        int r2 = set_smem(kernel, sc, plan.bytes); if (r2) return r2;
-        int bps = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kernel, BLOCK, plan.bytes));
-        if (bps < 1) return fail(B200RT_ECUDA, "closest_hit_kernel does not fit on an SM");
-        size_t want = (n + BLOCK - 1) / BLOCK;
-        uint32_t grid = (uint32_t)std::min<size_t>(want, (size_t)sc->sm_count * bps);      // persistent: one wave of CTAs
-        CU(cudaEventRecord(e0));
-        kernel<<<grid, BLOCK, plan.bytes>>>(a);
-        CU(cudaGetLastError());
-        CU(cudaEventRecord(e1));
-        return B200RT_OK;
-    };
-    // the one-FMA / centre-form slab tests are conservative only while |origin| * eps stays below the box padding (as in launch_render)
-    float max_origin = sc->max_abs_coord;
+    float max_origin = 0.f;
     for (size_t i = 0; i < n; ++i) max_origin = std::max(max_origin, std::max(std::fabs(rays[i].ox), std::max(std::fabs(rays[i].oy), std::fabs(rays[i].oz))));
-    const char* fs = getenv("B200RT_FAST_SLAB");
-    bool fast = sc->box_pad >= 4.0f * 1.1920929e-7f * max_origin && !(fs && atoi(fs) == 0);
     // traversal counters ride along with the full hit records (parity runs); ids-only calls — the BVH microbenchmark
     // shape of benches/my_benchmark.rs — run the kernel without them
-    const bool count = stats != nullptr && hits != nullptr;
-#define B200RT_K1(ACC) (!fast ? go(closest_hit_kernel<ACC, true, false>) : (count ? go(closest_hit_kernel<ACC, true, true>) : go(closest_hit_kernel<ACC, false, true>)))
-    if (plan.all_in_smem) rc = B200RT_K1(SmemAcc); else rc = B200RT_K1(GmemAcc);
-#undef B200RT_K1
-    if (rc == B200RT_OK) {
-        cudaError_t e = cudaDeviceSynchronize();
-        if (e != cudaSuccess) rc = fail(B200RT_ECUDA, "closest_hit: %s", cudaGetErrorString(e));
-    }
+    HitKernel kernel = hit_kernel(plan.all_in_smem, use_fast_slab(sc, max_origin), stats != nullptr && hits != nullptr);
+    if ((rc = set_smem(kernel, sc, plan.bytes))) return rc;
+    int bps = 0;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kernel, BLOCK, plan.bytes));
+    if (bps < 1) return fail(B200RT_ECUDA, "closest_hit_kernel does not fit on an SM");
+    size_t want = (n + BLOCK - 1) / BLOCK;
+    uint32_t grid = (uint32_t)std::min<size_t>(want, (size_t)sc->sm_count * bps);      // persistent: one wave of CTAs
+    cudaEvent_t e0, e1; CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));
+    cudaError_t e = cudaEventRecord(e0);
+    if (e == cudaSuccess) { kernel<<<grid, BLOCK, plan.bytes>>>(a); e = cudaGetLastError(); }
+    if (e == cudaSuccess) e = cudaEventRecord(e1);
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) rc = fail(B200RT_ECUDA, "closest_hit: %s", cudaGetErrorString(e));
     if (rc == B200RT_OK) {
         cudaMemcpy(ids, d_ids.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost);
         if (hits) cudaMemcpy(hits, d_hits.p, n * sizeof(B200rtHit), cudaMemcpyDeviceToHost);
@@ -1225,7 +1117,7 @@ int b200rt_closest_hit(const B200rtScene* csc, const B200rtRay* rays, size_t n, 
             stats->rays = c.rays; stats->node_visits = c.nodes; stats->prim_tests = c.prims; stats->launches = 1;
             float ms = 0; cudaEventElapsedTime(&ms, e0, e1); stats->kernel_ms = ms; stats->total_ms = ms;
         }
-        cudaError_t e = cudaGetLastError();
+        e = cudaGetLastError();
         if (e != cudaSuccess) rc = fail(B200RT_ECUDA, "closest_hit copy-back: %s", cudaGetErrorString(e));
     }
     cudaEventDestroy(e0); cudaEventDestroy(e1);

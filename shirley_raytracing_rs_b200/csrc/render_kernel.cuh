@@ -8,17 +8,7 @@ namespace b200rt {
 // ------------------------------------------------------------------------------------------
 // kernel arguments
 // ------------------------------------------------------------------------------------------
-constexpr int BLOCK = 256;          // threads per CTA of the parity-hook kernels (K1); the render kernel's CTA size is its BLK template argument (768 by default)
 constexpr size_t LBVH_AUTO_MIN = 262144;   // primitives from which scene_create builds the tree on the device
-constexpr int TILE_W = 8, TILE_H = 4;   // one warp renders an 8x4 pixel tile, one lane per pixel
-constexpr uint32_t MAX_CHUNKS = 64;     // sample ranges per tile
-
-struct SmemPlan {
-    uint32_t all_in_smem;           // 1: nodes + geom + mats + tex all staged (SmemAcc)
-    uint32_t n_top;                 // nodes staged when !all_in_smem
-    uint32_t stack_depth;           // entries per thread
-    uint32_t bytes;                 // dynamic shared memory per CTA
-};
 
 struct Counters {                   // device-side, one per in-flight render
     unsigned long long rays, paths, nodes, prims, exhausted;
@@ -83,8 +73,6 @@ template <> struct Stager<GmemAcc> {
     }
 };
 
-constexpr uint32_t RAYQ_SLOTS = 32, RAYQ_FIELDS = 9;   // v2: o, d, RNG state + stream, tile pixel
-
 // Per-pixel sums as 64-bit fixed point (2^-32) in shared memory: integer adds commute, so the
 // result does not depend on which lane traced which sample, nor on scheduling or sharding.
 // Contract (INTEGRATION.md): a sample whose radiance is NaN or infinite contributes nothing (the reference would
@@ -137,8 +125,8 @@ __device__ __forceinline__ void acc_add(long long* acc, uint32_t pixel, float3 v
 //    of scheduling, row ranges, tile shards and sample ranges.
 // DESIGN.md §3 has the measurements behind each of these.
 // ------------------------------------------------------------------------------------------
-template <class Acc, bool COUNT, bool FAST, int BLK, int MINB>
-__global__ void __launch_bounds__(BLK, MINB) path_trace_kernel_v2(const __grid_constant__ RenderArgs a) {
+template <class Acc, bool COUNT, bool FAST, int BLK>
+__global__ void __launch_bounds__(BLK, 1) path_trace_kernel_v2(const __grid_constant__ RenderArgs a) {
     extern __shared__ float4 smem[];
     int* stack_base;
     Acc acc = Stager<Acc>::stage(a.scene, a.plan, smem, &stack_base);

@@ -6,6 +6,7 @@
 #include <stdint.h>
 
 #include "../../include/b200rt.h"
+#include "launch_plan.hpp"
 
 namespace b200rt {
 
@@ -84,11 +85,6 @@ struct DeviceCamera {
 // wavefronts per warp instead of up to 32 L1 tag lookups) or resident in global memory
 // behind the read-only path (GmemAcc), where the shared memory not used is left to the L1 cache.
 // ------------------------------------------------------------------------------------------
-// Staged nodes are padded to SMEM_NODE_QUADS x 16 B (80 B instead of 64): with a 64-byte stride the quad k of every node falls
-// into one of only two 16-byte bank groups (node parity), so the divergent LDS.128 of a quarter-warp collide; a stride of 5
-// quads walks all eight groups (measured +1.2 % on the bench frame; padding the 32-byte geometry records to 48 B the same
-// way measured 3 % slower).
-constexpr int SMEM_NODE_QUADS = 5;
 struct SmemAcc {
     const float4* nodes; const float4* geom; const float4* mats; const float4* tex;
     __device__ __forceinline__ float4 node_q(int node, int k) const { return nodes[node * SMEM_NODE_QUADS + k]; }
@@ -112,18 +108,14 @@ struct GmemAcc {
     // Every node comes through the read-only global path and the hardware L1.  (A staged shared-memory copy of the
     // top levels was measured: ~90 KB staged 6.4 Grays/s, 8 KB 7.3, none 7.2 on the 1e6-sphere scene — and the
     // `node < n_top` select on each of the four quads cost 15 of the 63 instructions of a traversal step.)
-    __device__ __forceinline__ float4 node_q(int node, int k) const { return __ldg(nodes + node * 4 + k); }
-    // One 64-byte node = two 256-bit read-only loads (LDG.E.256 on sm_100): half the L1 requests of four 128-bit ones.
+    // One 64-byte node = two 256-bit read-only loads (LDG.E.256 on sm_100): half the L1 requests of four 128-bit ones
+    // (profiles/r02_experiments.md §15).
     __device__ __forceinline__ void load_node(int node, float4& q0, float4& q1, float4& q2, float4& q3) const {
-#ifdef B200RT_NO_LDG256
-        q0 = node_q(node, 0); q1 = node_q(node, 1); q2 = node_q(node, 2); q3 = node_q(node, 3);
-#else
         const float4* p = nodes + (size_t)node * 4;
         asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
                      : "=f"(q0.x), "=f"(q0.y), "=f"(q0.z), "=f"(q0.w), "=f"(q1.x), "=f"(q1.y), "=f"(q1.z), "=f"(q1.w) : "l"(p));
         asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
                      : "=f"(q2.x), "=f"(q2.y), "=f"(q2.z), "=f"(q2.w), "=f"(q3.x), "=f"(q3.y), "=f"(q3.z), "=f"(q3.w) : "l"(p + 2));
-#endif
     }
     __device__ __forceinline__ float4 geom0(int id) const { return __ldg(geom + id * 2); }
     __device__ __forceinline__ float4 geom1(int id) const { return __ldg(geom + id * 2 + 1); }
