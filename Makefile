@@ -34,7 +34,7 @@ build/.mode: FORCE
 	@if [ "$$(cat $@ 2>/dev/null)" != "$(MODE)" ]; then echo "$(MODE)" > $@; fi
 FORCE:
 
-build/b200rt.o: build/.mode $(CSRC)/b200rt.cu $(wildcard $(CSRC)/*.cuh) $(CSRC)/bvh_build.hpp $(CSRC)/launch_plan.hpp include/b200rt.h
+build/b200rt.o: build/.mode $(CSRC)/b200rt.cu $(wildcard $(CSRC)/*.cuh) $(CSRC)/bvh_build.hpp $(CSRC)/launch_plan.hpp $(CSRC)/adaptive_plan.hpp include/b200rt.h
 	@mkdir -p build
 	$(NVCC) $(NVFLAGS) -c $(CSRC)/b200rt.cu -o $@ 2> build/ptxas_b200rt.log || (cat build/ptxas_b200rt.log; false)
 	@grep -E "error|warning: .*spill|bytes spill" build/ptxas_b200rt.log | grep -v "0 bytes spill" | head -20 || true

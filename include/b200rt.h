@@ -239,6 +239,46 @@ int  b200rt_render_rgb8(const B200rtScene* scene, const B200rtCamera* camera,
                         const B200rtRenderParams* params, uint8_t* out_rgb8, float* accum,
                         B200rtStats* stats);
 
+/* Tile-adaptive sampling: every 8x4 tile is rendered until its estimated output error is at most `threshold`.
+ * Sampling runs in passes over the tiles still active.  After pass k each of them has
+ *     n_k = min(initial_samples * 2^k, max_samples)
+ * samples; pass k renders samples [n_{k-1}, n_k) (n_{-1} = 0), offset by params->sample_offset, with the same RNG keying as
+ * b200rt_render (sample s of pixel p depends only on (seed, p, sample_offset + s)).  After every pass k >= 1 each active tile's
+ * error is estimated from the two independent means of the samples before the pass (n of them, exact sum F) and of the pass
+ * (s of them, exact sum P); per pixel and channel c, with every mean clamped at 1 like to_image:
+ *     a_c = min(F_c / n, 1)   b_c = min(P_c / s, 1)   m_c = min((F_c + P_c) / (n + s), 1)
+ *     sigma_c = |a_c - b_c| * sqrt(n s) / (n + s)                   standard error of the combined mean
+ *     e_p = max_c sigma_c / (2 sqrt(max(m_c, 2^-16)))               the same error after to_image's sqrt, 0..1 output units
+ *     e_T = max of e_p over the tile's selected pixels
+ * A tile stops after pass k when e_T <= threshold or n_k == max_samples; no tile stops before its first estimate, so every
+ * selected pixel gets at least min(2 * initial_samples, max_samples) samples.  threshold = 1/255 is about one 8-bit level
+ * of standard error.
+ *
+ * params: seed, max_depth, sample_offset, rows and device as for b200rt_render; `samples` is ignored; COUNT_TRAVERSAL is
+ * honoured.  ACCUMULATE, shard_count > 1, initial_samples == 0, max_samples <= initial_samples, a negative or non-finite
+ * threshold and a NULL scene, camera, params or adaptive return B200RT_EINVAL.
+ * Outputs (each may be NULL; host buffers):
+ *   accum       H*W float4 as for b200rt_render, but .w is the pixel's own sample count; pixels outside the rows are zero.
+ *               A tile that stopped after n samples equals a plain n-sample b200rt_render of it bit for bit, as long as no
+ *               sample's channel exceeds 2e9 / max_samples (the fixed-point clamp is taken for max_samples; every shipped
+ *               scene stays far below it).
+ *   out_rgb8    the resolve with per-pixel counts: equal to b200rt_resolve_rgb8(accum, W, H, 0, ...).
+ *   tile_error  ceil(W/8) * ceil(H/4) floats, tile (tx, ty) covering x in [8tx, 8tx+8), y in [4ty, 4ty+4) (row 0 = bottom,
+ *               as in accum): the tile's e_T at its last pass; -1 for tiles with no selected pixel.
+ * stats: rays and paths summed over the passes (paths = the sum of .w over the selected pixels), kernel_ms = the summed
+ * path-tracing kernel times, total_ms and launches for the whole call.  The call synchronises once per pass to read how many
+ * tiles are still active. */
+typedef struct B200rtAdaptiveParams {
+    uint32_t initial_samples;   /* first pass, every selected tile; >= 1 */
+    uint32_t max_samples;       /* no pixel gets more; > initial_samples */
+    float    threshold;         /* stop a tile when e_T <= threshold (0..1 output units); >= 0, finite */
+    uint32_t _pad;
+} B200rtAdaptiveParams;
+
+int  b200rt_render_adaptive(const B200rtScene* scene, const B200rtCamera* camera,
+                            const B200rtRenderParams* params, const B200rtAdaptiveParams* adaptive,
+                            float* accum, uint8_t* out_rgb8, float* tile_error, B200rtStats* stats);
+
 /* render_scene on SEVERAL GPUs from one host process: `params->samples` is the total per pixel, split into
  * contiguous sample ranges over `devices[0 .. n_devices)` (each gets its own copy of the scene, uploaded by its
  * own host thread); devices[0] sums the per-device buffers inside the resolve through peer access and returns

@@ -92,6 +92,10 @@ class Stats(C.Structure):
                 ("launches", C.c_uint32), ("_pad", C.c_uint32), ("diag", C.c_uint64 * 8)]
 
 
+class AdaptiveParams(C.Structure):
+    _fields_ = [("initial_samples", C.c_uint32), ("max_samples", C.c_uint32), ("threshold", C.c_float), ("_pad", C.c_uint32)]
+
+
 class SceneInfo(C.Structure):
     _fields_ = [("n_prims", C.c_uint32), ("n_bvh_nodes", C.c_uint32), ("bvh_depth", C.c_uint32),
                 ("bvh_nodes_in_smem", C.c_uint32), ("device_bytes", C.c_uint64), ("bvh_build_ms", C.c_float), ("bvh_builder", C.c_uint32)]
@@ -123,6 +127,8 @@ SIGNATURES = {
     "b200rt_scene_info": (C.c_int, [C.c_void_p, _P(SceneInfo)]),
     "b200rt_render": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, _P(Stats)]),
     "b200rt_render_rgb8": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p, _P(Stats)]),
+    "b200rt_render_adaptive": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), _P(AdaptiveParams), C.c_void_p, C.c_void_p,
+                                         C.c_void_p, _P(Stats)]),
     "b200rt_render_rgb8_multi": (C.c_int, [_P(SceneDesc), _P(C.c_int), C.c_uint32, _P(Camera), _P(RenderParams), C.c_void_p, _P(Stats)]),
     "b200rt_render_device": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p]),
     "b200rt_render_device_finish": (C.c_int, [C.c_void_p, C.c_void_p, _P(Stats)]),

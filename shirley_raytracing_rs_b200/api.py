@@ -335,6 +335,25 @@ def render(scene: Scene, cam: F.Camera, samples: int = 100, max_depth: int = 50,
     return accum, st
 
 
+def render_adaptive(scene: Scene, cam: F.Camera, max_samples: int, threshold: float, initial_samples: int = 16, max_depth: int = 50,
+                    seed: int = 0, *, sample_offset: int = 0, rows=(0, 0), count_traversal: bool = False, device: int = -1):
+    """Tile-adaptive sampling (b200rt_render_adaptive): every 8x4 tile is rendered in passes of doubling sample counts,
+    from `initial_samples` up to at most `max_samples`, until its estimated standard error after to_image's gamma is at most
+    `threshold` (0..1 output units; 1/255 is about one 8-bit level).  Returns (accum[H, W, 4] float32 {sum r,g,b, n} with
+    n the pixel's own sample count, tile_error[ceil(H/4), ceil(W/8)] float32 (each tile's last estimate, -1 outside `rows`;
+    row 0 is the bottom, as in accum), Stats)."""
+    H, W = cam.image_height, cam.image_width
+    accum = np.empty((H, W, 4), dtype=np.float32)
+    tile_error = np.empty(((H + 3) // 4, (W + 7) // 8), dtype=np.float32)
+    p = F.RenderParams(sample_offset=sample_offset, max_depth=max_depth, flags=F.FLAG_COUNT_TRAVERSAL if count_traversal else 0,
+                       seed=seed, row_begin=rows[0], row_end=rows[1], device=-1)
+    ad = F.AdaptiveParams(initial_samples=initial_samples, max_samples=max_samples, threshold=threshold)
+    st = F.Stats()
+    F.check(lib.b200rt_render_adaptive(scene.device(device), C.byref(cam), C.byref(p), C.byref(ad), accum.ctypes.data, None,
+                                       tile_error.ctypes.data, C.byref(st)))
+    return accum, tile_error, st
+
+
 def resolve_rgb8(accum: np.ndarray, samples: int = 0, device: int = -1) -> np.ndarray:
     """to_image's pixel loop (image.rs:34-40): mean, sqrt gamma, saturating u8, vertical flip."""
     accum = np.ascontiguousarray(accum, dtype=np.float32)

@@ -5,6 +5,8 @@
 //   ray-cli [-v...] render {random|saved|demo|perlin|earth|box-light|cornell} [flags] [scene_input]
 //   ray-cli test
 // Extra flag (not in the reference): --seed N replaces the OS-seeded thread_rng.
+#include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -34,6 +36,8 @@ struct Args {
     uint64_t seed = 0x5EED5EEDull;
     std::string checkpoint;     // extra: accumulation-buffer checkpoint (resumed if it exists)
     int gpus = 1;               // extra: render on the first N GPUs of this box (one process, peer access)
+    double adaptive = -1.0;     // extra: tile-adaptive sampling to this standard error in 8-bit levels (< 0: off); --samples is the maximum
+    uint32_t adaptive_initial = 16;
 };
 
 [[noreturn]] void usage(const char* msg) {
@@ -56,7 +60,10 @@ struct Args {
             "      --seed <N>                   seed for scene generation and sampling\n"
             "      --gpus <N>                   split the samples over the first N GPUs (NVLink peers) and sum inside the resolve\n"
             "      --checkpoint <FILE>          save the accumulation buffer there; if FILE exists, continue from it:\n"
-            "                                   --samples more samples are added (same scene, camera and seed required)\n");
+            "                                   --samples more samples are added (same scene, camera and seed required)\n"
+            "      --adaptive <LEVELS>          tile-adaptive sampling: render each 8x4 tile until its estimated standard error\n"
+            "                                   is at most LEVELS 8-bit levels; --samples becomes the maximum per pixel\n"
+            "      --adaptive-initial <N>       samples of the first adaptive pass [default: 16]\n");
     exit(msg ? 2 : 0);
 }
 
@@ -93,9 +100,17 @@ Args parse(int argc, char** argv) {
         else if (s == "--seed") a.seed = strtoull(need("--seed").c_str(), nullptr, 0);
         else if (s == "--checkpoint") a.checkpoint = need("--checkpoint");
         else if (s == "--gpus") { a.gpus = atoi(need("--gpus").c_str()); if (a.gpus < 1) usage("--gpus needs a positive count"); }
+        else if (s == "--adaptive") {
+            char* end = nullptr; std::string v = need("--adaptive");
+            a.adaptive = strtod(v.c_str(), &end);
+            if (v.empty() || *end || !std::isfinite(a.adaptive) || a.adaptive < 0) usage("--adaptive needs a finite number of levels >= 0");
+        }
+        else if (s == "--adaptive-initial") { int n = atoi(need("--adaptive-initial").c_str()); if (n < 1) usage("--adaptive-initial needs a positive count"); a.adaptive_initial = (uint32_t)n; }
         else if (!s.empty() && s[0] == '-') usage(("unexpected argument " + s).c_str());
         else pos.push_back(s);
     }
+    if (a.adaptive >= 0 && a.gpus > 1) usage("--adaptive renders on one GPU: it cannot be combined with --gpus");
+    if (a.adaptive >= 0 && !a.checkpoint.empty()) usage("--adaptive cannot be combined with --checkpoint");
     if (pos.empty()) usage("a subcommand is required");
     if (pos[0] == "test") { a.sub = "test"; return a; }
     if (pos[0] != "render" || pos.size() < 2) usage("expected `render <scene>`");
@@ -134,7 +149,20 @@ int render_scene(const Args& args, const scene::SceneBuilder& builder, const cam
     B200rtRenderParams p{};
     p.samples = (uint32_t)samples; p.max_depth = (uint32_t)args.max_reflect; p.seed = args.seed; p.device = -1;
     B200rtStats st{};
-    if (args.checkpoint.empty()) {
+    if (args.adaptive >= 0) {
+        B200rtAdaptiveParams ad{};
+        ad.initial_samples = args.adaptive_initial; ad.max_samples = (uint32_t)samples; ad.threshold = (float)(args.adaptive / 255.0);
+        std::vector<float> accum((size_t)c.image_width * c.image_height * 4);
+        rc = b200rt_render_adaptive(dev, &c, &p, &ad, accum.data(), rgb.data(), nullptr, &st);
+        if (!rc && args.verbose >= 1) {
+            float most = 0.f;                          // the last pass brought the most-sampled tiles to this count
+            for (size_t k = 3; k < accum.size(); k += 4) most = std::max(most, accum[k]);
+            uint32_t passes = 1;
+            for (uint64_t n = ad.initial_samples; n < (uint64_t)most; n *= 2) ++passes;
+            fprintf(stderr, " INFO  adaptive to %g levels: %.1f spp on average (at most %zu), %u passes\n", args.adaptive,
+                    (double)st.paths / ((double)c.image_width * c.image_height), samples, passes);
+        }
+    } else if (args.checkpoint.empty()) {
         rc = b200rt_render_rgb8(dev, &c, &p, rgb.data(), nullptr, &st);
     } else {
         // progressive: continue the checkpoint's sample sequence (same seed, sample_offset = samples done)

@@ -9,6 +9,7 @@
 //   lbvh.cuh             K5 linear BVH built on the device                         (bvh/bbox_tree/constructor.rs:9-212)
 //   bvh_build.hpp        host binned-SAH builder
 //   launch_plan.hpp      CTA size, shared-memory plan, sample-range schedule and grid of a launch (pure host arithmetic)
+//   adaptive_plan.hpp    pass schedule and error estimate of tile-adaptive sampling (host and device)
 // No tensor cores: nothing on this path is a dense contraction.  No CPU fallback.
 #include <cuda_runtime.h>
 
@@ -71,7 +72,9 @@ struct Scratch {                     // per in-flight render: counters, events, 
     cudaStream_t launch_stream = nullptr; bool launched = false;   // where the render in flight was enqueued (scene_destroy waits for it)
     float4* d_accum = nullptr; size_t accum_bytes = 0;
     uint8_t* d_rgb = nullptr; size_t rgb_bytes = 0;
-    long long* d_fix = nullptr; size_t fix_bytes = 0;  // fixed-point sums of a launch whose tiles are split into sample chunks
+    long long* d_fix = nullptr; size_t fix_bytes = 0;  // fixed-point sums of a launch whose tiles are split into sample chunks (adaptive: F)
+    long long* d_pass = nullptr; size_t pass_bytes = 0;  // adaptive: the fixed-point sums of one pass (P)
+    uint32_t* d_tiles = nullptr; size_t tiles_bytes = 0;  // adaptive: two tile lists, keep flags, tile errors, the active count
     uint32_t launches = 0;
 };
 
@@ -287,7 +290,12 @@ template <class Acc> HitKernel hit_variant(bool fast, bool count) {
 }
 HitKernel hit_kernel(bool all_in_smem, bool fast, bool count) { return all_in_smem ? hit_variant<SmemAcc>(fast, count) : hit_variant<GmemAcc>(fast, count); }
 
-int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderParams* prm, float* d_accum, cudaStream_t stream, Scratch* scr) {
+// One pass of b200rt_render_adaptive: the tiles it renders (NULL: all of them), the fixed-point buffer its sums are added to,
+// and the sample count acc_add's clamp is taken for (max_samples, so that the sums of all passes cannot wrap).
+struct AdaptivePass { const uint32_t* tile_list; uint32_t n_tiles; long long* fix; uint32_t lim_samples; };
+
+int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderParams* prm, float* d_accum, cudaStream_t stream, Scratch* scr,
+                  const AdaptivePass* pass = nullptr) {
     if (cam->image_width == 0 || cam->image_height == 0) return fail(B200RT_EINVAL, "camera image dimensions are zero");
     if ((uint64_t)cam->image_width * cam->image_height > 0xFFFFFFFFull) return fail(B200RT_EINVAL, "image too large");
     RenderArgs a{};
@@ -295,6 +303,8 @@ int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderPa
     a.cam = make_camera(*cam);
     a.keys = rng_keys(prm->seed);
     a.samples = prm->samples == 0 ? 1 : prm->samples;   // src/main.rs:75-80
+    a.lim_samples = pass ? pass->lim_samples : a.samples;
+    a.tile_list = pass ? pass->tile_list : nullptr;
     a.sample_offset = prm->sample_offset;
     a.max_depth = prm->max_depth;
     uint32_t H = cam->image_height, W = cam->image_width;
@@ -329,20 +339,22 @@ int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderPa
     // The kernel stores every pixel of the tiles it renders; the buffer is cleared only when some pixels are outside them
     // ("pixels outside the selected rows/tiles are written as zeros", include/b200rt.h).
     const bool covers_frame = a.shard_count == 1 && a.row_begin == 0 && a.row_end == H;
-    if (!a.accumulate && !covers_frame) CU(cudaMemsetAsync(d_accum, 0, (size_t)W * H * sizeof(float4), stream));
+    // (adaptive passes write only through the merge kernel; b200rt_render_adaptive clears the buffer once)
+    if (!pass && !a.accumulate && !covers_frame) CU(cudaMemsetAsync(d_accum, 0, (size_t)W * H * sizeof(float4), stream));
     int rc = set_smem(kernel, sc, plan.bytes); if (rc) return rc;
     int blocks_per_sm = 0;
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kernel, block_threads, plan.bytes));
     if (blocks_per_sm < 1) return fail(B200RT_ECUDA, "path-tracing kernel does not fit on an SM (smem %u B, %u threads)", plan.bytes, block_threads);
     const uint32_t warps_per_block = block_threads / 32;
-    const uint32_t my_tiles = a.n_tiles > a.shard_index ? (a.n_tiles - a.shard_index + a.shard_count - 1) / a.shard_count : 0u;   // tiles t with t % shard_count == shard_index
+    const uint32_t my_tiles = pass ? pass->n_tiles
+                            : a.n_tiles > a.shard_index ? (a.n_tiles - a.shard_index + a.shard_count - 1) / a.shard_count : 0u;   // tiles t with t % shard_count == shard_index
     const uint32_t full_grid = (uint32_t)(sc->sm_count * blocks_per_sm);
     const SampleSchedule sched = sample_schedule(a.samples, my_tiles, full_grid * warps_per_block, plan.all_in_smem, env_int("B200RT_CHUNKS", 0));
     a.chunks = sched.chunks;
     a.my_tiles = my_tiles ? my_tiles : 1u;
     std::copy(sched.chunk_begin, sched.chunk_begin + MAX_CHUNKS + 1, a.chunk_begin);
-    a.fix = nullptr;
-    if (a.chunks > 1u) {
+    a.fix = pass ? pass->fix : nullptr;
+    if (!pass && a.chunks > 1u) {
         const size_t px = (size_t)W * H;
         cudaError_t e = grow(scr->d_fix, scr->fix_bytes, px * 3 * sizeof(long long));
         if (e != cudaSuccess) return fail(B200RT_ENOMEM, "fixed-point accumulation buffer (%zu px): %s", px, cudaGetErrorString(e));
@@ -353,7 +365,7 @@ int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderPa
     kernel<<<render_grid(full_grid, my_tiles, a.chunks, warps_per_block), block_threads, plan.bytes, stream>>>(a);
     CU(cudaGetLastError());
     scr->launches += 1;
-    if (a.chunks > 1u && a.row_end > a.row_begin) {
+    if (!pass && a.chunks > 1u && a.row_end > a.row_begin) {
         dim3 fb(128, 1), fg((W + 127) / 128, a.row_end - a.row_begin);
         finalize_kernel<<<fg, fb, 0, stream>>>(a);
         CU(cudaGetLastError());
@@ -751,6 +763,117 @@ int b200rt_render(const B200rtScene* csc, const B200rtCamera* cam, const B200rtR
 int b200rt_render_rgb8(const B200rtScene* csc, const B200rtCamera* cam, const B200rtRenderParams* prm, uint8_t* out_rgb8, float* accum, B200rtStats* stats) {
     if (!csc || !cam || !prm || !out_rgb8) return fail(B200RT_EINVAL, "NULL argument");
     return render_host_impl(csc, cam, prm, accum, out_rgb8, stats);
+}
+
+// Tile-adaptive sampling (b200rt_render_adaptive): passes over the still-active tiles (adaptive_plan.hpp), each one K2 launch over the tile list, the merge
+// kernel (estimate, F += P, stopped tiles' pixels) and the compaction of the next list; the host reads the active count after
+// each pass.  Pass 0 adds straight into F and renders every tile; pass 1 still renders every tile, so it needs no list either.
+static int render_adaptive_impl(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderParams* prm, const B200rtAdaptiveParams* ad,
+                                float* accum, uint8_t* out_rgb8, float* tile_error, B200rtStats* stats, Scratch* scr) {
+    const uint32_t W = cam->image_width, H = cam->image_height;
+    uint32_t row_begin = prm->row_begin, row_end = prm->row_end;
+    if (row_begin == 0 && row_end == 0) row_end = H;
+    const uint32_t tiles_x = (W + TILE_W - 1) / TILE_W, tile_row0 = row_begin / TILE_H, tile_row1 = (row_end + TILE_H - 1) / TILE_H;
+    const uint32_t n_tiles = row_end > row_begin ? tiles_x * (tile_row1 - tile_row0) : 0u;
+    const size_t px = (size_t)W * H;
+    cudaError_t e = grow(scr->d_accum, scr->accum_bytes, px * sizeof(float4));
+    if (e == cudaSuccess) e = grow(scr->d_fix, scr->fix_bytes, px * 3 * sizeof(long long));
+    if (e == cudaSuccess) e = grow(scr->d_pass, scr->pass_bytes, px * 3 * sizeof(long long));
+    if (e == cudaSuccess) e = grow(scr->d_tiles, scr->tiles_bytes, ((size_t)n_tiles * 4 + 1) * sizeof(uint32_t));
+    if (e == cudaSuccess && out_rgb8) e = grow(scr->d_rgb, scr->rgb_bytes, px * 3);
+    if (e != cudaSuccess) return fail(B200RT_ENOMEM, "adaptive sampling buffers (%zu px): %s", px, cudaGetErrorString(e));
+    uint32_t* lists[2] = {scr->d_tiles, scr->d_tiles + n_tiles};
+    uint32_t* keep = scr->d_tiles + 2 * (size_t)n_tiles;
+    float* d_err = reinterpret_cast<float*>(scr->d_tiles + 3 * (size_t)n_tiles);
+    uint32_t* d_count = scr->d_tiles + 4 * (size_t)n_tiles;
+    cudaStream_t stream = scr->own_stream;
+    // ev3 marks the start of the call; launch_render records ev0..ev2 per pass, and ev0 is recorded again to mark the end
+    CU(cudaEventRecord(scr->ev3, stream));
+    CU(cudaMemsetAsync(scr->d_accum, 0, px * sizeof(float4), stream));
+    CU(cudaMemsetAsync(scr->d_fix, 0, px * 3 * sizeof(long long), stream));
+    CU(cudaMemsetAsync(scr->d_pass, 0, px * 3 * sizeof(long long), stream));
+
+    B200rtRenderParams p = *prm;
+    p.flags &= B200RT_FLAG_COUNT_TRAVERSAL; p.shard_count = 1; p.shard_index = 0; p.row_begin = row_begin; p.row_end = row_end;
+    B200rtStats sum{};
+    uint32_t n_prev = 0, active = n_tiles, launches = 0, which = 0;
+    const uint32_t* list = nullptr;
+    for (uint32_t k = 0; active > 0; ++k) {
+        const uint32_t n = adaptive_samples_after(ad->initial_samples, ad->max_samples, k);
+        p.samples = n - n_prev; p.sample_offset = prm->sample_offset + n_prev;
+        const AdaptivePass pass{list, active, k == 0 ? scr->d_fix : scr->d_pass, ad->max_samples};
+        if (int rc = launch_render(sc, cam, &p, reinterpret_cast<float*>(scr->d_accum), stream, scr, &pass)) return rc;
+        launches += scr->launches;
+        uint32_t next = active;
+        if (k > 0) {
+            MergeArgs m{};
+            m.list = list; m.n_active = active; m.F = scr->d_fix; m.P = scr->d_pass; m.accum = scr->d_accum; m.tile_error = d_err; m.keep = keep;
+            m.n = n_prev; m.s = n - n_prev; m.last = n == ad->max_samples ? 1u : 0u; m.threshold = ad->threshold;
+            m.W = W; m.row_begin = row_begin; m.row_end = row_end; m.tiles_x = tiles_x; m.tile_row0 = tile_row0;
+            adaptive_merge_kernel<<<(active + 7) / 8, 256, 0, stream>>>(m);
+            CU(cudaGetLastError());
+            adaptive_compact_kernel<<<1, COMPACT_THREADS, 0, stream>>>(list, keep, active, lists[which], d_count);
+            CU(cudaGetLastError());
+            launches += 2;
+            CU(cudaMemcpyAsync(&next, d_count, sizeof next, cudaMemcpyDeviceToHost, stream));
+        }
+        CU(cudaStreamSynchronize(stream));
+        const Counters& c = *scr->h_counters;
+        sum.rays += c.rays; sum.paths += c.paths; sum.node_visits += c.nodes; sum.prim_tests += c.prims; sum.depth_exhausted += c.exhausted;
+        for (int d = 0; d < 8; ++d) sum.diag[d] += c.diag[d];
+        float ms = 0.f;
+        CU(cudaEventElapsedTime(&ms, scr->ev1, scr->ev2)); sum.kernel_ms += ms;
+        if (k > 0) { list = lists[which]; which ^= 1u; }
+        active = next; n_prev = n;
+    }
+    if (out_rgb8) {
+        if (int rc = b200rt_resolve_rgb8_device(reinterpret_cast<float*>(scr->d_accum), W, H, 0, scr->d_rgb, stream)) return rc;
+        launches += 1;
+        e = cudaMemcpyAsync(out_rgb8, scr->d_rgb, px * 3, cudaMemcpyDeviceToHost, stream);
+    }
+    if (e == cudaSuccess && accum) e = cudaMemcpyAsync(accum, scr->d_accum, px * sizeof(float4), cudaMemcpyDeviceToHost, stream);
+    if (e == cudaSuccess && tile_error) {
+        // tiles with no selected pixel: -1; the others sit in one contiguous block of tile rows
+        std::fill(tile_error, tile_error + (size_t)tiles_x * ((H + TILE_H - 1) / TILE_H), -1.0f);
+        if (n_tiles) e = cudaMemcpyAsync(tile_error + (size_t)tile_row0 * tiles_x, d_err, n_tiles * sizeof(float), cudaMemcpyDeviceToHost, stream);
+    }
+    if (e == cudaSuccess) e = cudaEventRecord(scr->ev0, stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+    if (e != cudaSuccess) return fail(B200RT_ECUDA, "adaptive sampling copy-back: %s", cudaGetErrorString(e));
+    if (stats) {
+        float ms = 0.f;
+        CU(cudaEventElapsedTime(&ms, scr->ev3, scr->ev0));
+        sum.total_ms = ms;
+        sum.launches = launches;
+        *stats = sum;
+    }
+    return B200RT_OK;
+}
+
+int b200rt_render_adaptive(const B200rtScene* csc, const B200rtCamera* cam, const B200rtRenderParams* prm, const B200rtAdaptiveParams* ad,
+                           float* accum, uint8_t* out_rgb8, float* tile_error, B200rtStats* stats) {
+    if (!csc || !cam || !prm || !ad) return fail(B200RT_EINVAL, "NULL argument");
+    if (prm->flags & B200RT_FLAG_ACCUMULATE) return fail(B200RT_EINVAL, "adaptive sampling cannot add to an earlier result (B200RT_FLAG_ACCUMULATE)");
+    if (prm->shard_count > 1) return fail(B200RT_EINVAL, "adaptive sampling renders whole frames: shard_count %u is not supported", prm->shard_count);
+    if (ad->initial_samples == 0) return fail(B200RT_EINVAL, "adaptive initial_samples is 0");
+    if (ad->max_samples <= ad->initial_samples) return fail(B200RT_EINVAL, "adaptive max_samples %u must exceed initial_samples %u", ad->max_samples, ad->initial_samples);
+    if (!(ad->threshold >= 0.0f) || !std::isfinite(ad->threshold)) return fail(B200RT_EINVAL, "adaptive threshold %g must be finite and >= 0", (double)ad->threshold);
+    B200rtScene* sc = const_cast<B200rtScene*>(csc);
+    if (prm->device >= 0 && prm->device != sc->device) return fail(B200RT_EINVAL, "params.device %d != scene device %d", prm->device, sc->device);
+    const uint32_t W = cam->image_width, H = cam->image_height;
+    if (W == 0 || H == 0) return fail(B200RT_EINVAL, "camera image dimensions are zero");
+    if ((uint64_t)W * H > 0xFFFFFFFFull) return fail(B200RT_EINVAL, "image too large");
+    const uint32_t row_end = prm->row_begin == 0 && prm->row_end == 0 ? H : prm->row_end;
+    if (row_end > H || prm->row_begin > row_end) return fail(B200RT_EINVAL, "row range [%u,%u) outside image height %u", prm->row_begin, row_end, H);
+
+    DeviceGuard guard(sc->device);
+    int key_local; void* key = &key_local;   // private key: concurrent host threads never collide
+    Scratch* scr; int rc = get_scratch(sc, key, &scr); if (rc) return rc;
+    rc = render_adaptive_impl(sc, cam, prm, ad, accum, out_rgb8, tile_error, stats, scr);
+    if (rc) cudaStreamSynchronize(scr->own_stream);   // nothing of a failed call may still run when its scratch is reused
+    scr->launched = false;
+    put_scratch(sc, key);
+    return rc;
 }
 
 // ---- render_scene on several GPUs from ONE host process (what a `ray-cli` user has) -------------------------------

@@ -1,6 +1,7 @@
 // render_kernel.cuh — K2: kernel arguments, scene staging and the persistent path-tracing kernel (path_trace_kernel_v2), the default
 // (included by b200rt.cu; everything lives in namespace b200rt)
 #pragma once
+#include "adaptive_plan.hpp"
 #include "rt_device.cuh"
 
 namespace b200rt {
@@ -26,13 +27,16 @@ struct RenderArgs {
     uint32_t tiles_x, tile_row0, n_tiles;       // tile grid covering [row_begin, row_end)
     uint32_t shard_count, shard_index;
     uint32_t accumulate;
-    uint32_t chunks;                            // work item = (tile, one of `chunks` contiguous sample ranges); > 1: sums go to `fix`
+    uint32_t chunks;                            // work item = (tile, one of `chunks` contiguous sample ranges)
     // Items are handed out chunk by chunk (all tiles' first ranges, then all second ones, ...) and the ranges SHRINK
     // (chunk_begin[k] .. chunk_begin[k + 1]): big items while the grid is full, small ones at the end of the launch, where the
     // last items to finish decide how long the other SMs idle.  my_tiles = this shard's tiles.
     uint32_t my_tiles;
     uint32_t chunk_begin[MAX_CHUNKS + 1];
-    long long* fix;                             // chunks > 1: per-pixel 2^-32 fixed-point sums [H][W][3] in global memory (finalize_kernel converts)
+    long long* fix;                             // non-NULL: the sums are added to these per-pixel 2^-32 fixed-point sums [H][W][3] in global memory
+                                                // (plain renders: when chunks > 1, finalize_kernel converts; adaptive passes: the pass buffer)
+    const uint32_t* tile_list;                  // non-NULL: item j renders tile tile_list[j % my_tiles] (adaptive passes: the active tiles)
+    uint32_t lim_samples;                       // acc_add's clamp is 2e9 / lim_samples: `samples` for plain renders, max_samples for adaptive passes
     uint32_t trav_threshold;                    // leave the traversal loop when fewer lanes than this still traverse
     uint32_t regen_min;                         // hand out new paths only when at least this many lanes are free
     float4* accum;
@@ -77,7 +81,7 @@ template <> struct Stager<GmemAcc> {
 // result does not depend on which lane traced which sample, nor on scheduling or sharding.
 // Contract (INTEGRATION.md): a sample whose radiance is NaN or infinite contributes nothing (the reference would
 // carry the NaN into the pixel, which to_image writes as 0).  Each channel of a finite sample is clamped to +-`lim` =
-// 2e9 / samples-per-call, so a pixel's 2^-32 fixed-point sum (63 bits: |sum| < 2^31 = 2.1e9) cannot wrap whatever the
+// 2e9 / samples-per-call (adaptive passes: 2e9 / max_samples, over all passes), so a pixel's 2^-32 fixed-point sum (63 bits: |sum| < 2^31 = 2.1e9) cannot wrap whatever the
 // emitters' strength; a clamped sample still saturates the pixel (to_image clips the mean at 1).
 // The 64-bit add is two native 32-bit shared-memory atomics (low word with the old value returned, then the high word
 // plus the carry, skipped when both are zero — the usual case: samples below 1.0 have no high word): integer adds
@@ -155,7 +159,7 @@ __global__ void __launch_bounds__(BLK, 1) path_trace_kernel_v2(const __grid_cons
     const bool has_perlin = a.scene.perlin != nullptr;
     // (the Perlin tables stay in global memory behind L1: a shared-memory copy reached through generic loads measured 0.4 % slower)
     const PerlinRec* perlin_tables = a.scene.perlin;
-    const float sample_lim = 2.0e9f / (float)a.samples;   // acc_add: the per-call fixed-point sum cannot wrap
+    const float sample_lim = 2.0e9f / (float)a.lim_samples;   // acc_add: the fixed-point sum cannot wrap
 
     unsigned long long w_rays = 0, w_paths = 0, w_exh = 0, w_nodes = 0, w_prims = 0;
     // lane-utilisation diagnostics (COUNT only, lane 0 of each warp):
@@ -165,15 +169,19 @@ __global__ void __launch_bounds__(BLK, 1) path_trace_kernel_v2(const __grid_cons
     unsigned long long d0 = 0, d1 = 0, d2 = 0, d3 = 0, d4 = 0, d5 = 0, d6 = 0, d7 = 0;
 
     for (;;) {
-        unsigned int j = 0;
-        if (lane == 0) j = atomicAdd(&a.counters->tile_counter, 1u);
+        unsigned int j = 0, listed = 0;
+        if (lane == 0) {
+            j = atomicAdd(&a.counters->tile_counter, 1u);
+            if (a.tile_list && j < a.chunks * a.my_tiles) listed = a.tile_list[j % a.my_tiles];
+        }
         j = __shfl_sync(FULL, j, 0);
         // Work item j = (sample range j / my_tiles, tile j % my_tiles): a tile's samples are split over several warps when the
         // frame has too few tiles to balance the grid (1200x800 at 500 spp is 10.5 whole tiles per warp: the kernel ran 18 %
         // below its rate on frames with 4x the tiles).  Bottom rows first within every range.
         const uint32_t chunk = j / a.my_tiles;
         if (chunk >= a.chunks) break;
-        const uint32_t t = (j - chunk * a.my_tiles) * a.shard_count + a.shard_index;
+        uint32_t t = (j - chunk * a.my_tiles) * a.shard_count + a.shard_index;
+        if (a.tile_list) t = __shfl_sync(FULL, listed, 0);
         const uint32_t s_begin = a.chunk_begin[chunk];
         const uint32_t s_count = a.chunk_begin[chunk + 1u] - s_begin;
         uint32_t ty = t / a.tiles_x, tx = t - ty * a.tiles_x;
@@ -334,8 +342,8 @@ __global__ void __launch_bounds__(BLK, 1) path_trace_kernel_v2(const __grid_cons
         }
         __syncwarp();
         if (valid) {
-            if (a.chunks > 1u) {
-                // several warps hold partial sums of this pixel: exact 64-bit integer adds in global memory (native RED.ADD.64),
+            if (a.fix) {
+                // several warps (or passes) hold partial sums of this pixel: exact 64-bit integer adds in global memory (native RED.ADD.64),
                 // so the total — and the float finalize_kernel derives from it — is the same whatever the split or the order
                 unsigned long long* f = reinterpret_cast<unsigned long long*>(a.fix) + ((size_t)my_py * a.cam.width + my_px) * 3;
                 atomicAdd(f + 0, (unsigned long long)wacc[lane * 3 + 0]);
@@ -388,6 +396,79 @@ __global__ void finalize_kernel(const __grid_constant__ RenderArgs a) {
     float4 v = make_float4((float)a.fix[p * 3 + 0] * inv, (float)a.fix[p * 3 + 1] * inv, (float)a.fix[p * 3 + 2] * inv, (float)a.samples);
     if (a.accumulate) { float4 o = a.accum[p]; v.x += o.x; v.y += o.y; v.z += o.z; v.w += o.w; }
     a.accum[p] = v;
+}
+
+// ------------------------------------------------------------------------------------------
+// Tile-adaptive sampling (b200rt_render_adaptive).  After pass k >= 1 the pass buffer P holds the sums of the samples
+// [n, n + s) of every active tile and F those of [0, n).  One warp per active tile, one lane per pixel: e_p from the two
+// independent means (adaptive_plan.hpp), e_T = the warp maximum; P is added into F exactly (64-bit integers) and zeroed for the
+// next pass; a tile that stops writes its float4 pixels with finalize_kernel's arithmetic, so they equal a plain render of
+// n + s samples bit for bit.
+// ------------------------------------------------------------------------------------------
+struct MergeArgs {
+    const uint32_t* list;       // the active tiles (NULL: all tiles 0 .. n_active)
+    uint32_t n_active;
+    long long* F;               // [H][W][3] sums before the pass
+    long long* P;               // [H][W][3] sums of the pass
+    float4* accum;
+    float* tile_error;          // per tile of the grid covering [row_begin, row_end): e_T at its last pass
+    uint32_t* keep;             // per list entry: 1 = still active
+    uint32_t n, s;              // samples before the pass, samples of the pass
+    uint32_t last;              // n + s == max_samples: every tile stops
+    float threshold;
+    uint32_t W, row_begin, row_end, tiles_x, tile_row0;
+};
+
+__global__ void adaptive_merge_kernel(const __grid_constant__ MergeArgs a) {
+    const uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const uint32_t lane = threadIdx.x & 31u;
+    if (i >= a.n_active) return;                 // warp-uniform
+    const uint32_t t = a.list ? a.list[i] : i;
+    const uint32_t ty = t / a.tiles_x, tx = t - ty * a.tiles_x;
+    const uint32_t x = tx * TILE_W + (lane & (TILE_W - 1)), y = (a.tile_row0 + ty) * TILE_H + (lane >> 3);
+    const bool valid = x < a.W && y >= a.row_begin && y < a.row_end;
+    const size_t p = ((size_t)y * a.W + x) * 3;
+    float e = 0.0f;
+    long long sum[3] = {0, 0, 0};
+    if (valid) {
+        const long long f[3] = {a.F[p], a.F[p + 1], a.F[p + 2]};
+        const long long q[3] = {a.P[p], a.P[p + 1], a.P[p + 2]};
+        e = adaptive_pixel_error(f, q, a.n, a.s);
+        for (int c = 0; c < 3; ++c) { sum[c] = f[c] + q[c]; a.F[p + c] = sum[c]; a.P[p + c] = 0; }
+    }
+    for (int o = 16; o > 0; o >>= 1) e = fmaxf(e, __shfl_xor_sync(0xffffffffu, e, o));
+    const bool stop = a.last != 0u || e <= a.threshold;
+    if (valid && stop) {
+        const float inv = 1.0f / 4294967296.0f;
+        a.accum[p / 3] = make_float4((float)sum[0] * inv, (float)sum[1] * inv, (float)sum[2] * inv, (float)(a.n + a.s));
+    }
+    if (lane == 0) { a.tile_error[t] = e; a.keep[i] = stop ? 0u : 1u; }
+}
+
+// The next pass's tile list: the entries of `list` (NULL: 0 .. n) whose keep flag is set, in ascending order, so that the next
+// pass still schedules bottom rows first and is the same run to run.  One CTA: a few hundred thousand flags at most.
+constexpr int COMPACT_THREADS = 1024;
+__global__ void __launch_bounds__(COMPACT_THREADS) adaptive_compact_kernel(const uint32_t* list, const uint32_t* keep, uint32_t n,
+                                                                            uint32_t* out, uint32_t* out_count) {
+    __shared__ uint32_t warp_counts[COMPACT_THREADS / 32];
+    __shared__ uint32_t base;
+    const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
+    if (threadIdx.x == 0) base = 0;
+    __syncthreads();
+    for (uint32_t i0 = 0; i0 < n; i0 += COMPACT_THREADS) {
+        const uint32_t i = i0 + threadIdx.x;
+        const bool k = i < n && keep[i] != 0u;
+        const unsigned m = __ballot_sync(0xffffffffu, k);
+        if (lane == 0) warp_counts[w] = (uint32_t)__popc(m);
+        __syncthreads();
+        uint32_t at = base;
+        for (uint32_t v = 0; v < w; ++v) at += warp_counts[v];
+        if (k) out[at + (uint32_t)__popc(m & ((1u << lane) - 1u))] = list ? list[i] : i;
+        __syncthreads();
+        if (threadIdx.x == 0) { uint32_t total = 0; for (uint32_t v = 0; v < COMPACT_THREADS / 32; ++v) total += warp_counts[v]; base += total; }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *out_count = base;
 }
 
 }  // namespace b200rt
