@@ -279,6 +279,42 @@ int  b200rt_render_adaptive(const B200rtScene* scene, const B200rtCamera* camera
                             const B200rtRenderParams* params, const B200rtAdaptiveParams* adaptive,
                             float* accum, uint8_t* out_rgb8, float* tile_error, B200rtStats* stats);
 
+/* Denoised render: a low-sample frame reconstructed by an edge-avoiding à-trous wavelet filter (Dammertz et al. 2010) with
+ * SVGF's variance-guided luminance edge-stop (Schied et al. 2017), guided by features of the render's own primary rays.
+ * The n = params->samples samples are rendered as two halves, [0, h) and [h, n) with h = n / 2 (offset by sample_offset, same RNG
+ * keying as b200rt_render), into exact 64-bit fixed-point sums with the clamp taken for n.  So:
+ *   accum     H*W float4 {sum r,g,b, n}: the plain n-sample b200rt_render of the frame, bit for bit;
+ *   the halves are two independent means of every pixel.  The filter's per-pixel variance is their two-means estimate
+ *   (adaptive_pixel_error's, squared and before the gamma step).
+ * features  2*H*W float4, two planes, each summed over samples [0, feature_samples) of the render's own primary rays in sample
+ *           order in f32 and divided by feature_samples:
+ *             plane 0 (normal.xyz, depth)  the face-flipped normal of the first hit and t |d|; a miss adds 0
+ *             plane 1 (albedo.rgb, 0)      texture value (Lambertian, lights), albedo (Metal), (1,1,1) (Dielectric), background (miss)
+ * denoised  H*W float4 {mean * n, n}: the filtered frame in the accumulation layout, so b200rt_resolve_rgb8(.., samples = 0)
+ *           takes it unchanged.  It equals b200rt_denoise of plain renders of [0, h) and [h, n) and these features, as long as
+ *           no sample's channel exceeds 2e9 / n.  The formulas and constants are in csrc/denoise_plan.hpp.
+ * out_rgb8  the resolve of `denoised`.
+ * Every output may be NULL.  stats: rays and paths of the two halves, kernel_ms = their path-tracing kernel times, total_ms and
+ * launches for the whole call.
+ * params: seed, max_depth, sample_offset, device and COUNT_TRAVERSAL as for b200rt_render.  samples < 2, feature_samples of 0 or
+ * above samples, iterations outside 1..5, ACCUMULATE, a row range other than the whole frame, shard_count > 1 and a NULL scene,
+ * camera, params or denoise return B200RT_EINVAL: the filter needs every neighbour. */
+typedef struct B200rtDenoiseParams {
+    uint32_t feature_samples;   /* primary rays per pixel of the feature pass, 1..samples */
+    uint32_t iterations;        /* à-trous passes (steps 1, 2, 4, ...), 1..5 */
+    uint32_t _pad[2];
+} B200rtDenoiseParams;
+
+int  b200rt_render_denoised(const B200rtScene* scene, const B200rtCamera* camera,
+                            const B200rtRenderParams* params, const B200rtDenoiseParams* denoise,
+                            float* accum, float* denoised, float* features, uint8_t* out_rgb8, B200rtStats* stats);
+
+/* The filter of b200rt_render_denoised alone, on host buffers: accum_a and accum_b are two independent H*W float4 accumulation
+ * buffers of the same pixels ({sum r,g,b, count}: the counts are taken from .w), `features` the 2*H*W float4 planes described
+ * above.  `out` (H*W float4) receives {mean * n, n} with n = the two counts' sum.  `device` -1 = current. */
+int  b200rt_denoise(const float* accum_a, const float* accum_b, const float* features, uint32_t width, uint32_t height,
+                    uint32_t iterations, float* out, int device);
+
 /* render_scene on SEVERAL GPUs from one host process: `params->samples` is the total per pixel, split into
  * contiguous sample ranges over `devices[0 .. n_devices)` (each gets its own copy of the scene, uploaded by its
  * own host thread); devices[0] sums the per-device buffers inside the resolve through peer access and returns

@@ -96,6 +96,10 @@ class AdaptiveParams(C.Structure):
     _fields_ = [("initial_samples", C.c_uint32), ("max_samples", C.c_uint32), ("threshold", C.c_float), ("_pad", C.c_uint32)]
 
 
+class DenoiseParams(C.Structure):
+    _fields_ = [("feature_samples", C.c_uint32), ("iterations", C.c_uint32), ("_pad", C.c_uint32 * 2)]
+
+
 class SceneInfo(C.Structure):
     _fields_ = [("n_prims", C.c_uint32), ("n_bvh_nodes", C.c_uint32), ("bvh_depth", C.c_uint32),
                 ("bvh_nodes_in_smem", C.c_uint32), ("device_bytes", C.c_uint64), ("bvh_build_ms", C.c_float), ("bvh_builder", C.c_uint32)]
@@ -129,6 +133,9 @@ SIGNATURES = {
     "b200rt_render_rgb8": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p, _P(Stats)]),
     "b200rt_render_adaptive": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), _P(AdaptiveParams), C.c_void_p, C.c_void_p,
                                          C.c_void_p, _P(Stats)]),
+    "b200rt_render_denoised": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), _P(DenoiseParams), C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_void_p, _P(Stats)]),
+    "b200rt_denoise": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_int]),
     "b200rt_render_rgb8_multi": (C.c_int, [_P(SceneDesc), _P(C.c_int), C.c_uint32, _P(Camera), _P(RenderParams), C.c_void_p, _P(Stats)]),
     "b200rt_render_device": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p]),
     "b200rt_render_device_finish": (C.c_int, [C.c_void_p, C.c_void_p, _P(Stats)]),

@@ -354,6 +354,39 @@ def render_adaptive(scene: Scene, cam: F.Camera, max_samples: int, threshold: fl
     return accum, tile_error, st
 
 
+def render_denoised(scene: Scene, cam: F.Camera, samples: int, feature_samples: int = 4, iterations: int = 5, max_depth: int = 50,
+                    seed: int = 0, *, sample_offset: int = 0, count_traversal: bool = False, device: int = -1):
+    """A `samples`-spp frame reconstructed by the feature-guided à-trous filter (b200rt_render_denoised).  Returns
+    (denoised[H, W, 4] float32 {mean * n, n}, accum[H, W, 4] float32 (the plain `samples`-spp render, bit for bit),
+    features[2, H, W, 4] float32 (plane 0: mean normal xyz and hit distance, plane 1: mean albedo and 0), Stats).
+    resolve_rgb8(denoised, samples=0) gives the picture."""
+    H, W = cam.image_height, cam.image_width
+    denoised = np.empty((H, W, 4), dtype=np.float32)
+    accum = np.empty((H, W, 4), dtype=np.float32)
+    features = np.empty((2, H, W, 4), dtype=np.float32)
+    p = F.RenderParams(samples=samples, sample_offset=sample_offset, max_depth=max_depth,
+                       flags=F.FLAG_COUNT_TRAVERSAL if count_traversal else 0, seed=seed, device=-1)
+    dn = F.DenoiseParams(feature_samples=feature_samples, iterations=iterations)
+    st = F.Stats()
+    F.check(lib.b200rt_render_denoised(scene.device(device), C.byref(cam), C.byref(p), C.byref(dn), accum.ctypes.data,
+                                       denoised.ctypes.data, features.ctypes.data, None, C.byref(st)))
+    return denoised, accum, features, st
+
+
+def denoise(accum_a: np.ndarray, accum_b: np.ndarray, features: np.ndarray, iterations: int = 5, device: int = -1) -> np.ndarray:
+    """The filter of render_denoised alone (b200rt_denoise): two independent accumulation buffers of the same pixels
+    ([H, W, 4] {sum r,g,b, count}) and their features ([2, H, W, 4]) -> [H, W, 4] float32 {mean * n, n}."""
+    a = np.ascontiguousarray(accum_a, dtype=np.float32)
+    b = np.ascontiguousarray(accum_b, dtype=np.float32)
+    f = np.ascontiguousarray(features, dtype=np.float32)
+    H, W = a.shape[:2]
+    if a.shape != (H, W, 4) or b.shape != (H, W, 4) or f.shape != (2, H, W, 4):
+        raise ValueError("accum_a and accum_b must be (H, W, 4) and features (2, H, W, 4)")
+    out = np.empty((H, W, 4), dtype=np.float32)
+    F.check(lib.b200rt_denoise(a.ctypes.data, b.ctypes.data, f.ctypes.data, W, H, iterations, out.ctypes.data, device))
+    return out
+
+
 def resolve_rgb8(accum: np.ndarray, samples: int = 0, device: int = -1) -> np.ndarray:
     """to_image's pixel loop (image.rs:34-40): mean, sqrt gamma, saturating u8, vertical flip."""
     accum = np.ascontiguousarray(accum, dtype=np.float32)

@@ -38,6 +38,8 @@ struct Args {
     int gpus = 1;               // extra: render on the first N GPUs of this box (one process, peer access)
     double adaptive = -1.0;     // extra: tile-adaptive sampling to this standard error in 8-bit levels (< 0: off); --samples is the maximum
     uint32_t adaptive_initial = 16;
+    bool denoise = false;       // extra: reconstruct the frame with the feature-guided à-trous denoiser
+    uint32_t denoise_features = 0;   // 0: the default, min(4, samples)
 };
 
 [[noreturn]] void usage(const char* msg) {
@@ -63,7 +65,9 @@ struct Args {
             "                                   --samples more samples are added (same scene, camera and seed required)\n"
             "      --adaptive <LEVELS>          tile-adaptive sampling: render each 8x4 tile until its estimated standard error\n"
             "                                   is at most LEVELS 8-bit levels; --samples becomes the maximum per pixel\n"
-            "      --adaptive-initial <N>       samples of the first adaptive pass [default: 16]\n");
+            "      --adaptive-initial <N>       samples of the first adaptive pass [default: 16]\n"
+            "      --denoise                    write the frame denoised by the feature-guided a-trous filter (needs -s >= 2)\n"
+            "      --denoise-features <N>       primary rays per pixel of the denoiser's feature pass, 1..samples [default: 4]\n");
     exit(msg ? 2 : 0);
 }
 
@@ -106,11 +110,19 @@ Args parse(int argc, char** argv) {
             if (v.empty() || *end || !std::isfinite(a.adaptive) || a.adaptive < 0) usage("--adaptive needs a finite number of levels >= 0");
         }
         else if (s == "--adaptive-initial") { int n = atoi(need("--adaptive-initial").c_str()); if (n < 1) usage("--adaptive-initial needs a positive count"); a.adaptive_initial = (uint32_t)n; }
+        else if (s == "--denoise") a.denoise = true;
+        else if (s == "--denoise-features") { int n = atoi(need("--denoise-features").c_str()); if (n < 1) usage("--denoise-features needs a positive count"); a.denoise_features = (uint32_t)n; }
         else if (!s.empty() && s[0] == '-') usage(("unexpected argument " + s).c_str());
         else pos.push_back(s);
     }
     if (a.adaptive >= 0 && a.gpus > 1) usage("--adaptive renders on one GPU: it cannot be combined with --gpus");
     if (a.adaptive >= 0 && !a.checkpoint.empty()) usage("--adaptive cannot be combined with --checkpoint");
+    if (a.denoise && a.adaptive >= 0) usage("--denoise cannot be combined with --adaptive");
+    if (a.denoise && a.gpus > 1) usage("--denoise renders on one GPU: it cannot be combined with --gpus");
+    if (a.denoise && !a.checkpoint.empty()) usage("--denoise cannot be combined with --checkpoint");
+    if (a.denoise && a.samples < 2) usage("--denoise needs at least 2 samples per pixel");
+    if (a.denoise && a.denoise_features > a.samples) usage("--denoise-features cannot exceed --samples");
+    if (a.denoise_features == 0) a.denoise_features = (uint32_t)std::min<size_t>(4, a.samples);
     if (pos.empty()) usage("a subcommand is required");
     if (pos[0] == "test") { a.sub = "test"; return a; }
     if (pos[0] != "render" || pos.size() < 2) usage("expected `render <scene>`");
@@ -162,6 +174,10 @@ int render_scene(const Args& args, const scene::SceneBuilder& builder, const cam
             fprintf(stderr, " INFO  adaptive to %g levels: %.1f spp on average (at most %zu), %u passes\n", args.adaptive,
                     (double)st.paths / ((double)c.image_width * c.image_height), samples, passes);
         }
+    } else if (args.denoise) {
+        B200rtDenoiseParams dn{};
+        dn.feature_samples = args.denoise_features; dn.iterations = 5;
+        rc = b200rt_render_denoised(dev, &c, &p, &dn, nullptr, nullptr, nullptr, rgb.data(), &st);
     } else if (args.checkpoint.empty()) {
         rc = b200rt_render_rgb8(dev, &c, &p, rgb.data(), nullptr, &st);
     } else {

@@ -10,6 +10,8 @@
 //   bvh_build.hpp        host binned-SAH builder
 //   launch_plan.hpp      CTA size, shared-memory plan, sample-range schedule and grid of a launch (pure host arithmetic)
 //   adaptive_plan.hpp    pass schedule and error estimate of tile-adaptive sampling (host and device)
+//   denoise_kernels.cuh  feature pass (first hits of the render's primary rays) and the à-trous filter of b200rt_render_denoised
+//   denoise_plan.hpp     the filter's weights and variance (host and device)
 // No tensor cores: nothing on this path is a dense contraction.  No CPU fallback.
 #include <cuda_runtime.h>
 
@@ -55,6 +57,7 @@ static int fail(int code, const char* fmt, ...) {
 
 #include "render_kernel.cuh"
 #include "aux_kernels.cuh"
+#include "denoise_kernels.cuh"
 
 
 // ==========================================================================================
@@ -75,6 +78,7 @@ struct Scratch {                     // per in-flight render: counters, events, 
     long long* d_fix = nullptr; size_t fix_bytes = 0;  // fixed-point sums of a launch whose tiles are split into sample chunks (adaptive: F)
     long long* d_pass = nullptr; size_t pass_bytes = 0;  // adaptive: the fixed-point sums of one pass (P)
     uint32_t* d_tiles = nullptr; size_t tiles_bytes = 0;  // adaptive: two tile lists, keep flags, tile errors, the active count
+    float4* d_denoise = nullptr; size_t denoise_bytes = 0;  // denoised renders: the two halves, the features, the filter's two buffers
     uint32_t launches = 0;
 };
 
@@ -143,6 +147,9 @@ SceneSize scene_size(const B200rtScene* sc) { return {sc->ds.n_nodes, sc->ds.n_p
 // `max_origin` is the largest |coordinate| of a ray origin.  B200RT_FAST_SLAB=0 forces the exact Aabb::hit2 arithmetic.
 bool use_fast_slab(const B200rtScene* sc, float max_origin) {
     return sc->box_pad >= 4.0f * 1.1920929e-7f * std::max(sc->max_abs_coord, max_origin) && env_int("B200RT_FAST_SLAB", 1) != 0;
+}
+bool use_fast_slab(const B200rtScene* sc, const B200rtCamera* cam) {
+    return use_fast_slab(sc, std::max(std::fabs((float)cam->origin[0]), std::max(std::fabs((float)cam->origin[1]), std::fabs((float)cam->origin[2]))));
 }
 
 int resolve_device(int device, int* out) {
@@ -326,7 +333,7 @@ int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderPa
     // New paths are handed out only when >= 6 lanes are free (the hand-out block then runs at >= 6 lanes instead of ~5 every
     // iteration): 14.66 -> 15.0 Grays/s on the bench frame, +5 % on the earth frame, 4..8 within 0.5 % of each other.
     a.regen_min = (uint32_t)std::min(32, std::max(1, env_int("B200RT_REGEN_MIN", 6)));
-    const bool fast = use_fast_slab(sc, std::max(std::fabs((float)cam->origin[0]), std::max(std::fabs((float)cam->origin[1]), std::fabs((float)cam->origin[2]))));
+    const bool fast = use_fast_slab(sc, cam);
     const auto [block_threads, plan] = render_shape(scene_size(sc), sc->smem_optin);
     a.plan = plan;
     RenderKernel kernel = render_kernel(plan.all_in_smem, block_threads, fast, count);
@@ -390,6 +397,55 @@ int finish_render(Scratch* scr, cudaStream_t stream, cudaEvent_t end_event, B200
         CU(cudaEventElapsedTime(&ms, scr->ev0, end_event)); stats->total_ms = ms;
         stats->launches = scr->launches;
     }
+    return B200RT_OK;
+}
+
+// The feature pass of b200rt_render_denoised: one kernel per (accessor, slab form), shaped like the render launch (its CTA size
+// and shared-memory plan: the staged scene and the stack columns), persistent over the frame.
+using FeatureKernel = void (*)(FeatureArgs);
+FeatureKernel feature_kernel(bool all_in_smem, bool fast) {
+    if (all_in_smem) return fast ? denoise_feature_kernel<SmemAcc, true> : denoise_feature_kernel<SmemAcc, false>;
+    return fast ? denoise_feature_kernel<GmemAcc, true> : denoise_feature_kernel<GmemAcc, false>;
+}
+
+int launch_features(B200rtScene* sc, const B200rtCamera* cam, uint64_t seed, uint32_t sample_offset, uint32_t k, float4* d_feat,
+                    cudaStream_t stream, uint32_t* launches) {
+    const auto [block_threads, plan] = render_shape(scene_size(sc), sc->smem_optin);
+    FeatureKernel kernel = feature_kernel(plan.all_in_smem, use_fast_slab(sc, cam));
+    FeatureArgs f{};
+    f.scene = sc->ds; f.cam = make_camera(*cam); f.plan = plan; f.keys = rng_keys(seed);
+    f.sample_offset = sample_offset; f.k = k; f.feat = d_feat;
+    int rc = set_smem(kernel, sc, plan.bytes); if (rc) return rc;
+    int blocks_per_sm = 0;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kernel, block_threads, plan.bytes));
+    if (blocks_per_sm < 1) return fail(B200RT_ECUDA, "feature kernel does not fit on an SM (smem %u B, %u threads)", plan.bytes, block_threads);
+    const uint64_t px = (uint64_t)cam->image_width * cam->image_height;
+    const uint32_t grid = (uint32_t)std::min<uint64_t>((px + block_threads - 1) / block_threads, (uint64_t)sc->sm_count * blocks_per_sm);
+    kernel<<<grid, block_threads, plan.bytes, stream>>>(f);
+    CU(cudaGetLastError());
+    *launches += 1;
+    return B200RT_OK;
+}
+
+// The filter on device buffers (denoise_plan.hpp): demodulation and variance into X0, then `iterations` à-trous passes between
+// X0 and X1, the last one remodulating.  *out = the buffer holding the result, {mean * n, n} per pixel.
+int launch_filter(const float4* d_a, const float4* d_b, const float4* d_feat, uint32_t W, uint32_t H, uint32_t iterations,
+                  float4* x0, float4* x1, cudaStream_t stream, float4** out, uint32_t* launches) {
+    FilterArgs f{};
+    f.acc_a = d_a; f.acc_b = d_b; f.feat = d_feat; f.W = W; f.H = H;
+    const dim3 block(32, 8), grid((W + 31) / 32, (H + 7) / 8);
+    f.x_out = x0;
+    denoise_demodulate_kernel<<<grid, block, 0, stream>>>(f);
+    CU(cudaGetLastError());
+    float4* buf[2] = {x0, x1};
+    for (uint32_t i = 0; i < iterations; ++i) {
+        f.x_in = buf[i & 1u]; f.x_out = buf[(i + 1u) & 1u];
+        f.step = 1u << i; f.last = i + 1 == iterations ? 1u : 0u;
+        denoise_atrous_kernel<<<grid, block, 0, stream>>>(f);
+        CU(cudaGetLastError());
+    }
+    *launches += 1 + iterations;
+    *out = buf[iterations & 1u];
     return B200RT_OK;
 }
 
@@ -874,6 +930,135 @@ int b200rt_render_adaptive(const B200rtScene* csc, const B200rtCamera* cam, cons
     scr->launched = false;
     put_scratch(sc, key);
     return rc;
+}
+
+// Denoised render (b200rt_render_denoised): the two halves [0, h) and [h, n) as two K2 launches into the fixed-point buffers
+// F and P (the adaptive pass mechanism over all tiles, clamp taken for n), their float4 forms and the whole render's, the
+// feature pass, the filter, the optional resolve and the copies.
+static int render_denoised_impl(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderParams* prm, const B200rtDenoiseParams* dn,
+                                float* accum, float* denoised, float* features, uint8_t* out_rgb8, B200rtStats* stats, Scratch* scr) {
+    const uint32_t W = cam->image_width, H = cam->image_height;
+    const uint32_t n = prm->samples, h = n / 2;
+    const uint32_t n_tiles = ((W + TILE_W - 1) / TILE_W) * ((H + TILE_H - 1) / TILE_H);
+    const size_t px = (size_t)W * H;
+    cudaError_t e = grow(scr->d_accum, scr->accum_bytes, px * sizeof(float4));
+    if (e == cudaSuccess) e = grow(scr->d_fix, scr->fix_bytes, px * 3 * sizeof(long long));
+    if (e == cudaSuccess) e = grow(scr->d_pass, scr->pass_bytes, px * 3 * sizeof(long long));
+    if (e == cudaSuccess) e = grow(scr->d_denoise, scr->denoise_bytes, px * 6 * sizeof(float4));
+    if (e == cudaSuccess && out_rgb8) e = grow(scr->d_rgb, scr->rgb_bytes, px * 3);
+    if (e != cudaSuccess) return fail(B200RT_ENOMEM, "denoising buffers (%zu px): %s", px, cudaGetErrorString(e));
+    float4* d_a = scr->d_denoise;
+    float4* d_b = d_a + px;
+    float4* d_feat = d_b + px;          // two planes
+    float4* x0 = d_feat + 2 * px;
+    float4* x1 = x0 + px;
+    cudaStream_t stream = scr->own_stream;
+    // ev3 marks the start of the call; launch_render records ev0..ev2 per half, and ev0 is recorded again to mark the end
+    CU(cudaEventRecord(scr->ev3, stream));
+    CU(cudaMemsetAsync(scr->d_fix, 0, px * 3 * sizeof(long long), stream));
+    CU(cudaMemsetAsync(scr->d_pass, 0, px * 3 * sizeof(long long), stream));
+    B200rtRenderParams p = *prm;
+    p.flags &= B200RT_FLAG_COUNT_TRAVERSAL; p.shard_count = 1; p.shard_index = 0; p.row_begin = 0; p.row_end = H;
+    B200rtStats sum{};
+    uint32_t launches = 0;
+    for (uint32_t half = 0; half < 2; ++half) {
+        p.samples = half ? n - h : h; p.sample_offset = prm->sample_offset + (half ? h : 0u);
+        const AdaptivePass pass{nullptr, n_tiles, half ? scr->d_pass : scr->d_fix, n};
+        if (int rc = launch_render(sc, cam, &p, reinterpret_cast<float*>(scr->d_accum), stream, scr, &pass)) return rc;
+        launches += scr->launches;
+        CU(cudaStreamSynchronize(stream));   // the counters and events of this half
+        const Counters& c = *scr->h_counters;
+        sum.rays += c.rays; sum.paths += c.paths; sum.node_visits += c.nodes; sum.prim_tests += c.prims; sum.depth_exhausted += c.exhausted;
+        for (int d = 0; d < 8; ++d) sum.diag[d] += c.diag[d];
+        float ms = 0.f;
+        CU(cudaEventElapsedTime(&ms, scr->ev1, scr->ev2)); sum.kernel_ms += ms;
+    }
+    denoise_halves_kernel<<<(unsigned)((px + 255) / 256), 256, 0, stream>>>(scr->d_fix, scr->d_pass, (uint32_t)px, h, n - h, d_a, d_b, scr->d_accum);
+    CU(cudaGetLastError());
+    launches += 1;
+    if (int rc = launch_features(sc, cam, prm->seed, prm->sample_offset, dn->feature_samples, d_feat, stream, &launches)) return rc;
+    float4* d_out = nullptr;
+    if (int rc = launch_filter(d_a, d_b, d_feat, W, H, dn->iterations, x0, x1, stream, &d_out, &launches)) return rc;
+    if (out_rgb8) {
+        if (int rc = b200rt_resolve_rgb8_device(reinterpret_cast<float*>(d_out), W, H, 0, scr->d_rgb, stream)) return rc;
+        launches += 1;
+        e = cudaMemcpyAsync(out_rgb8, scr->d_rgb, px * 3, cudaMemcpyDeviceToHost, stream);
+    }
+    if (e == cudaSuccess && accum) e = cudaMemcpyAsync(accum, scr->d_accum, px * sizeof(float4), cudaMemcpyDeviceToHost, stream);
+    if (e == cudaSuccess && denoised) e = cudaMemcpyAsync(denoised, d_out, px * sizeof(float4), cudaMemcpyDeviceToHost, stream);
+    if (e == cudaSuccess && features) e = cudaMemcpyAsync(features, d_feat, 2 * px * sizeof(float4), cudaMemcpyDeviceToHost, stream);
+    if (e == cudaSuccess) e = cudaEventRecord(scr->ev0, stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+    if (e != cudaSuccess) return fail(B200RT_ECUDA, "denoised render: %s", cudaGetErrorString(e));
+    if (stats) {
+        float ms = 0.f;
+        CU(cudaEventElapsedTime(&ms, scr->ev3, scr->ev0));
+        sum.total_ms = ms;
+        sum.launches = launches;
+        *stats = sum;
+    }
+    return B200RT_OK;
+}
+
+int b200rt_render_denoised(const B200rtScene* csc, const B200rtCamera* cam, const B200rtRenderParams* prm, const B200rtDenoiseParams* dn,
+                           float* accum, float* denoised, float* features, uint8_t* out_rgb8, B200rtStats* stats) {
+    if (!csc || !cam || !prm || !dn) return fail(B200RT_EINVAL, "NULL argument");
+    if (prm->samples < 2) return fail(B200RT_EINVAL, "denoising needs at least 2 samples (two independent halves), got %u", prm->samples);
+    if (dn->feature_samples == 0 || dn->feature_samples > prm->samples)
+        return fail(B200RT_EINVAL, "feature_samples %u must be in 1..samples (%u)", dn->feature_samples, prm->samples);
+    if (dn->iterations < 1 || dn->iterations > (uint32_t)DN_MAX_ITERATIONS)
+        return fail(B200RT_EINVAL, "iterations %u outside 1..%d", dn->iterations, DN_MAX_ITERATIONS);
+    if (prm->flags & B200RT_FLAG_ACCUMULATE) return fail(B200RT_EINVAL, "a denoised render cannot add to an earlier result (B200RT_FLAG_ACCUMULATE)");
+    if (prm->shard_count > 1) return fail(B200RT_EINVAL, "the denoiser needs every neighbour: shard_count %u is not supported", prm->shard_count);
+    B200rtScene* sc = const_cast<B200rtScene*>(csc);
+    if (prm->device >= 0 && prm->device != sc->device) return fail(B200RT_EINVAL, "params.device %d != scene device %d", prm->device, sc->device);
+    const uint32_t W = cam->image_width, H = cam->image_height;
+    if (W == 0 || H == 0) return fail(B200RT_EINVAL, "camera image dimensions are zero");
+    if ((uint64_t)W * H > 0xFFFFFFFFull) return fail(B200RT_EINVAL, "image too large");
+    if (!(prm->row_begin == 0 && (prm->row_end == 0 || prm->row_end == H)))
+        return fail(B200RT_EINVAL, "the denoiser needs every neighbour: row range [%u,%u) is not the whole frame of %u rows", prm->row_begin, prm->row_end, H);
+
+    DeviceGuard guard(sc->device);
+    int key_local; void* key = &key_local;   // private key: concurrent host threads never collide
+    Scratch* scr; int rc = get_scratch(sc, key, &scr); if (rc) return rc;
+    rc = render_denoised_impl(sc, cam, prm, dn, accum, denoised, features, out_rgb8, stats, scr);
+    if (rc) cudaStreamSynchronize(scr->own_stream);   // nothing of a failed call may still run when its scratch is reused
+    scr->launched = false;
+    put_scratch(sc, key);
+    return rc;
+}
+
+int b200rt_denoise(const float* accum_a, const float* accum_b, const float* features, uint32_t W, uint32_t H, uint32_t iterations,
+                   float* out, int device) {
+    if (!accum_a || !accum_b || !features || !out) return fail(B200RT_EINVAL, "NULL argument");
+    if (W == 0 || H == 0) return fail(B200RT_EINVAL, "image dimensions are zero");
+    if ((uint64_t)W * H > 0xFFFFFFFFull) return fail(B200RT_EINVAL, "image too large");
+    if (iterations < 1 || iterations > (uint32_t)DN_MAX_ITERATIONS) return fail(B200RT_EINVAL, "iterations %u outside 1..%d", iterations, DN_MAX_ITERATIONS);
+    int rc = resolve_device(device, &device); if (rc) return rc;
+    DeviceGuard guard(device);
+    const size_t px = (size_t)W * H;
+    DevBuf buf;
+    if ((rc = buf.alloc(px * 6 * sizeof(float4)))) return rc;
+    float4* d_a = buf.as<float4>();
+    float4* d_b = d_a + px;
+    float4* d_feat = d_b + px;
+    float4* x0 = d_feat + 2 * px;
+    float4* x1 = x0 + px;
+    cudaStream_t stream = nullptr;
+    CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    cudaError_t e = cudaMemcpyAsync(d_a, accum_a, px * sizeof(float4), cudaMemcpyHostToDevice, stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_b, accum_b, px * sizeof(float4), cudaMemcpyHostToDevice, stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_feat, features, 2 * px * sizeof(float4), cudaMemcpyHostToDevice, stream);
+    float4* d_out = nullptr;
+    uint32_t launches = 0;
+    if (e == cudaSuccess) rc = launch_filter(d_a, d_b, d_feat, W, H, iterations, x0, x1, stream, &d_out, &launches);
+    if (e == cudaSuccess && rc == B200RT_OK) e = cudaMemcpyAsync(out, d_out, px * sizeof(float4), cudaMemcpyDeviceToHost, stream);
+    const cudaError_t es = cudaStreamSynchronize(stream);
+    cudaStreamDestroy(stream);
+    if (rc) return rc;
+    if (e == cudaSuccess) e = es;
+    if (e != cudaSuccess) return fail(B200RT_ECUDA, "denoise: %s", cudaGetErrorString(e));
+    return B200RT_OK;
 }
 
 // ---- render_scene on several GPUs from ONE host process (what a `ray-cli` user has) -------------------------------
