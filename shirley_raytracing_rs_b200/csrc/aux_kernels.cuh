@@ -78,7 +78,7 @@ __global__ void __launch_bounds__(BLOCK) closest_hit_kernel(const __grid_constan
                 ray.o = f3(in.ox, in.oy, in.oz); ray.d = f3(in.dx, in.dy, in.dz);
                 float3 inv_e = f3(__frcp_rn(ray.d.x), __frcp_rn(ray.d.y), __frcp_rn(ray.d.z));
                 ray.inv = FAST ? f3(clamp_inv(inv_e.x), clamp_inv(inv_e.y), clamp_inv(inv_e.z)) : inv_e;
-                ray.ood = f3(ray.o.x * ray.inv.x, ray.o.y * ray.inv.y, ray.o.z * ray.inv.z);
+                ray.nood = f3(-(ray.o.x * ray.inv.x), -(ray.o.y * ray.inv.y), -(ray.o.z * ray.inv.z));
                 c.t = a.t_max; c.code = -1;
 #pragma unroll 1
                 for (uint32_t k = 0; k < a.scene.n_top_prims; ++k) {

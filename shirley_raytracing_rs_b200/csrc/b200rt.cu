@@ -597,29 +597,16 @@ int b200rt_scene_create(const B200rtSceneDesc* d, int device, B200rtScene** out)
     }
 
     static_assert(sizeof(HostNode) == sizeof(BvhNode), "node layout");
-    // The device's copy of the tree: each child box as centre + half-extent (rt_device.cuh: aabb_center),
-    // re-derived outwards from the builder's (lo, hi): c = (lo+hi)/2, h = max(hi - c, c - lo) bumped up one ulp,
-    // so [c - h, c + h] contains [lo, hi].  An empty child (lo > hi) gets h = -1: near > far on every axis, never
-    // entered.  ONE copy is uploaded; the exact-slab fallback derives (c - h, c + h) on the fly.
+    // The device's copy of the tree: the builder's (lo, hi) child boxes packed as centre + half-extent pairs
+    // (node_layout.hpp).  ONE copy is uploaded; the exact-slab fallback derives (c - h, c + h) on the fly.
     auto centre_form = [](const std::vector<HostNode>& src) {
         std::vector<BvhNode> out(src.size());
 #pragma omp parallel for schedule(static) if (src.size() >= 65536)
         for (long long i = 0; i < (long long)src.size(); ++i) {
-            const float* q = reinterpret_cast<const float*>(&src[i]);
-            float* o = reinterpret_cast<float*>(&out[i]);
-            for (int ch = 0; ch < 2; ++ch) {
-                const float* lo = q + 6 * ch; const float* hi = lo + 3;
-                for (int k = 0; k < 3; ++k) {
-                    float c = 0.f, h = -1.f;
-                    if (lo[k] <= hi[k]) {
-                        c = 0.5f * lo[k] + 0.5f * hi[k];
-                        h = std::nextafterf(std::max(hi[k] - c, c - lo[k]), INFINITY);
-                        if (!std::isfinite(c) || !std::isfinite(h)) { c = 0.f; h = 3.0e38f; }   // unbounded box: always entered
-                    }
-                    o[6 * ch + k] = c; o[6 * ch + 3 + k] = h;
-                }
-            }
-            o[12] = q[12]; o[13] = q[13]; o[14] = q[14]; o[15] = q[15];
+            const float* q = src[i].q;
+            int ref0, ref1;
+            memcpy(&ref0, &q[12], 4); memcpy(&ref1, &q[13], 4);
+            pack_node(q, q + 3, q + 6, q + 9, ref0, ref1, reinterpret_cast<float*>(&out[i]));
         }
         return out;
     };

@@ -56,7 +56,7 @@ __global__ void __launch_bounds__(768, 1) denoise_feature_kernel(const __grid_co
             if (in_range) {
                 float3 inv_e = f3(__frcp_rn(ray.d.x), __frcp_rn(ray.d.y), __frcp_rn(ray.d.z));
                 ray.inv = FAST ? f3(clamp_inv(inv_e.x), clamp_inv(inv_e.y), clamp_inv(inv_e.z)) : inv_e;
-                ray.ood = f3(ray.o.x * ray.inv.x, ray.o.y * ray.inv.y, ray.o.z * ray.inv.z);
+                ray.nood = f3(-(ray.o.x * ray.inv.x), -(ray.o.y * ray.inv.y), -(ray.o.z * ray.inv.z));
 #pragma unroll 1
                 for (uint32_t t = 0; t < a.scene.n_top_prims; ++t) hit_leaf(ray, acc, a.scene.top_prims[t], T_MIN, c, &inv_e);
                 node = 0;

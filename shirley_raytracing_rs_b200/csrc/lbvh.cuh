@@ -10,8 +10,7 @@
 //   3. one thread per internal node finds its key range and split -> children, parents
 //   4. bottom-up refit: the second thread to arrive at a node (atomic counter) joins its
 //      children's boxes and depths and climbs on
-//   5. one thread per internal node emits the 64-byte traversal node in both forms the
-//      kernels read (children's boxes as lo/hi and as centre/half-extent)
+//   5. one thread per internal node emits the 64-byte traversal node (node_layout.hpp: pack_node)
 // Closest-hit results do not depend on the tree (ties are resolved by hit id), so parity is
 // unaffected; on the config-4 scene the tree costs 2 % more node visits than the SAH one (profiles/).
 #pragma once
@@ -116,12 +115,6 @@ __global__ void refit_kernel(const PrimBox* __restrict__ prims, const uint32_t* 
     }
 }
 
-__device__ __forceinline__ void to_center(float lo, float hi, float* c, float* h) {
-    *c = 0.5f * lo + 0.5f * hi;
-    *h = nextafterf(fmaxf(hi - *c, *c - lo), INFINITY);
-    if (!isfinite(*c) || !isfinite(*h)) { *c = 0.f; *h = 3.0e38f; }
-}
-
 __global__ void emit_kernel(const PrimBox* __restrict__ prims, const uint32_t* __restrict__ order, int n, const int2* __restrict__ children,
                             const SubBox* __restrict__ sub, BvhNode* nodes) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -132,13 +125,10 @@ __global__ void emit_kernel(const PrimBox* __restrict__ prims, const uint32_t* _
     child_box(c.y, prims, order, sub, l1, h1, &d1);
     int r0 = c.x >= 0 ? c.x : ~__float_as_int(prims[order[~c.x]].lo.w);   // leaf: ~((type << 28) | id)
     int r1 = c.y >= 0 ? c.y : ~__float_as_int(prims[order[~c.y]].lo.w);
-    BvhNode q;
-    q.q3 = make_float4(__int_as_float(r0), __int_as_float(r1), 0.f, 0.f);
-    float cc0[3], hh0[3], cc1[3], hh1[3];
-    for (int k = 0; k < 3; ++k) { to_center(l0[k], h0[k], &cc0[k], &hh0[k]); to_center(l1[k], h1[k], &cc1[k], &hh1[k]); }
-    q.q0 = make_float4(cc0[0], cc0[1], cc0[2], hh0[0]); q.q1 = make_float4(hh0[1], hh0[2], cc1[0], cc1[1]);
-    q.q2 = make_float4(cc1[2], hh1[0], hh1[1], hh1[2]);
-    nodes[i] = q;
+    float q[16];
+    pack_node(l0, h0, l1, h1, r0, r1, q);
+    nodes[i] = BvhNode{make_float4(q[0], q[1], q[2], q[3]), make_float4(q[4], q[5], q[6], q[7]), make_float4(q[8], q[9], q[10], q[11]),
+                       make_float4(q[12], q[13], q[14], q[15])};
 }
 
 // Builds the tree of `prims` (host array, boxes already padded; at least 2 entries) into

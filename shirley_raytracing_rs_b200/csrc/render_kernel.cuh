@@ -313,7 +313,7 @@ __global__ void __launch_bounds__(BLK, 1) path_trace_kernel_v2(const __grid_cons
                 // (bit-reproducible on the CPU), and the slab tests take them too
                 float3 inv_e = f3(__frcp_rn(ray.d.x), __frcp_rn(ray.d.y), __frcp_rn(ray.d.z));
                 ray.inv = FAST ? f3(clamp_inv(inv_e.x), clamp_inv(inv_e.y), clamp_inv(inv_e.z)) : inv_e;
-                ray.ood = f3(ray.o.x * ray.inv.x, ray.o.y * ray.inv.y, ray.o.z * ray.inv.z);
+                ray.nood = f3(-(ray.o.x * ray.inv.x), -(ray.o.y * ray.inv.y), -(ray.o.z * ray.inv.z));
                 c.t = INFINITY; c.code = -1;
                 // the list is indexed in the kernel parameters (constant bank): a register copy indexed by a
                 // loop counter would live in local memory

@@ -7,6 +7,7 @@
 
 #include "../../include/b200rt.h"
 #include "launch_plan.hpp"
+#include "node_layout.hpp"
 
 namespace b200rt {
 
@@ -14,10 +15,11 @@ namespace b200rt {
 // Device scene layout (all arrays 16-byte aligned, read-only during a launch)
 // ------------------------------------------------------------------------------------------
 // BVH2 inner node, 64 B = 4 x float4 (one 16-byte vector load each); each child box is stored as
-// centre c and half-extent h (the three-FMA slab test below), rounded outwards from (lo, hi):
-//   q0 = (c0.c.x, c0.c.y, c0.c.z, c0.h.x)
-//   q1 = (c0.h.y, c0.h.z, c1.c.x, c1.c.y)
-//   q2 = (c1.c.z, c1.h.x, c1.h.y, c1.h.z)
+// centre c and half-extent h (the three-FMA slab test below), rounded outwards from (lo, hi), and
+// each component as a (child 0, child 1) pair for the packed slab test (node_layout.hpp):
+//   q0 = (c0.x, c1.x, c0.y, c1.y)
+//   q1 = (c0.z, c1.z, h0.x, h1.x)
+//   q2 = (h0.y, h1.y, h0.z, h1.z)
 //   q3 = (bits(child0), bits(child1), 0, 0)
 // child >= 0: inner-node index; child < 0: leaf, ~child = (prim_type << 28) | hit_id.
 // An empty child has h = -1 (never entered), an unbounded one c = 0, h = 3e38.
@@ -194,13 +196,15 @@ struct RayF {
     float3 inv;         // 1/d for the BOX tests only (clamped to +-1e18 for the centre-form slab test: boxes
                         // only cull and are padded).  Primitive tests take their own IEEE reciprocals so
                         // they stay bit-reproducible on the CPU.
-    float3 ood;         // o * inv, for the one-FMA-per-plane slab test
+    float3 nood;        // -(o * inv), for the one-FMA-per-plane slab test.  Stored negated so the packed slab test takes it
+                        // as its addend as is: a negation written there was hoisted out of the traversal loop as three
+                        // extra instructions per segment instead of being folded into FFMA2
 };
 __device__ __forceinline__ RayF make_ray(float3 o, float3 d) {
     RayF r;
     r.o = o; r.d = d;
     r.inv = f3(__frcp_rn(d.x), __frcp_rn(d.y), __frcp_rn(d.z));
-    r.ood = f3(o.x * r.inv.x, o.y * r.inv.y, o.z * r.inv.z);
+    r.nood = f3(-(o.x * r.inv.x), -(o.y * r.inv.y), -(o.z * r.inv.z));
     return r;
 }
 // The slab tests take a reciprocal clamped to +-1e18: with an infinite one (direction component exactly 0) the
@@ -212,7 +216,7 @@ __device__ __forceinline__ float clamp_inv(float x) { return fminf(fmaxf(x, -1e1
 __device__ __forceinline__ RayF make_ray_shade(float3 o, float3 d) {
     RayF r;
     r.o = o; r.d = d;
-    r.inv = f3(0.f, 0.f, 0.f); r.ood = r.inv;
+    r.inv = f3(0.f, 0.f, 0.f); r.nood = r.inv;
     return r;
 }
 
@@ -238,21 +242,70 @@ __device__ __forceinline__ bool aabb_hit2(const RayF& r, float lox, float loy, f
     return !(hi <= lo);
 }
 
+// Packed FP32 FMA: (a.x * b.x + c.x, a.y * b.y + c.y), each lane rounded exactly like fmaf (fma.rn.f32x2 = one FFMA2 on
+// sm_100).  A broadcast operand is passed as (s, s); ptxas folds it into the instruction's scalar operand.  The pairs are
+// formed inside this one asm statement on purpose: a (s, s) pair of a ray constant packed in a statement of its own is
+// loop-invariant, gets hoisted out of the traversal loop and then stays live there as an extra register pair.
+__device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c) {
+    float2 d;
+    asm("{\n\t"
+        ".reg .b64 a, b, c, d;\n\t"
+        "mov.b64 a, {%2, %3};\n\t"
+        "mov.b64 b, {%4, %5};\n\t"
+        "mov.b64 c, {%6, %7};\n\t"
+        "fma.rn.f32x2 d, a, b, c;\n\t"
+        "mov.b64 {%0, %1}, d;\n\t"
+        "}"
+        : "=f"(d.x), "=f"(d.y) : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y), "f"(c.x), "f"(c.y));
+    return d;
+}
+// a - b and a * b per lane, rounded like __fsub_rn / __fmul_rn (FADD2 / FMUL2).
+__device__ __forceinline__ float2 sub2(float2 a, float2 b) {
+    float2 d;
+    asm("{\n\t"
+        ".reg .b64 a, b, d;\n\t"
+        "mov.b64 a, {%2, %3};\n\t"
+        "mov.b64 b, {%4, %5};\n\t"
+        "sub.rn.f32x2 d, a, b;\n\t"
+        "mov.b64 {%0, %1}, d;\n\t"
+        "}"
+        : "=f"(d.x), "=f"(d.y) : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y));
+    return d;
+}
+__device__ __forceinline__ float2 mul2(float2 a, float2 b) {
+    float2 d;
+    asm("{\n\t"
+        ".reg .b64 a, b, d;\n\t"
+        "mov.b64 a, {%2, %3};\n\t"
+        "mov.b64 b, {%4, %5};\n\t"
+        "mul.rn.f32x2 d, a, b;\n\t"
+        "mov.b64 {%0, %1}, d;\n\t"
+        "}"
+        : "=f"(d.x), "=f"(d.y) : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y));
+    return d;
+}
+
 // Slab test on a box given as centre + half-extent: per axis
 //   t_c = c * inv - o * inv,   t_near = t_c - h |inv|,   t_far = t_c + h |inv|
 // — three FMAs and no min/max pair.  Against (plane - o) * inv each plane carries an extra absolute error of
 // eps * |o * inv| (eps * |o| in space) plus eps * |c| for the centre; the BVH boxes are padded by more than that
 // (scene_create), so a box can only be entered EARLY: the test is conservative and the closest hit unchanged.  ncu on the min/max form: the ALU pipe (FMNMX, selects,
 // integer ops; half the FMA pipes' rate on sm_100) was 58 % busy against 23 % for the FMA pipes,
-// with 10 ALU-pipe operations per box; this form has 4.  
-__device__ __forceinline__ void aabb_center(const RayF& r, float cx, float cy, float cz, float hx, float hy, float hz,
-                                            float t_min, float t_max, float* lo, float* hi) {
-    float tx = fmaf(cx, r.inv.x, -r.ood.x), ty = fmaf(cy, r.inv.y, -r.ood.y), tz = fmaf(cz, r.inv.z, -r.ood.z);
-    float ax = fabsf(r.inv.x), ay = fabsf(r.inv.y), az = fabsf(r.inv.z);      // |x| is an operand modifier of FFMA
-    float nx = fmaf(-hx, ax, tx), ny = fmaf(-hy, ay, ty), nz = fmaf(-hz, az, tz);
-    float fx = fmaf(hx, ax, tx), fy = fmaf(hy, ay, ty), fz = fmaf(hz, az, tz);
-    *lo = fmaxf(fmaxf(nx, ny), fmaxf(nz, t_min));
-    *hi = fminf(fminf(fx, fy), fminf(fz, t_max));
+// with 10 ALU-pipe operations per box; this form has 4.
+// Both children of a node at once, from its child-paired quads (node_layout.hpp): each of the nine FMAs is one FFMA2 over
+// (child 0, child 1) with the ray constant as the broadcast operand, so each child gets exactly the bits of three scalar fmaf
+// per axis.
+__device__ __forceinline__ void aabb_center2(const RayF& r, float4 q0, float4 q1, float4 q2, float t_min, float t_max,
+                                             float* lo0, float* hi0, float* lo1, float* hi1) {
+    const float2 ix = make_float2(r.inv.x, r.inv.x), iy = make_float2(r.inv.y, r.inv.y), iz = make_float2(r.inv.z, r.inv.z);
+    const float2 ox = make_float2(r.nood.x, r.nood.x), oy = make_float2(r.nood.y, r.nood.y), oz = make_float2(r.nood.z, r.nood.z);
+    const float2 ax = make_float2(fabsf(r.inv.x), fabsf(r.inv.x)), ay = make_float2(fabsf(r.inv.y), fabsf(r.inv.y)),
+                 az = make_float2(fabsf(r.inv.z), fabsf(r.inv.z));      // |x| is an operand modifier of FFMA2's scalar
+    float2 tx = fma2(make_float2(q0.x, q0.y), ix, ox), ty = fma2(make_float2(q0.z, q0.w), iy, oy), tz = fma2(make_float2(q1.x, q1.y), iz, oz);
+    float2 nx = fma2(make_float2(-q1.z, -q1.w), ax, tx), ny = fma2(make_float2(-q2.x, -q2.y), ay, ty), nz = fma2(make_float2(-q2.z, -q2.w), az, tz);
+    float2 fx = fma2(make_float2(q1.z, q1.w), ax, tx), fy = fma2(make_float2(q2.x, q2.y), ay, ty), fz = fma2(make_float2(q2.z, q2.w), az, tz);
+    *lo0 = fmaxf(fmaxf(nx.x, ny.x), fmaxf(nz.x, t_min)); *hi0 = fminf(fminf(fx.x, fy.x), fminf(fz.x, t_max));
+    *lo1 = fmaxf(fmaxf(nx.y, ny.y), fmaxf(nz.y, t_min)); *hi1 = fminf(fminf(fx.y, fy.y), fminf(fz.y, t_max));
 }
 
 // ------------------------------------------------------------------------------------------
@@ -345,8 +398,11 @@ __device__ __forceinline__ void hit_rect(const RayF& r, uint32_t type, float4 g0
 // 4 (y) — the first face index of the reference's pair.
 __device__ __forceinline__ void hit_box(const RayF& r, float4 lo, float4 hi, int id, float t_min, Closest& c, const float3* inv_e = nullptr) {
     float ix = inv_e ? inv_e->x : rcp_exact(r.d.x), iy = inv_e ? inv_e->y : rcp_exact(r.d.y), iz = inv_e ? inv_e->z : rcp_exact(r.d.z);
-    float ax = __fmul_rn(__fsub_rn(lo.x, r.o.x), ix), bx = __fmul_rn(__fsub_rn(hi.x, r.o.x), ix);
-    float ay = __fmul_rn(__fsub_rn(lo.y, r.o.y), iy), by = __fmul_rn(__fsub_rn(hi.y, r.o.y), iy);
+    // the x and y planes as (x, y) pairs: FADD2 + FMUL2 for the lo planes, again for the hi planes; each lane rounds as
+    // __fsub_rn / __fmul_rn do, so the hit is bit for bit the scalar one
+    const float2 oxy = make_float2(r.o.x, r.o.y), ixy = make_float2(ix, iy);
+    const float2 axy = mul2(sub2(make_float2(lo.x, lo.y), oxy), ixy), bxy = mul2(sub2(make_float2(hi.x, hi.y), oxy), ixy);
+    float ax = axy.x, ay = axy.y, bx = bxy.x, by = bxy.y;
     float az = __fmul_rn(__fsub_rn(lo.z, r.o.z), iz), bz = __fmul_rn(__fsub_rn(hi.z, r.o.z), iz);
     float nx = fminf(ax, bx), fx = fmaxf(ax, bx);
     float ny = fminf(ay, by), fy = fmaxf(ay, by);
@@ -403,6 +459,8 @@ struct TravCounters { uint32_t nodes, prims; };
 // pop needs neither an index multiply nor an emptiness test: the sentinel ends the traversal.
 // The step is written branch-free (selects + one predicated store / load): the three outcomes
 // (both children hit / one / none) otherwise diverge inside nearly every warp step.
+// With FAST slabs the whole step is 35 SASS instructions in the shared-memory render kernel and 34 in the global-memory one
+// (9 FFMA2, 8 min/max, the node loads, the predicated push / pop); with one scalar FFMA per child and plane it was 44 and 42.
 template <bool COUNT, bool FAST, class Acc>
 __device__ __forceinline__ void trav_inner_s(const RayF& r, const Acc& acc, uint32_t& top, int stride_bytes, float t_min, const Closest& c,
                                              int& node, TravCounters& tc) {
@@ -411,14 +469,13 @@ __device__ __forceinline__ void trav_inner_s(const RayF& r, const Acc& acc, uint
     if (COUNT) tc.nodes++;
     float lo0, hi0, lo1, hi1;
     if (FAST) {
-        aabb_center(r, q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, t_min, c.t, &lo0, &hi0);
-        aabb_center(r, q1.z, q1.w, q2.x, q2.y, q2.z, q2.w, t_min, c.t, &lo1, &hi1);
+        aabb_center2(r, q0, q1, q2, t_min, c.t, &lo0, &hi0, &lo1, &hi1);
     } else {
         // Exact path (ray origins far outside the scene, B200RT_FAST_SLAB=0): Aabb::hit2's arithmetic on the box
         // [c - h, c + h] (a superset of the primitive's box: a box only culls).  Its verdict as an interval: a miss
-        // becomes an empty one.
-        bool h0 = aabb_hit2(r, q0.x - q0.w, q0.y - q1.x, q0.z - q1.y, q0.x + q0.w, q0.y + q1.x, q0.z + q1.y, t_min, c.t, &lo0);
-        bool h1 = aabb_hit2(r, q1.z - q2.y, q1.w - q2.z, q2.x - q2.w, q1.z + q2.y, q1.w + q2.z, q2.x + q2.w, t_min, c.t, &lo1);
+        // becomes an empty one.  Child 0's c and h are the .x / .z lanes of the quads, child 1's the .y / .w lanes.
+        bool h0 = aabb_hit2(r, q0.x - q1.z, q0.z - q2.x, q1.x - q2.z, q0.x + q1.z, q0.z + q2.x, q1.x + q2.z, t_min, c.t, &lo0);
+        bool h1 = aabb_hit2(r, q0.y - q1.w, q0.w - q2.y, q1.y - q2.w, q0.y + q1.w, q0.w + q2.y, q1.y + q2.w, t_min, c.t, &lo1);
         hi0 = h0 ? INFINITY : -INFINITY; hi1 = h1 ? INFINITY : -INFINITY;
         lo0 = h0 ? lo0 : 0.0f; lo1 = h1 ? lo1 : 0.0f;
     }
