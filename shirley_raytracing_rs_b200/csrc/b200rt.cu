@@ -143,13 +143,30 @@ int env_int(const char* name, int dflt) { const char* v = getenv(name); return v
 
 SceneSize scene_size(const B200rtScene* sc) { return {sc->ds.n_nodes, sc->ds.n_prims, sc->ds.n_tex, sc->ds.bvh_depth}; }
 
-// The centre-form (one-FMA) slab planes are conservative only while |origin| * eps stays below the box padding;
-// `max_origin` is the largest |coordinate| of a ray origin.  B200RT_FAST_SLAB=0 forces the exact Aabb::hit2 arithmetic.
-bool use_fast_slab(const B200rtScene* sc, float max_origin) {
-    return sc->box_pad >= 4.0f * 1.1920929e-7f * std::max(sc->max_abs_coord, max_origin) && env_int("B200RT_FAST_SLAB", 1) != 0;
+// The centre-form (one-FMA) slab planes are conservative only while |origin| * eps stays below the box padding and no
+// direction is so short that the clamped reciprocal culls a hit (launch_plan.hpp: fast_slab_ok); `max_origin` is the largest
+// |coordinate| of a ray origin, `min_dir_inf` the smallest max_k |d_k| of a ray.  B200RT_FAST_SLAB=0 forces the exact
+// Aabb::hit2 arithmetic.
+bool use_fast_slab(const B200rtScene* sc, float max_origin, float min_dir_inf) {
+    return fast_slab_ok(sc->box_pad, sc->max_abs_coord, max_origin, min_dir_inf) && env_int("B200RT_FAST_SLAB", 1) != 0;
 }
+// Primary rays: pixel_ray forms d = llo + x hw + y vh - offset with x in [0, width], y in [0, height] and the lens offset a
+// combination of ul and vl with weights in [-1, 1].  Along the unit view axis w, |d.w| >= |llo.w| - width |hw.w| -
+// height |vh.w| - |ul.w| - |vl.w| (every term but the first is 0 for a camera whose u, v are perpendicular to w), less the
+// f32 rounding of d, and |d|inf >= |d.w| / sqrt(3).  Secondary rays are not bounded here (DESIGN.md §3 item 7).
+DeviceCamera make_camera(const B200rtCamera& c);
 bool use_fast_slab(const B200rtScene* sc, const B200rtCamera* cam) {
-    return use_fast_slab(sc, std::max(std::fabs((float)cam->origin[0]), std::max(std::fabs((float)cam->origin[1]), std::fabs((float)cam->origin[2]))));
+    const DeviceCamera dc = make_camera(*cam);
+    const double wn = std::sqrt(cam->w[0] * cam->w[0] + cam->w[1] * cam->w[1] + cam->w[2] * cam->w[2]);
+    auto along = [&](float3 v) { return std::fabs((v.x * cam->w[0] + v.y * cam->w[1] + v.z * cam->w[2]) / wn); };
+    auto norm1 = [](float3 v) { return (double)std::fabs(v.x) + std::fabs(v.y) + std::fabs(v.z); };
+    const double W = dc.width, H = dc.height;
+    const double spread = W * along(dc.hw) + H * along(dc.vh) + along(dc.ul) + along(dc.vl);
+    const double rounding = 4.0 * 1.1920929e-7 * (norm1(dc.llo) + W * norm1(dc.hw) + H * norm1(dc.vh) + norm1(dc.ul) + norm1(dc.vl));
+    const double bound = (along(dc.llo) - spread - rounding) / std::sqrt(3.0);
+    const float min_dir_inf = wn > 0.0 && bound > 0.0 ? (float)bound : 0.0f;
+    return use_fast_slab(sc, std::max(std::fabs((float)cam->origin[0]), std::max(std::fabs((float)cam->origin[1]), std::fabs((float)cam->origin[2]))),
+                         min_dir_inf);
 }
 
 int resolve_device(int device, int* out) {
@@ -1387,11 +1404,18 @@ int b200rt_closest_hit(const B200rtScene* csc, const B200rtRay* rays, size_t n, 
     a.next_ray = &d_ctr.as<Counters>()->diag[0];     // zeroed with the counters
     const SmemPlan plan = hook_plan(scene_size(sc), sc->smem_optin);
     a.plan = plan;
-    float max_origin = 0.f;
-    for (size_t i = 0; i < n; ++i) max_origin = std::max(max_origin, std::max(std::fabs(rays[i].ox), std::max(std::fabs(rays[i].oy), std::fabs(rays[i].oz))));
+    // A NaN origin component is skipped (both slab forms leave that axis unconstrained); a NaN direction component takes
+    // the exact path: clamp_inv turns its NaN reciprocal into -1e18, where Aabb::hit2 leaves the axis unconstrained.
+    float max_origin = 0.f, min_dir_inf = INFINITY;
+    for (size_t i = 0; i < n; ++i) {
+        const B200rtRay& r = rays[i];
+        max_origin = std::max(max_origin, std::max(std::fabs(r.ox), std::max(std::fabs(r.oy), std::fabs(r.oz))));
+        const float d_inf = std::max(std::fabs(r.dx), std::max(std::fabs(r.dy), std::fabs(r.dz)));
+        min_dir_inf = std::isnan(r.dx) || std::isnan(r.dy) || std::isnan(r.dz) ? 0.f : std::min(min_dir_inf, d_inf);
+    }
     // traversal counters ride along with the full hit records (parity runs); ids-only calls — the BVH microbenchmark
     // shape of benches/my_benchmark.rs — run the kernel without them
-    HitKernel kernel = hit_kernel(plan.all_in_smem, use_fast_slab(sc, max_origin), stats != nullptr && hits != nullptr);
+    HitKernel kernel = hit_kernel(plan.all_in_smem, use_fast_slab(sc, max_origin, min_dir_inf), stats != nullptr && hits != nullptr);
     if ((rc = set_smem(kernel, sc, plan.bytes))) return rc;
     int bps = 0;
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kernel, BLOCK, plan.bytes));

@@ -58,6 +58,30 @@ inline SmemPlan hook_plan(const SceneSize& s, size_t smem_optin) {
     return plan;
 }
 
+// Whether a launch may test boxes with the centre-form slab test (rt_device.cuh: aabb_center2) instead of the exact
+// Aabb::hit2 arithmetic.  `box_pad` is how far every BVH box was grown (scene_create: 4e-6 x max_abs_coord), `max_abs_coord`
+// the largest |coordinate| of any primitive box, `max_origin` the largest |coordinate| of a ray origin and `min_dir_inf` the
+// smallest max_k |d_k| over the rays (NaN or 0: never fast).  The centre form must be conservative, entering a box early but
+// never culling a box the ray meets.  Let M = max(max_abs_coord, max_origin) and eps = 2^-23.
+//  * Rounding.  A plane distance takes three roundings (-(o * inv), then the two FMAs) of values below |o|, |c| + |o| and
+//    |c| + h + |o| in units of |inv|: at most eps / 2 x (3 |o| + 2 |c| + h) <= 3 eps M |inv| in all, against the pad of
+//    >= 4 eps M |inv| the first condition asks for.  So a plane `pad` outside the primitive's box is computed at least
+//    pad / 4 outside it.
+//  * The reciprocal clamp.  On an axis whose |d_k| < 1e-18 the slab test takes |inv| = 1e18 (clamp_inv) instead of
+//    1 / |d_k|, so its far plane comes in to (its distance in space) x 1e18.  A hit point p of the primitive has p_k inside
+//    the primitive's box, so (say d_k > 0) the padded far plane is hi_k + pad - o_k >= pad + t d_k >= pad away from the
+//    origin, and the computed far distance is at least pad / 4 x 1e18.  On the axis j of the largest |d_j|,
+//    t |d_j| = |p_j - o_j| <= max_abs_coord + M.  So the clamp culls no hit while
+//        |d|inf >= 4 (max_abs_coord + M) / (pad x 1e18),
+//    about 1e-11 at the largest origin the first condition allows (M = 8.4 max_abs_coord), whatever the scene's scale.
+//    Shorter directions (the reference's Ray is not normalised) take the exact path.
+// tests/native/slab_guard_check.cpp runs the centre-form test on the CPU against the f64 box interval over this range.
+inline bool fast_slab_ok(float box_pad, float max_abs_coord, float max_origin, float min_dir_inf) {
+    const float M = std::max(max_abs_coord, max_origin);
+    return box_pad >= 4.0f * 1.1920929e-7f * M
+        && min_dir_inf > 0.0f && (double)min_dir_inf * box_pad * 1e18 >= 4.0 * ((double)max_abs_coord + M);
+}
+
 struct RenderShape { uint32_t block_threads; SmemPlan plan; };
 
 // The path tracer runs one 768-thread CTA per SM (profiles/r02_experiments.md §16).  A deep tree (the device-built linear

@@ -223,9 +223,9 @@ __device__ __forceinline__ RayF make_ray_shade(float3 o, float3 d) {
 // Aabb::hit2 (bvh/aabb.rs:62-79) in f32 with the reference's exact NaN/inf behaviour:
 // the swap is selected by the sign of 1/d (not by min/max of the two plane distances), a
 // NaN plane distance (0 * inf) leaves the interval unchanged, `t_max <= t_min` misses.
-// Returns the entry distance through *t_enter.
+// Returns the entry distance through *t_enter and, when asked, the exit distance through *t_exit.
 __device__ __forceinline__ bool aabb_hit2(const RayF& r, float lox, float loy, float loz, float hix, float hiy, float hiz,
-                                          float t_min, float t_max, float* t_enter) {
+                                          float t_min, float t_max, float* t_enter, float* t_exit = nullptr) {
     float ax = __fmul_rn(__fsub_rn(lox, r.o.x), r.inv.x), bx = __fmul_rn(__fsub_rn(hix, r.o.x), r.inv.x);
     float ay = __fmul_rn(__fsub_rn(loy, r.o.y), r.inv.y), by = __fmul_rn(__fsub_rn(hiy, r.o.y), r.inv.y);
     float az = __fmul_rn(__fsub_rn(loz, r.o.z), r.inv.z), bz = __fmul_rn(__fsub_rn(hiz, r.o.z), r.inv.z);
@@ -239,6 +239,7 @@ __device__ __forceinline__ bool aabb_hit2(const RayF& r, float lox, float loy, f
     float lo = fmaxf(fmaxf(t0x, t0y), fmaxf(t0z, t_min));
     float hi = fminf(fminf(t1x, t1y), fminf(t1z, t_max));
     *t_enter = lo;
+    if (t_exit) *t_exit = hi;
     return !(hi <= lo);
 }
 
@@ -474,8 +475,13 @@ __device__ __forceinline__ void trav_inner_s(const RayF& r, const Acc& acc, uint
         // Exact path (ray origins far outside the scene, B200RT_FAST_SLAB=0): Aabb::hit2's arithmetic on the box
         // [c - h, c + h] (a superset of the primitive's box: a box only culls).  Its verdict as an interval: a miss
         // becomes an empty one.  Child 0's c and h are the .x / .z lanes of the quads, child 1's the .y / .w lanes.
-        bool h0 = aabb_hit2(r, q0.x - q1.z, q0.z - q2.x, q1.x - q2.z, q0.x + q1.z, q0.z + q2.x, q1.x + q2.z, t_min, c.t, &lo0);
-        bool h1 = aabb_hit2(r, q0.y - q1.w, q0.w - q2.y, q1.y - q2.w, q0.y + q1.w, q0.w + q2.y, q1.y + q2.w, t_min, c.t, &lo1);
+        // A single-point interval [t, t] is entered, as the centre form enters it: Aabb::hit2's `t_max <= t_min` would
+        // cull it, and when the closest hit so far sits at t == t_min that drops a primitive hit at the same t with a
+        // higher id (accept_t's tie rule), so the winner of the tie would depend on the visiting order.
+        float e0, e1;
+        aabb_hit2(r, q0.x - q1.z, q0.z - q2.x, q1.x - q2.z, q0.x + q1.z, q0.z + q2.x, q1.x + q2.z, t_min, c.t, &lo0, &e0);
+        aabb_hit2(r, q0.y - q1.w, q0.w - q2.y, q1.y - q2.w, q0.y + q1.w, q0.w + q2.y, q1.y + q2.w, t_min, c.t, &lo1, &e1);
+        const bool h0 = !(e0 < lo0), h1 = !(e1 < lo1);
         hi0 = h0 ? INFINITY : -INFINITY; hi1 = h1 ? INFINITY : -INFINITY;
         lo0 = h0 ? lo0 : 0.0f; lo1 = h1 ? lo1 : 0.0f;
     }
