@@ -186,7 +186,10 @@ typedef struct B200rtSceneInfo {
     uint32_t bvh_builder;       /* 0 = binned SAH on the host, 1 = linear BVH built on the device (large scenes) */
 } B200rtSceneInfo;
 
-typedef struct B200rtScene B200rtScene;    /* opaque, immutable after create */
+/* Opaque.  Its contents change only through b200rt_scene_update; every other call only reads it, so renders and hooks may run
+ * on one scene from several host threads at once.  An update must not overlap any other call on the same scene: the caller
+ * serialises them (device work that earlier calls left in flight is waited for by the update itself). */
+typedef struct B200rtScene B200rtScene;
 
 /* ---- parity-hook records ----------------------------------------------------------------- */
 typedef struct B200rtRay { float ox, oy, oz, dx, dy, dz; } B200rtRay;     /* core/vec3.rs:240-244 */
@@ -221,6 +224,29 @@ int  b200rt_device_count(void);
 int  b200rt_scene_create(const B200rtSceneDesc* desc, int device, B200rtScene** out);
 void b200rt_scene_destroy(B200rtScene* scene);
 int  b200rt_scene_info(const B200rtScene* scene, B200rtSceneInfo* out);
+
+/* Replace the contents of a scene in place: geometry, materials, textures, image texels, Perlin tables and skybox are
+ * taken from `desc`; the BVH keeps its topology and its boxes are refit on the device.  Meant for a host that changes a
+ * scene between frames (animation, look development) without paying b200rt_scene_create's flattening, tree build and
+ * whole upload every frame.
+ *   May change: every value in spheres[], rects[] (except kind), boxes[], materials[] (kind, texture, albedo, param),
+ *     textures[], the image texels, the Perlin tables and the skybox.
+ *   Must not change: n_prims and every prims[i] (type, index); n_spheres, n_rects, n_boxes, n_textures, n_images,
+ *     n_perlin; each image's width and height; and whether a primitive's box is valid.  A box that was inverted or
+ *     NaN at creation has no leaf and must stay so, and vice versa: a sphere's radius may not cross zero.
+ *   Any violation, and anything b200rt_scene_create rejects, returns B200RT_EINVAL and leaves the scene exactly as it
+ *     was.  A CUDA error during the copies or the refit returns B200RT_ECUDA and leaves the contents undefined.
+ *   The scene-spanning primitives tested up front (chosen at creation by their share of the scene's area) stay up
+ *     front; this affects speed only, never hits.  The box padding, the largest coordinate that guards the fast slab
+ *     test and the emitter flag are recomputed from the new contents, and every leaf box is padded anew.
+ *   Closest hits do not depend on the tree's topology, so renders and hooks after an update equal those of a scene
+ *     created from `desc`, bit for bit, and an update with an unchanged description leaves every BVH node unchanged.
+ *     The tree's quality can drift as primitives move; when to rebuild (destroy + create) is the caller's choice.
+ *   Ordering: before anything is overwritten the update waits for device work of earlier calls on this scene,
+ *     including b200rt_render_device launches not yet finished; when it returns, the new contents are on the device.
+ *     It must not overlap other calls on the same scene (see B200rtScene).
+ *   B200rtSceneInfo is unchanged by an update.  The first update allocates the refit's links (about 60 B per node). */
+int  b200rt_scene_update(B200rtScene* scene, const B200rtSceneDesc* desc);
 
 /* Replaces the frame loop of render_scene (src/main.rs:85-126): every pixel of the
  * selected rows/tiles gets SUM over `samples` of ray_color(pixel_ray(..)) exactly like

@@ -129,6 +129,7 @@ SIGNATURES = {
     "b200rt_scene_create": (C.c_int, [_P(SceneDesc), C.c_int, _P(C.c_void_p)]),
     "b200rt_scene_destroy": (None, [C.c_void_p]),
     "b200rt_scene_info": (C.c_int, [C.c_void_p, _P(SceneInfo)]),
+    "b200rt_scene_update": (C.c_int, [C.c_void_p, _P(SceneDesc)]),
     "b200rt_render": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, _P(Stats)]),
     "b200rt_render_rgb8": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p, _P(Stats)]),
     "b200rt_render_adaptive": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), _P(AdaptiveParams), C.c_void_p, C.c_void_p,

@@ -193,6 +193,21 @@ class Scene:
         F.check(lib.b200rt_scene_info(self.device(device), C.byref(out)))
         return out
 
+    def update(self, new: "Scene") -> None:
+        """Take `new`'s contents in place (b200rt_scene_update on every device copy): geometry, materials, textures, image
+        texels, Perlin tables and skybox may change, while the primitive list (types and indices), the array counts, the image
+        sizes and whether each primitive's box is valid (e.g. a sphere's radius may not cross zero) must stay as they were.
+        Each device copy keeps its BVH topology and refits its boxes on the device, so hits and renders equal those of a scene
+        created from `new`, bit for bit; only the tree's quality can drift. A rejected update raises B200rtError and changes
+        nothing. On success `new`'s host arrays become this scene's own (so `desc`, `to_json` and later `device()` calls see
+        them) and `new` is closed. With no device copy yet, the scene simply takes `new`'s contents."""
+        if new is self:
+            raise ValueError("a scene cannot be updated from itself")
+        for h in self._dev.values():
+            F.check(lib.b200rt_scene_update(h, new.desc))
+        self._host, new._host = new._host, self._host
+        new.close()
+
     def to_json(self) -> str:
         p, n = C.c_void_p(), C.c_size_t()
         F.check(lib.b200rt_host_scene_to_json(self._host, C.byref(p), C.byref(n)), host=True)

@@ -7,6 +7,8 @@
 //                        K3 resolve_kernel (+ resolve_peers_kernel, flag barrier)  (image.rs:34-40, core/color.rs:31-38)
 //                        K4 scatter / camera_rays / texture_value / aabb_hit / rng parity hooks, FFMA-chain microbenchmark
 //   lbvh.cuh             K5 linear BVH built on the device                         (bvh/bbox_tree/constructor.rs:9-212)
+//   refit.cuh            K6 BVH refit of b200rt_scene_update (either builder's tree, new geometry)
+//   prim_box.hpp         a primitive's leaf box, its validity and padding, the host twin of the refit (host and device)
 //   bvh_build.hpp        host binned-SAH builder
 //   launch_plan.hpp      CTA size, shared-memory plan, sample-range schedule and grid of a launch (pure host arithmetic)
 //   adaptive_plan.hpp    pass schedule and error estimate of tile-adaptive sampling (host and device)
@@ -32,6 +34,7 @@
 #include "bvh_build.hpp"
 #include "launch_plan.hpp"
 #include "lbvh.cuh"
+#include "refit.cuh"
 #include "rt_device.cuh"
 
 namespace b200rt {
@@ -111,6 +114,13 @@ struct B200rtScene {
     std::map<void*, Scratch*> inflight;   // keyed by stream
     float box_pad = 0.f;          // how far every BVH box was grown
     float max_abs_coord = 0.f;    // largest |coordinate| of any primitive box
+    // What b200rt_scene_update must find unchanged (the tree's leaves and the arena layout depend on it), and where it writes.
+    std::vector<B200rtPrimRef> prims;          // (type, index) of every primitive
+    std::vector<uint8_t> valid;                // its box was valid at creation: it has a leaf or is up front
+    uint32_t n_spheres = 0, n_rects = 0, n_boxes = 0, n_images = 0;
+    std::vector<uint32_t> image_wh;            // width, height of each image
+    std::vector<size_t> off_img;               // arena offset of each image's RGBA texels
+    b200rt::refit::State refit;                // links and scratch of the refit, from the first update on
 };
 
 namespace {
@@ -226,6 +236,75 @@ int validate(const B200rtSceneDesc* d) {
         if (!d->images[i].rgb8 || d->images[i].width == 0 || d->images[i].height == 0) return fail(B200RT_EINVAL, "image %u: empty", i);
     if (d->skybox.kind > B200RT_SKY_NONE) return fail(B200RT_EINVAL, "bad skybox kind %u", d->skybox.kind);
     return B200RT_OK;
+}
+
+// The flattening shared by b200rt_scene_create and b200rt_scene_update: the device records of primitive i and its unpadded box
+// (prim_box.hpp), the texture, image and Perlin records, and the scene-wide shading fields.
+struct FlatPrim { GeomRec geom; MatRec mat; HostBox box; bool valid; };
+FlatPrim flatten_prim(const B200rtSceneDesc* d, uint32_t i) {
+    const B200rtPrimRef& p = d->prims[i];
+    FlatPrim f{};
+    GeomRec& g = f.geom;
+    if (p.type == B200RT_PRIM_SPHERE) {
+        const B200rtSphere& s = d->spheres[p.index];
+        g.g0 = make_float4(s.cx, s.cy, s.cz, s.radius);
+    } else if (p.type == B200RT_PRIM_BOX) {
+        const B200rtBox& x = d->boxes[p.index];
+        g.g0 = make_float4(x.min[0], x.min[1], x.min[2], 0.f);
+        g.g1 = make_float4(x.max[0], x.max[1], x.max[2], 0.f);
+    } else {
+        const B200rtRect& r = d->rects[p.index];
+        g.g0 = make_float4(r.d1_min, r.d1_max, r.d2_min, r.d2_max);
+        g.g1 = make_float4(r.offset, 0.f, 0.f, 0.f);
+    }
+    prim_box(p.type, g.g0, g.g1, f.box.lo, f.box.hi);
+    f.valid = box_valid(f.box.lo, f.box.hi);
+    const B200rtMaterial& m = d->materials[i];
+    MatRec& mr = f.mat;
+    mr.kind = m.kind; mr.tex = -1;
+    mr.m0 = make_float4(m.albedo[0], m.albedo[1], m.albedo[2], m.param);
+    if (m.kind == B200RT_MAT_METAL) mr.m0.w = m.param > 1.0f ? 1.0f : m.param;   // metal.rs:18-21
+    if (m.kind == B200RT_MAT_LAMBERTIAN || m.kind == B200RT_MAT_DIFFUSE_LIGHT || m.kind == B200RT_MAT_FAIRY_LIGHT) {
+        const B200rtTexture& t = d->textures[m.texture];
+        if (t.kind == B200RT_TEX_SOLID) mr.m0 = make_float4(t.rgb[0], t.rgb[1], t.rgb[2], 0.f);   // resolved at upload
+        else mr.tex = m.texture;
+    }
+    return f;
+}
+
+std::vector<TexRec> tex_recs(const B200rtSceneDesc* d) {
+    std::vector<TexRec> out(d->n_textures);
+    for (uint32_t t = 0; t < d->n_textures; ++t) {
+        const B200rtTexture& x = d->textures[t];
+        TexRec r{}; r.kind = x.kind; r.r = x.rgb[0]; r.g = x.rgb[1]; r.b = x.rgb[2]; r.scalar = x.scalar; r.odd = x.odd; r.even = x.even; r.image = x.image;
+        out[t] = r;
+    }
+    return out;
+}
+
+// images: RGB8 -> RGBA8 so a texel is one 4-byte load
+void image_rgba(const B200rtImage& im, std::vector<uchar4>& out) {
+    const size_t n = (size_t)im.width * im.height;
+    out.resize(n);
+    for (size_t k = 0; k < n; ++k) out[k] = make_uchar4(im.rgb8[3 * k], im.rgb8[3 * k + 1], im.rgb8[3 * k + 2], 255);
+}
+
+std::vector<PerlinRec> perlin_recs(const B200rtSceneDesc* d) {
+    std::vector<PerlinRec> out(d->n_perlin);
+    for (uint32_t i = 0; i < d->n_perlin; ++i) {
+        for (int k = 0; k < 256; ++k) out[i].ranfloat[k] = make_float4(d->perlin[i].ranfloat[k][0], d->perlin[i].ranfloat[k][1], d->perlin[i].ranfloat[k][2], 0.f);
+        memcpy(out[i].perm_x, d->perlin[i].perm_x, 256); memcpy(out[i].perm_y, d->perlin[i].perm_y, 256); memcpy(out[i].perm_z, d->perlin[i].perm_z, 256);
+    }
+    return out;
+}
+
+void set_shading(DeviceScene& ds, const B200rtSceneDesc* d) {
+    ds.sky_kind = d->skybox.kind == B200RT_SKY_ABOVE ? B200RT_SKY_ABOVE : B200RT_SKY_FLAT;
+    ds.has_emitters = 0;      // DiffuseLight / FairyLight present: ray_color's `emitted` accumulator is live (render kernel)
+    for (uint32_t i = 0; i < d->n_prims; ++i)
+        if (d->materials[i].kind == B200RT_MAT_DIFFUSE_LIGHT || d->materials[i].kind == B200RT_MAT_FAIRY_LIGHT) { ds.has_emitters = 1; break; }
+    bool flat = d->skybox.kind == B200RT_SKY_FLAT;
+    ds.sky_r = flat ? d->skybox.rgb[0] : 0.f; ds.sky_g = flat ? d->skybox.rgb[1] : 0.f; ds.sky_b = flat ? d->skybox.rgb[2] : 0.f;
 }
 
 DeviceCamera make_camera(const B200rtCamera& c) {
@@ -502,51 +581,19 @@ int b200rt_scene_create(const B200rtSceneDesc* d, int device, B200rtScene** out)
 
     std::vector<GeomRec> geom(d->n_prims);
     std::vector<MatRec> mats(d->n_prims);
+    std::vector<uint8_t> valid(d->n_prims);
     std::vector<BuildPrim> bprims;
     std::vector<BuildPrim> bp_all(d->n_prims);       // one slot per primitive (code < 0: no leaf), compacted below
     float max_abs = 0.f;
 #pragma omp parallel for schedule(static) reduction(max : max_abs) if (d->n_prims >= 65536)
     for (long long ii = 0; ii < (long long)d->n_prims; ++ii) {
         const uint32_t i = (uint32_t)ii;
-        const B200rtPrimRef& p = d->prims[i];
-        GeomRec g{}; HostBox b{};
-        if (p.type == B200RT_PRIM_SPHERE) {
-            const B200rtSphere& s = d->spheres[p.index];
-            g.g0 = make_float4(s.cx, s.cy, s.cz, s.radius);
-            // sphere.rs:54-60: center -/+ (r,r,r); a negative radius yields an inverted box
-            b.lo[0] = s.cx - s.radius; b.lo[1] = s.cy - s.radius; b.lo[2] = s.cz - s.radius;
-            b.hi[0] = s.cx + s.radius; b.hi[1] = s.cy + s.radius; b.hi[2] = s.cz + s.radius;
-        } else if (p.type == B200RT_PRIM_BOX) {
-            const B200rtBox& x = d->boxes[p.index];
-            g.g0 = make_float4(x.min[0], x.min[1], x.min[2], 0.f);
-            g.g1 = make_float4(x.max[0], x.max[1], x.max[2], 0.f);
-            for (int k = 0; k < 3; ++k) { b.lo[k] = x.min[k]; b.hi[k] = x.max[k]; }   // rect.rs:158-163
-        } else {
-            const B200rtRect& r = d->rects[p.index];
-            g.g0 = make_float4(r.d1_min, r.d1_max, r.d2_min, r.d2_max);
-            g.g1 = make_float4(r.offset, 0.f, 0.f, 0.f);
-            int d1 = p.type == B200RT_PRIM_RECT_YZ ? 1 : 0, d2 = p.type == B200RT_PRIM_RECT_XY ? 1 : 2, dn = 3 - d1 - d2;
-            b.lo[d1] = r.d1_min; b.hi[d1] = r.d1_max; b.lo[d2] = r.d2_min; b.hi[d2] = r.d2_max;
-            b.lo[dn] = r.offset - 0.0001f; b.hi[dn] = r.offset + 0.0001f;             // rect.rs:9,82-99
-        }
-        geom[i] = g;
-        const B200rtMaterial& m = d->materials[i];
-        MatRec mr{};
-        mr.kind = m.kind; mr.tex = -1;
-        mr.m0 = make_float4(m.albedo[0], m.albedo[1], m.albedo[2], m.param);
-        if (m.kind == B200RT_MAT_METAL) mr.m0.w = m.param > 1.0f ? 1.0f : m.param;   // metal.rs:18-21
-        if (m.kind == B200RT_MAT_LAMBERTIAN || m.kind == B200RT_MAT_DIFFUSE_LIGHT || m.kind == B200RT_MAT_FAIRY_LIGHT) {
-            const B200rtTexture& t = d->textures[m.texture];
-            if (t.kind == B200RT_TEX_SOLID) mr.m0 = make_float4(t.rgb[0], t.rgb[1], t.rgb[2], 0.f);   // resolved at upload
-            else mr.tex = m.texture;
-        }
-        mats[i] = mr;
-        // the reference keeps inverted boxes in its tree, where Aabb::hit2 can never pass;
-        // here they simply get no leaf.  NaN boxes likewise.
-        bool valid = true;
-        for (int k = 0; k < 3; ++k) valid = valid && (b.lo[k] <= b.hi[k]);
-        BuildPrim bp; bp.box = b; bp.code = valid ? (int)((p.type << B200RT_LEAF_TYPE_SHIFT) | i) : -1;
-        for (int k = 0; k < 3; ++k) { bp.centroid[k] = 0.5f * (b.lo[k] + b.hi[k]); if (valid) max_abs = std::max(max_abs, std::max(std::fabs(b.lo[k]), std::fabs(b.hi[k]))); }
+        const FlatPrim f = flatten_prim(d, i);
+        geom[i] = f.geom; mats[i] = f.mat; valid[i] = f.valid;
+        const HostBox& b = f.box;
+        BuildPrim bp; bp.box = b; bp.code = f.valid ? (int)((d->prims[i].type << B200RT_LEAF_TYPE_SHIFT) | i) : -1;
+        for (int k = 0; k < 3; ++k) bp.centroid[k] = 0.5f * (b.lo[k] + b.hi[k]);
+        if (f.valid) max_abs = std::max(max_abs, box_max_abs(b.lo, b.hi));
         bp_all[i] = bp;
     }
     bprims.reserve(d->n_prims);
@@ -573,8 +620,8 @@ int b200rt_scene_create(const B200rtSceneDesc* d, int device, B200rtScene** out)
     // then conservative with respect to the f32 primitive tests — for the exact form always,
     // for the one-FMA form (extra error eps * |origin| per axis) while ray origins stay
     // within ~8x the scene extent (checked per launch).  A box only culls.
-    float pad = max_abs * 4e-6f;
-    for (auto& bp : bprims) for (int k = 0; k < 3; ++k) { bp.box.lo[k] -= pad; bp.box.hi[k] += pad; }
+    const float pad = box_pad_for(max_abs);
+    for (auto& bp : bprims) pad_box(bp.box.lo, bp.box.hi, pad);
     // Builder: binned SAH on the host (bvh_build.hpp), or — for scenes large enough that the host build
     // would dominate a frame — the linear BVH built on the device (lbvh.cuh).  B200RT_BUILDER=sah|lbvh forces one.
     bool use_lbvh = bprims.size() >= LBVH_AUTO_MIN;
@@ -595,12 +642,7 @@ int b200rt_scene_create(const B200rtSceneDesc* d, int device, B200rtScene** out)
     }
 
     lap(use_lbvh ? "top list + padding" : "top list + padding + host SAH");
-    std::vector<TexRec> tex(d->n_textures);
-    for (uint32_t t = 0; t < d->n_textures; ++t) {
-        const B200rtTexture& x = d->textures[t];
-        TexRec r{}; r.kind = x.kind; r.r = x.rgb[0]; r.g = x.rgb[1]; r.b = x.rgb[2]; r.scalar = x.scalar; r.odd = x.odd; r.even = x.even; r.image = x.image;
-        tex[t] = r;
-    }
+    std::vector<TexRec> tex = tex_recs(d);
 
     B200rtScene* sc = new B200rtScene();
     sc->device = device;
@@ -634,23 +676,16 @@ int b200rt_scene_create(const B200rtSceneDesc* d, int device, B200rtScene** out)
     Arena arena;
     size_t off_nodes = use_lbvh ? arena.reserve(n_nodes * sizeof(BvhNode)) : arena.put(cnodes);
     size_t off_geom = arena.put(geom), off_mats = arena.put(mats), off_tex = arena.put(tex);
-    // images: RGB8 -> RGBA8 so a texel is one 4-byte load
     std::vector<ImageRec> images(d->n_images);
     std::vector<size_t> off_img(d->n_images);
     std::vector<std::vector<uchar4>> rgba(d->n_images);
     for (uint32_t i = 0; i < d->n_images; ++i) {
         const B200rtImage& im = d->images[i];
-        size_t n = (size_t)im.width * im.height;
-        rgba[i].resize(n);
-        for (size_t k = 0; k < n; ++k) rgba[i][k] = make_uchar4(im.rgb8[3 * k], im.rgb8[3 * k + 1], im.rgb8[3 * k + 2], 255);
+        image_rgba(im, rgba[i]);
         off_img[i] = arena.put(rgba[i]);
         images[i].width = im.width; images[i].height = im.height; images[i].pad = 0;
     }
-    std::vector<PerlinRec> perlin(d->n_perlin);
-    for (uint32_t i = 0; i < d->n_perlin; ++i) {
-        for (int k = 0; k < 256; ++k) perlin[i].ranfloat[k] = make_float4(d->perlin[i].ranfloat[k][0], d->perlin[i].ranfloat[k][1], d->perlin[i].ranfloat[k][2], 0.f);
-        memcpy(perlin[i].perm_x, d->perlin[i].perm_x, 256); memcpy(perlin[i].perm_y, d->perlin[i].perm_y, 256); memcpy(perlin[i].perm_z, d->perlin[i].perm_z, 256);
-    }
+    std::vector<PerlinRec> perlin = perlin_recs(d);
     size_t off_perlin = arena.put(perlin);
     size_t off_images = arena.put(images);      // the texel pointers are filled in below, before the upload
     lap("lay out arena");
@@ -711,14 +746,14 @@ int b200rt_scene_create(const B200rtSceneDesc* d, int device, B200rtScene** out)
     for (int k = 0; k < 7; ++k) sc->ds.top_prims[k] = ds_top.top_prims[k];
     sc->box_pad = pad; sc->max_abs_coord = max_abs;
     sc->ds.n_nodes = (uint32_t)n_nodes; sc->ds.n_prims = d->n_prims; sc->ds.n_tex = d->n_textures; sc->ds.bvh_depth = bvh.depth;
-    sc->ds.sky_kind = d->skybox.kind == B200RT_SKY_ABOVE ? B200RT_SKY_ABOVE : B200RT_SKY_FLAT;
-    sc->ds.has_emitters = 0;      // DiffuseLight / FairyLight present: ray_color's `emitted` accumulator is live (render kernel)
-    for (uint32_t i = 0; i < d->n_prims; ++i)
-        if (d->materials[i].kind == B200RT_MAT_DIFFUSE_LIGHT || d->materials[i].kind == B200RT_MAT_FAIRY_LIGHT) { sc->ds.has_emitters = 1; break; }
-    bool flat = d->skybox.kind == B200RT_SKY_FLAT;
-    sc->ds.sky_r = flat ? d->skybox.rgb[0] : 0.f; sc->ds.sky_g = flat ? d->skybox.rgb[1] : 0.f; sc->ds.sky_b = flat ? d->skybox.rgb[2] : 0.f;
+    set_shading(sc->ds, d);
     sc->info.n_prims = d->n_prims; sc->info.n_bvh_nodes = sc->ds.n_nodes; sc->info.bvh_depth = bvh.depth;
     sc->info.bvh_nodes_in_smem = hook_plan(scene_size(sc), sc->smem_optin).n_top;
+    sc->prims.assign(d->prims, d->prims + d->n_prims);
+    sc->valid.swap(valid);
+    sc->n_spheres = d->n_spheres; sc->n_rects = d->n_rects; sc->n_boxes = d->n_boxes; sc->n_images = d->n_images;
+    for (uint32_t i = 0; i < d->n_images; ++i) { sc->image_wh.push_back(d->images[i].width); sc->image_wh.push_back(d->images[i].height); }
+    sc->off_img.swap(off_img);
     *out = sc;
     return B200RT_OK;
 }
@@ -735,6 +770,7 @@ void b200rt_scene_destroy(B200rtScene* sc) {
             g_scratch_pool[sc->device].push_back(kv.second);
         }
     }
+    sc->refit.release();
     if (sc->arena) {   // one arena holds every scene array: back to the pool (every render on it has been waited for above)
         bool pooled = false;
         {
@@ -745,6 +781,89 @@ void b200rt_scene_destroy(B200rtScene* sc) {
         if (!pooled) cudaFree(sc->arena);
     }
     delete sc;
+}
+
+int b200rt_scene_update(B200rtScene* sc, const B200rtSceneDesc* d) {
+    if (!sc) return fail(B200RT_EINVAL, "scene is NULL");
+    const bool timing = getenv("B200RT_TIMING") != nullptr;
+    auto t_prev = std::chrono::steady_clock::now();
+    auto lap = [&](const char* what) {
+        if (!timing) return;
+        auto now = std::chrono::steady_clock::now();
+        fprintf(stderr, "[b200rt] scene_update %-28s %8.2f ms\n", what, std::chrono::duration<double, std::milli>(now - t_prev).count());
+        t_prev = now;
+    };
+    // Everything is checked before anything is overwritten: a rejected update leaves the scene as it was.
+    int rc = validate(d); if (rc) return rc;
+    if (d->n_prims != sc->prims.size()) return fail(B200RT_EINVAL, "scene update: n_prims %u != %zu at creation", d->n_prims, sc->prims.size());
+    if (d->n_spheres != sc->n_spheres || d->n_rects != sc->n_rects || d->n_boxes != sc->n_boxes || d->n_textures != sc->ds.n_tex ||
+        d->n_images != sc->n_images || d->n_perlin != sc->ds.n_perlin)
+        return fail(B200RT_EINVAL, "scene update: array counts differ from the scene's at creation");
+    for (uint32_t i = 0; i < d->n_prims; ++i)
+        if (d->prims[i].type != sc->prims[i].type || d->prims[i].index != sc->prims[i].index)
+            return fail(B200RT_EINVAL, "scene update: prim %u is (%u, %u), was (%u, %u)", i, d->prims[i].type, d->prims[i].index, sc->prims[i].type, sc->prims[i].index);
+    for (uint32_t i = 0; i < d->n_images; ++i)
+        if (d->images[i].width != sc->image_wh[2 * i] || d->images[i].height != sc->image_wh[2 * i + 1])
+            return fail(B200RT_EINVAL, "scene update: image %u is %ux%u, was %ux%u", i, d->images[i].width, d->images[i].height, sc->image_wh[2 * i], sc->image_wh[2 * i + 1]);
+    std::vector<GeomRec> geom(d->n_prims);
+    std::vector<MatRec> mats(d->n_prims);
+    float max_abs = 0.f;
+    long long changed = -1;   // a primitive whose box became valid or invalid (it would gain or lose its leaf)
+#pragma omp parallel for schedule(static) reduction(max : max_abs, changed) if (d->n_prims >= 65536)
+    for (long long ii = 0; ii < (long long)d->n_prims; ++ii) {
+        const FlatPrim f = flatten_prim(d, (uint32_t)ii);
+        geom[ii] = f.geom; mats[ii] = f.mat;
+        if (f.valid) max_abs = std::max(max_abs, box_max_abs(f.box.lo, f.box.hi));
+        if (f.valid != (sc->valid[ii] != 0)) changed = std::max(changed, ii);
+    }
+    if (changed >= 0)
+        return fail(B200RT_EINVAL, "scene update: prim %lld would %s its BVH leaf (its box became %s)", changed, sc->valid[changed] ? "lose" : "gain",
+                    sc->valid[changed] ? "inverted or NaN" : "valid");
+    const std::vector<TexRec> tex = tex_recs(d);
+    std::vector<std::vector<uchar4>> rgba(d->n_images);
+    for (uint32_t i = 0; i < d->n_images; ++i) image_rgba(d->images[i], rgba[i]);
+    const std::vector<PerlinRec> perlin = perlin_recs(d);
+    lap("validate + flatten");
+
+    DeviceGuard guard(sc->device);
+    if (!guard.ok) return fail(B200RT_ECUDA, "cudaSetDevice(%d) failed", sc->device);
+    {   // device work of earlier calls may still read the arena: renders enqueued by b200rt_render_device and not yet finished
+        std::lock_guard<std::mutex> lk(sc->mu);
+        for (auto& kv : sc->inflight)
+            if (kv.second->launched) CU(cudaStreamSynchronize(kv.second->launch_stream));
+    }
+    if (!sc->refit.base) {
+        cudaError_t e = sc->refit.init(sc->ds.nodes, sc->ds.n_nodes, d->n_prims);
+        if (e != cudaSuccess) return fail(e == cudaErrorMemoryAllocation ? B200RT_ENOMEM : B200RT_ECUDA, "scene update: refit links: %s", cudaGetErrorString(e));
+        lap("refit links (first update)");
+    }
+    // Past this point only a CUDA error can fail the update, and the scene's contents are then undefined.
+    cudaStream_t st = sc->refit.stream;
+    uint8_t* base = static_cast<uint8_t*>(sc->arena);
+    auto put = [&](const void* dst, const void* src, size_t bytes) {
+        return bytes ? cudaMemcpyAsync(const_cast<void*>(dst), src, bytes, cudaMemcpyHostToDevice, st) : cudaSuccess;
+    };
+    cudaError_t e = cudaEventRecord(sc->refit.ev_h2d, st);
+    if (e == cudaSuccess) e = put(sc->ds.geom, geom.data(), geom.size() * sizeof(GeomRec));
+    if (e == cudaSuccess) e = put(sc->ds.mats, mats.data(), mats.size() * sizeof(MatRec));
+    if (e == cudaSuccess) e = put(sc->ds.tex, tex.data(), tex.size() * sizeof(TexRec));
+    for (uint32_t i = 0; i < d->n_images && e == cudaSuccess; ++i) e = put(base + sc->off_img[i], rgba[i].data(), rgba[i].size() * sizeof(uchar4));
+    if (e == cudaSuccess && d->n_perlin) e = put(sc->ds.perlin, perlin.data(), perlin.size() * sizeof(PerlinRec));
+    const float pad = box_pad_for(max_abs);
+    if (e == cudaSuccess) e = sc->refit.run(const_cast<BvhNode*>(sc->ds.nodes), sc->ds.n_nodes, sc->ds.geom, d->n_prims, pad);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return fail(B200RT_ECUDA, "scene update: %s", cudaGetErrorString(e));
+    if (timing) {   // device time from the events around the copies and the refit kernel
+        float ms = 0.f;
+        cudaEventElapsedTime(&ms, sc->refit.ev_h2d, sc->refit.ev1);
+        fprintf(stderr, "[b200rt] scene_update %-28s %8.3f ms\n", "H2D + refit (device)", ms);
+        cudaEventElapsedTime(&ms, sc->refit.ev0, sc->refit.ev1);
+        fprintf(stderr, "[b200rt] scene_update %-28s %8.3f ms\n", "refit kernel (device)", ms);
+    }
+    lap("H2D + refit");
+    sc->box_pad = pad; sc->max_abs_coord = max_abs;
+    set_shading(sc->ds, d);
+    return B200RT_OK;
 }
 
 int b200rt_scene_info(const B200rtScene* sc, B200rtSceneInfo* out) {
