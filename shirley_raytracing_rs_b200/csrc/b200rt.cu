@@ -73,7 +73,8 @@ namespace {
 struct Scratch {                     // per in-flight render: counters, events, staging
     Counters* d_counters = nullptr;
     Counters* h_counters = nullptr;  // pinned
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev2 = nullptr, ev3 = nullptr;
+    // total_ms runs from call_begin to call_end (b200rt_render_device: to kernel_end), kernel_ms from kernel_begin to kernel_end
+    cudaEvent_t call_begin = nullptr, kernel_begin = nullptr, kernel_end = nullptr, call_end = nullptr;
     cudaStream_t own_stream = nullptr;
     cudaStream_t launch_stream = nullptr; bool launched = false;   // where the render in flight was enqueued (scene_destroy waits for it)
     float4* d_accum = nullptr; size_t accum_bytes = 0;
@@ -343,10 +344,8 @@ int get_scratch(B200rtScene* sc, void* stream_key, Scratch** out) {
         s = new Scratch();
         cudaError_t e = cudaMalloc(&s->d_counters, sizeof(Counters));
         if (e == cudaSuccess) e = cudaMallocHost(&s->h_counters, sizeof(Counters));
-        if (e == cudaSuccess) e = cudaEventCreate(&s->ev0);
-        if (e == cudaSuccess) e = cudaEventCreate(&s->ev1);
-        if (e == cudaSuccess) e = cudaEventCreate(&s->ev2);
-        if (e == cudaSuccess) e = cudaEventCreate(&s->ev3);
+        for (cudaEvent_t* ev : {&s->call_begin, &s->kernel_begin, &s->kernel_end, &s->call_end})
+            if (e == cudaSuccess) e = cudaEventCreate(ev);
         if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&s->own_stream, cudaStreamNonBlocking);
         if (e != cudaSuccess) { delete s; return fail(B200RT_ECUDA, "scratch allocation: %s", cudaGetErrorString(e)); }
     }
@@ -362,13 +361,45 @@ void put_scratch(B200rtScene* sc, void* stream_key) {
     sc->inflight.erase(it);
 }
 
-// The attribute belongs to the kernel function, not to a launch: host threads rendering different scenes at once would
-// lower it under each other's feet if it were set to each launch's own size ("too many resources requested for launch",
-// found by tests/test_gpu_scale.py::test_concurrent_renders_from_host_threads).  It is therefore always raised to the device's
-// opt-in maximum — the same value from every thread; the carve-out still follows the bytes each launch asks for.
-template <class K> int set_smem(K kernel, const B200rtScene* sc, uint32_t bytes) {
-    if (bytes > sc->smem_optin) return fail(B200RT_ECUDA, "kernel needs %u B of shared memory, the device offers %zu", bytes, (size_t)sc->smem_optin);
+// A host-buffer render: body(scratch) on the scene's device, with a scratch taken under a key private to the call (concurrent
+// host threads never collide).
+template <class Body> int with_private_scratch(B200rtScene* sc, Body&& body) {
+    DeviceGuard guard(sc->device);
+    int key_local; void* key = &key_local;
+    Scratch* scr; int rc = get_scratch(sc, key, &scr); if (rc) return rc;
+    rc = body(scr);
+    if (rc) cudaStreamSynchronize(scr->own_stream);   // nothing of a failed call may still run when its scratch is reused
+    scr->launched = false;
+    put_scratch(sc, key);
+    return rc;
+}
+
+// The arguments every render entry checks on the frame: params.device, the image size and the row range; *g = its tiles.
+int check_frame(const B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderParams* prm, TileGrid* g) {
+    if (prm->device >= 0 && prm->device != sc->device) return fail(B200RT_EINVAL, "params.device %d != scene device %d", prm->device, sc->device);
+    const uint32_t W = cam->image_width, H = cam->image_height;
+    if (W == 0 || H == 0) return fail(B200RT_EINVAL, "camera image dimensions are zero");
+    if ((uint64_t)W * H > 0xFFFFFFFFull) return fail(B200RT_EINVAL, "image too large");
+    *g = tile_grid(W, H, prm->row_begin, prm->row_end);
+    if (!g->ok) return fail(B200RT_EINVAL, "row range [%u,%u) outside image height %u", g->row_begin, g->row_end, H);
+    return B200RT_OK;
+}
+
+void add_counters(B200rtStats& s, const Counters& c) {
+    s.rays += c.rays; s.paths += c.paths; s.node_visits += c.nodes; s.prim_tests += c.prims; s.depth_exhausted += c.exhausted;
+    for (int k = 0; k < 8; ++k) s.diag[k] += c.diag[k];
+}
+
+// Readies `kernel` for CTAs of `threads` threads and `smem` bytes of dynamic shared memory; *blocks_per_sm = how many fit.
+// The shared-memory attribute belongs to the kernel function, not to a launch: host threads rendering different scenes at
+// once would lower it under each other's feet if it were set to each launch's own size ("too many resources requested for
+// launch", found by tests/test_gpu_scale.py::test_concurrent_renders_from_host_threads).  It is therefore always raised to
+// the device's opt-in maximum — the same value from every thread; the carve-out still follows the bytes each launch asks for.
+template <class K> int fit_kernel(K kernel, const char* name, const B200rtScene* sc, uint32_t threads, uint32_t smem, int* blocks_per_sm) {
+    if (smem > sc->smem_optin) return fail(B200RT_ECUDA, "kernel needs %u B of shared memory, the device offers %zu", smem, (size_t)sc->smem_optin);
     CU(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_optin));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, kernel, threads, smem));
+    if (*blocks_per_sm < 1) return fail(B200RT_ECUDA, "%s does not fit on an SM (smem %u B, %u threads)", name, smem, threads);
     return B200RT_OK;
 }
 
@@ -393,14 +424,14 @@ template <class Acc> HitKernel hit_variant(bool fast, bool count) {
 }
 HitKernel hit_kernel(bool all_in_smem, bool fast, bool count) { return all_in_smem ? hit_variant<SmemAcc>(fast, count) : hit_variant<GmemAcc>(fast, count); }
 
-// One pass of b200rt_render_adaptive: the tiles it renders (NULL: all of them), the fixed-point buffer its sums are added to,
-// and the sample count acc_add's clamp is taken for (max_samples, so that the sums of all passes cannot wrap).
-struct AdaptivePass { const uint32_t* tile_list; uint32_t n_tiles; long long* fix; uint32_t lim_samples; };
+// One pass of a render made of several (an adaptive pass, a half of a denoised render): the tiles it renders (NULL: all of
+// them), the fixed-point buffer its sums are added to, and the sample count acc_add's clamp is taken for (the whole render's,
+// so that the sums of all passes cannot wrap).
+struct PassTarget { const uint32_t* tile_list; uint32_t n_tiles; long long* fix; uint32_t lim_samples; };
 
-int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderParams* prm, float* d_accum, cudaStream_t stream, Scratch* scr,
-                  const AdaptivePass* pass = nullptr) {
-    if (cam->image_width == 0 || cam->image_height == 0) return fail(B200RT_EINVAL, "camera image dimensions are zero");
-    if ((uint64_t)cam->image_width * cam->image_height > 0xFFFFFFFFull) return fail(B200RT_EINVAL, "image too large");
+// `g` is the tile grid check_frame returned for the frame; prm's row range is not read again.
+int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderParams* prm, const TileGrid& g, float4* d_accum, cudaStream_t stream,
+                  Scratch* scr, const PassTarget* pass = nullptr) {
     RenderArgs a{};
     a.scene = sc->ds;
     a.cam = make_camera(*cam);
@@ -410,19 +441,14 @@ int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderPa
     a.tile_list = pass ? pass->tile_list : nullptr;
     a.sample_offset = prm->sample_offset;
     a.max_depth = prm->max_depth;
-    uint32_t H = cam->image_height, W = cam->image_width;
-    a.row_begin = prm->row_begin; a.row_end = prm->row_end;
-    if (a.row_begin == 0 && a.row_end == 0) a.row_end = H;
-    if (a.row_end > H || a.row_begin > a.row_end) return fail(B200RT_EINVAL, "row range [%u,%u) outside image height %u", a.row_begin, a.row_end, H);
-    a.tiles_x = (W + TILE_W - 1) / TILE_W;
-    a.tile_row0 = a.row_begin / TILE_H;
-    uint32_t tile_row1 = (a.row_end + TILE_H - 1) / TILE_H;
-    a.n_tiles = a.tiles_x * (tile_row1 - a.tile_row0);
+    const uint32_t H = cam->image_height, W = cam->image_width;
+    a.row_begin = g.row_begin; a.row_end = g.row_end;
+    a.tiles_x = g.tiles_x; a.tile_row0 = g.tile_row0; a.n_tiles = g.n_tiles;
     a.shard_count = prm->shard_count == 0 ? 1 : prm->shard_count;
     a.shard_index = prm->shard_index;
     if (a.shard_index >= a.shard_count) return fail(B200RT_EINVAL, "shard_index %u >= shard_count %u", a.shard_index, a.shard_count);
     a.accumulate = (prm->flags & B200RT_FLAG_ACCUMULATE) ? 1 : 0;
-    a.accum = reinterpret_cast<float4*>(d_accum);
+    a.accum = d_accum;
     a.counters = scr->d_counters;
     bool count = (prm->flags & B200RT_FLAG_COUNT_TRAVERSAL) != 0;
     a.trav_threshold = (uint32_t)std::min(32, std::max(1, env_int("B200RT_TRAV_THRESHOLD", 8)));
@@ -437,17 +463,15 @@ int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderPa
 
     scr->launches = 0;
     scr->launch_stream = stream; scr->launched = true;
-    CU(cudaEventRecord(scr->ev0, stream));
+    if (!pass) CU(cudaEventRecord(scr->call_begin, stream));   // a render made of passes marks its own beginning
     CU(cudaMemsetAsync(scr->d_counters, 0, sizeof(Counters), stream));
     // The kernel stores every pixel of the tiles it renders; the buffer is cleared only when some pixels are outside them
     // ("pixels outside the selected rows/tiles are written as zeros", include/b200rt.h).
     const bool covers_frame = a.shard_count == 1 && a.row_begin == 0 && a.row_end == H;
     // (adaptive passes write only through the merge kernel; b200rt_render_adaptive clears the buffer once)
     if (!pass && !a.accumulate && !covers_frame) CU(cudaMemsetAsync(d_accum, 0, (size_t)W * H * sizeof(float4), stream));
-    int rc = set_smem(kernel, sc, plan.bytes); if (rc) return rc;
     int blocks_per_sm = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kernel, block_threads, plan.bytes));
-    if (blocks_per_sm < 1) return fail(B200RT_ECUDA, "path-tracing kernel does not fit on an SM (smem %u B, %u threads)", plan.bytes, block_threads);
+    if (int rc = fit_kernel(kernel, "path-tracing kernel", sc, block_threads, plan.bytes, &blocks_per_sm)) return rc;
     const uint32_t warps_per_block = block_threads / 32;
     const uint32_t my_tiles = pass ? pass->n_tiles
                             : a.n_tiles > a.shard_index ? (a.n_tiles - a.shard_index + a.shard_count - 1) / a.shard_count : 0u;   // tiles t with t % shard_count == shard_index
@@ -464,7 +488,7 @@ int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderPa
         a.fix = scr->d_fix;
         CU(cudaMemsetAsync(scr->d_fix, 0, px * 3 * sizeof(long long), stream));
     }
-    CU(cudaEventRecord(scr->ev1, stream));
+    CU(cudaEventRecord(scr->kernel_begin, stream));
     kernel<<<render_grid(full_grid, my_tiles, a.chunks, warps_per_block), block_threads, plan.bytes, stream>>>(a);
     CU(cudaGetLastError());
     scr->launches += 1;
@@ -474,27 +498,75 @@ int launch_render(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderPa
         CU(cudaGetLastError());
         scr->launches += 1;
     }
-    CU(cudaEventRecord(scr->ev2, stream));
+    CU(cudaEventRecord(scr->kernel_end, stream));
     CU(cudaMemcpyAsync(scr->h_counters, scr->d_counters, sizeof(Counters), cudaMemcpyDeviceToHost, stream));
     return B200RT_OK;
 }
 
-int finish_render(Scratch* scr, cudaStream_t stream, cudaEvent_t end_event, B200rtStats* stats) {
-    CU(cudaStreamSynchronize(stream));
-    scr->launched = false;
-    if (stats) {
-        memset(stats, 0, sizeof *stats);
-        stats->rays = scr->h_counters->rays; stats->paths = scr->h_counters->paths;
-        stats->node_visits = scr->h_counters->nodes; stats->prim_tests = scr->h_counters->prims;
-        stats->depth_exhausted = scr->h_counters->exhausted;
-        for (int k = 0; k < 8; ++k) stats->diag[k] = scr->h_counters->diag[k];
-        float ms = 0.f;
-        CU(cudaEventElapsedTime(&ms, scr->ev1, scr->ev2)); stats->kernel_ms = ms;
-        CU(cudaEventElapsedTime(&ms, scr->ev0, end_event)); stats->total_ms = ms;
-        stats->launches = scr->launches;
-    }
+// Adds the counters, kernel time and launches of the scratch's last launch_render, once waited for, to `sum`.
+int add_launch(B200rtStats& sum, const Scratch* scr) {
+    add_counters(sum, *scr->h_counters);
+    float ms = 0.f;
+    CU(cudaEventElapsedTime(&ms, scr->kernel_begin, scr->kernel_end));
+    sum.kernel_ms += ms;
+    sum.launches += scr->launches;
     return B200RT_OK;
 }
+
+// b200rt_render_device_finish: the wait, then the launch's stats, whose total_ms ends with the kernels.
+int finish_render(Scratch* scr, cudaStream_t stream, B200rtStats* stats) {
+    CU(cudaStreamSynchronize(stream));
+    scr->launched = false;
+    if (!stats) return B200RT_OK;
+    B200rtStats sum{};
+    if (int rc = add_launch(sum, scr)) return rc;
+    float ms = 0.f;
+    CU(cudaEventElapsedTime(&ms, scr->call_begin, scr->kernel_end));
+    sum.total_ms = ms;
+    *stats = sum;
+    return B200RT_OK;
+}
+
+// One pass of a render made of several, on the scratch's stream: its launch, then `then()` (work of the pass enqueued behind
+// it, such as the adaptive merge), the wait, and the pass's counters, kernel time and launches added to the call's totals.
+template <class Then> int run_pass(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderParams* p, const TileGrid& g, const PassTarget& pass,
+                                   Scratch* scr, B200rtStats& sum, Then&& then) {
+    if (int rc = launch_render(sc, cam, p, g, scr->d_accum, scr->own_stream, scr, &pass)) return rc;
+    if (int rc = then()) return rc;
+    CU(cudaStreamSynchronize(scr->own_stream));
+    return add_launch(sum, scr);
+}
+
+struct HostCopy { void* host; const void* dev; size_t bytes; };
+
+// The end of a host-buffer render on the scratch's stream: with out_rgb8, d_image resolved to RGB8 at `samples` (0: the count
+// in .w) and copied there; each copy whose host pointer is set; the call's end and the wait; then sum.total_ms, and the resolve
+// counted in sum.launches.  `what` names the call in a CUDA error.
+int finish_frame(Scratch* scr, const B200rtCamera* cam, const float4* d_image, uint32_t samples, uint8_t* out_rgb8,
+                 std::initializer_list<HostCopy> copies, const char* what, B200rtStats& sum) {
+    const uint32_t W = cam->image_width, H = cam->image_height;
+    const cudaStream_t stream = scr->own_stream;
+    cudaError_t e = cudaSuccess;
+    if (out_rgb8) {
+        if (int rc = b200rt_resolve_rgb8_device(reinterpret_cast<const float*>(d_image), W, H, samples, scr->d_rgb, stream)) return rc;
+        sum.launches += 1;
+        e = cudaMemcpyAsync(out_rgb8, scr->d_rgb, (size_t)W * H * 3, cudaMemcpyDeviceToHost, stream);
+    }
+    for (const HostCopy& c : copies)
+        if (e == cudaSuccess && c.host && c.bytes) e = cudaMemcpyAsync(c.host, c.dev, c.bytes, cudaMemcpyDeviceToHost, stream);
+    if (e == cudaSuccess) e = cudaEventRecord(scr->call_end, stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+    if (e != cudaSuccess) return fail(B200RT_ECUDA, "%s: %s", what, cudaGetErrorString(e));
+    float ms = 0.f;
+    CU(cudaEventElapsedTime(&ms, scr->call_begin, scr->call_end));
+    sum.total_ms = ms;
+    return B200RT_OK;
+}
+
+// The denoiser's buffer of DN_PLANES x px float4: the two halves, the features (two planes) and the filter's two buffers.
+constexpr size_t DN_PLANES = 6;
+struct DenoiseBufs { float4 *a, *b, *feat, *x0, *x1; };
+DenoiseBufs carve_denoise(float4* base, size_t px) { return {base, base + px, base + 2 * px, base + 4 * px, base + 5 * px}; }
 
 // The feature pass of b200rt_render_denoised: one kernel per (accessor, slab form), shaped like the render launch (its CTA size
 // and shared-memory plan: the staged scene and the stack columns), persistent over the frame.
@@ -511,10 +583,8 @@ int launch_features(B200rtScene* sc, const B200rtCamera* cam, uint64_t seed, uin
     FeatureArgs f{};
     f.scene = sc->ds; f.cam = make_camera(*cam); f.plan = plan; f.keys = rng_keys(seed);
     f.sample_offset = sample_offset; f.k = k; f.feat = d_feat;
-    int rc = set_smem(kernel, sc, plan.bytes); if (rc) return rc;
     int blocks_per_sm = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kernel, block_threads, plan.bytes));
-    if (blocks_per_sm < 1) return fail(B200RT_ECUDA, "feature kernel does not fit on an SM (smem %u B, %u threads)", plan.bytes, block_threads);
+    if (int rc = fit_kernel(kernel, "feature kernel", sc, block_threads, plan.bytes, &blocks_per_sm)) return rc;
     const uint64_t px = (uint64_t)cam->image_width * cam->image_height;
     const uint32_t grid = (uint32_t)std::min<uint64_t>((px + block_threads - 1) / block_threads, (uint64_t)sc->sm_count * blocks_per_sm);
     kernel<<<grid, block_threads, plan.bytes, stream>>>(f);
@@ -525,15 +595,14 @@ int launch_features(B200rtScene* sc, const B200rtCamera* cam, uint64_t seed, uin
 
 // The filter on device buffers (denoise_plan.hpp): demodulation and variance into X0, then `iterations` à-trous passes between
 // X0 and X1, the last one remodulating.  *out = the buffer holding the result, {mean * n, n} per pixel.
-int launch_filter(const float4* d_a, const float4* d_b, const float4* d_feat, uint32_t W, uint32_t H, uint32_t iterations,
-                  float4* x0, float4* x1, cudaStream_t stream, float4** out, uint32_t* launches) {
+int launch_filter(const DenoiseBufs& d, uint32_t W, uint32_t H, uint32_t iterations, cudaStream_t stream, float4** out, uint32_t* launches) {
     FilterArgs f{};
-    f.acc_a = d_a; f.acc_b = d_b; f.feat = d_feat; f.W = W; f.H = H;
+    f.acc_a = d.a; f.acc_b = d.b; f.feat = d.feat; f.W = W; f.H = H;
     const dim3 block(32, 8), grid((W + 31) / 32, (H + 7) / 8);
-    f.x_out = x0;
+    f.x_out = d.x0;
     denoise_demodulate_kernel<<<grid, block, 0, stream>>>(f);
     CU(cudaGetLastError());
-    float4* buf[2] = {x0, x1};
+    float4* buf[2] = {d.x0, d.x1};
     for (uint32_t i = 0; i < iterations; ++i) {
         f.x_in = buf[i & 1u]; f.x_out = buf[(i + 1u) & 1u];
         f.step = 1u << i; f.last = i + 1 == iterations ? 1u : 0u;
@@ -877,7 +946,9 @@ int b200rt_render_device(const B200rtScene* csc, const B200rtCamera* cam, const 
     B200rtScene* sc = const_cast<B200rtScene*>(csc);
     DeviceGuard guard(sc->device);
     Scratch* scr; int rc = get_scratch(sc, cuda_stream, &scr); if (rc) return rc;
-    rc = launch_render(sc, cam, prm, d_accum, (cudaStream_t)cuda_stream, scr);
+    TileGrid g;
+    rc = check_frame(sc, cam, prm, &g);
+    if (!rc) rc = launch_render(sc, cam, prm, g, reinterpret_cast<float4*>(d_accum), (cudaStream_t)cuda_stream, scr);
     if (rc) put_scratch(sc, cuda_stream);
     return rc;
 }
@@ -889,49 +960,40 @@ int b200rt_render_device_finish(const B200rtScene* csc, void* cuda_stream, B200r
     Scratch* scr = nullptr;
     { std::lock_guard<std::mutex> lk(sc->mu); auto it = sc->inflight.find(cuda_stream); if (it != sc->inflight.end()) scr = it->second; }
     if (!scr) return fail(B200RT_EINVAL, "no render in flight on this stream");
-    int rc = finish_render(scr, (cudaStream_t)cuda_stream, scr->ev2, stats);
+    int rc = finish_render(scr, (cudaStream_t)cuda_stream, stats);
     put_scratch(sc, cuda_stream);
     return rc;
 }
 
 static int render_host_impl(const B200rtScene* csc, const B200rtCamera* cam, const B200rtRenderParams* prm, float* accum, uint8_t* out_rgb8, B200rtStats* stats) {
     B200rtScene* sc = const_cast<B200rtScene*>(csc);
-    int device = sc->device;
-    if (prm->device >= 0 && prm->device != device) return fail(B200RT_EINVAL, "params.device %d != scene device %d", prm->device, device);
-    DeviceGuard guard(device);
-    int key_local; void* key = &key_local;   // private key: concurrent host threads never collide
-    Scratch* scr; int rc = get_scratch(sc, key, &scr); if (rc) return rc;
-    size_t px = (size_t)cam->image_width * cam->image_height;
-    auto done = [&](int code) { put_scratch(sc, key); return code; };
-    if (cudaError_t e = grow(scr->d_accum, scr->accum_bytes, px * sizeof(float4)))
-        return done(fail(B200RT_ENOMEM, "accumulation buffer (%zu px): %s", px, cudaGetErrorString(e)));
-    if (out_rgb8) {
-        if (cudaError_t e = grow(scr->d_rgb, scr->rgb_bytes, px * 3)) return done(fail(B200RT_ENOMEM, "rgb8 buffer: %s", cudaGetErrorString(e)));
-    }
-    // Progressive rendering with host buffers: with B200RT_FLAG_ACCUMULATE the caller's float4 sums
-    // (an earlier call's output, or a checkpoint) are uploaded first and the new samples are added.
-    B200rtRenderParams p = *prm;
-    const bool progressive = (p.flags & B200RT_FLAG_ACCUMULATE) && accum;
-    if (!progressive) p.flags &= ~B200RT_FLAG_ACCUMULATE;
-    if (progressive) {
-        cudaError_t eu = cudaMemcpyAsync(scr->d_accum, accum, px * sizeof(float4), cudaMemcpyHostToDevice, scr->own_stream);
-        if (eu != cudaSuccess) return done(fail(B200RT_ECUDA, "H2D copy of the accumulation buffer: %s", cudaGetErrorString(eu)));
-    }
-    rc = launch_render(sc, cam, &p, reinterpret_cast<float*>(scr->d_accum), scr->own_stream, scr);
-    if (rc) return done(rc);
-    cudaError_t e = cudaSuccess;
-    if (out_rgb8) {
+    TileGrid g;
+    if (int rc = check_frame(sc, cam, prm, &g)) return rc;
+    return with_private_scratch(sc, [&](Scratch* scr) {
+        const size_t px = (size_t)cam->image_width * cam->image_height;
+        if (cudaError_t e = grow(scr->d_accum, scr->accum_bytes, px * sizeof(float4)))
+            return fail(B200RT_ENOMEM, "accumulation buffer (%zu px): %s", px, cudaGetErrorString(e));
+        if (out_rgb8) {
+            if (cudaError_t e = grow(scr->d_rgb, scr->rgb_bytes, px * 3)) return fail(B200RT_ENOMEM, "rgb8 buffer: %s", cudaGetErrorString(e));
+        }
+        // Progressive rendering with host buffers: with B200RT_FLAG_ACCUMULATE the caller's float4 sums
+        // (an earlier call's output, or a checkpoint) are uploaded first and the new samples are added.
+        B200rtRenderParams p = *prm;
+        const bool progressive = (p.flags & B200RT_FLAG_ACCUMULATE) && accum;
+        if (!progressive) p.flags &= ~B200RT_FLAG_ACCUMULATE;
+        if (progressive) {
+            cudaError_t eu = cudaMemcpyAsync(scr->d_accum, accum, px * sizeof(float4), cudaMemcpyHostToDevice, scr->own_stream);
+            if (eu != cudaSuccess) return fail(B200RT_ECUDA, "H2D copy of the accumulation buffer: %s", cudaGetErrorString(eu));
+        }
+        if (int rc = launch_render(sc, cam, &p, g, scr->d_accum, scr->own_stream, scr)) return rc;
+        B200rtStats sum{};
         // progressive: n = the summed sample count in .w
-        rc = b200rt_resolve_rgb8_device(reinterpret_cast<float*>(scr->d_accum), cam->image_width, cam->image_height, progressive ? 0 : (p.samples == 0 ? 1 : p.samples), scr->d_rgb, scr->own_stream);
-        if (rc) return done(rc);
-        scr->launches += 1;
-        e = cudaMemcpyAsync(out_rgb8, scr->d_rgb, px * 3, cudaMemcpyDeviceToHost, scr->own_stream);
-    }
-    if (e == cudaSuccess && accum) e = cudaMemcpyAsync(accum, scr->d_accum, px * sizeof(float4), cudaMemcpyDeviceToHost, scr->own_stream);
-    if (e == cudaSuccess) e = cudaEventRecord(scr->ev3, scr->own_stream);
-    if (e != cudaSuccess) return done(fail(B200RT_ECUDA, "D2H copy: %s", cudaGetErrorString(e)));
-    rc = finish_render(scr, scr->own_stream, scr->ev3, stats);
-    return done(rc);
+        int rc = finish_frame(scr, cam, scr->d_accum, progressive ? 0 : (p.samples == 0 ? 1 : p.samples), out_rgb8,
+                              {{accum, scr->d_accum, px * sizeof(float4)}}, "D2H copy", sum);
+        if (!rc) rc = add_launch(sum, scr);
+        if (!rc && stats) *stats = sum;
+        return rc;
+    });
 }
 
 int b200rt_render(const B200rtScene* csc, const B200rtCamera* cam, const B200rtRenderParams* prm, float* accum, B200rtStats* stats) {
@@ -948,12 +1010,8 @@ int b200rt_render_rgb8(const B200rtScene* csc, const B200rtCamera* cam, const B2
 // kernel (estimate, F += P, stopped tiles' pixels) and the compaction of the next list; the host reads the active count after
 // each pass.  Pass 0 adds straight into F and renders every tile; pass 1 still renders every tile, so it needs no list either.
 static int render_adaptive_impl(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderParams* prm, const B200rtAdaptiveParams* ad,
-                                float* accum, uint8_t* out_rgb8, float* tile_error, B200rtStats* stats, Scratch* scr) {
-    const uint32_t W = cam->image_width, H = cam->image_height;
-    uint32_t row_begin = prm->row_begin, row_end = prm->row_end;
-    if (row_begin == 0 && row_end == 0) row_end = H;
-    const uint32_t tiles_x = (W + TILE_W - 1) / TILE_W, tile_row0 = row_begin / TILE_H, tile_row1 = (row_end + TILE_H - 1) / TILE_H;
-    const uint32_t n_tiles = row_end > row_begin ? tiles_x * (tile_row1 - tile_row0) : 0u;
+                                const TileGrid& g, float* accum, uint8_t* out_rgb8, float* tile_error, B200rtStats* stats, Scratch* scr) {
+    const uint32_t W = cam->image_width, H = cam->image_height, n_tiles = g.n_tiles;
     const size_t px = (size_t)W * H;
     cudaError_t e = grow(scr->d_accum, scr->accum_bytes, px * sizeof(float4));
     if (e == cudaSuccess) e = grow(scr->d_fix, scr->fix_bytes, px * 3 * sizeof(long long));
@@ -966,66 +1024,46 @@ static int render_adaptive_impl(B200rtScene* sc, const B200rtCamera* cam, const 
     float* d_err = reinterpret_cast<float*>(scr->d_tiles + 3 * (size_t)n_tiles);
     uint32_t* d_count = scr->d_tiles + 4 * (size_t)n_tiles;
     cudaStream_t stream = scr->own_stream;
-    // ev3 marks the start of the call; launch_render records ev0..ev2 per pass, and ev0 is recorded again to mark the end
-    CU(cudaEventRecord(scr->ev3, stream));
+    CU(cudaEventRecord(scr->call_begin, stream));
     CU(cudaMemsetAsync(scr->d_accum, 0, px * sizeof(float4), stream));
     CU(cudaMemsetAsync(scr->d_fix, 0, px * 3 * sizeof(long long), stream));
     CU(cudaMemsetAsync(scr->d_pass, 0, px * 3 * sizeof(long long), stream));
 
     B200rtRenderParams p = *prm;
-    p.flags &= B200RT_FLAG_COUNT_TRAVERSAL; p.shard_count = 1; p.shard_index = 0; p.row_begin = row_begin; p.row_end = row_end;
+    p.flags &= B200RT_FLAG_COUNT_TRAVERSAL; p.shard_count = 1; p.shard_index = 0;
     B200rtStats sum{};
-    uint32_t n_prev = 0, active = n_tiles, launches = 0, which = 0;
+    uint32_t n_prev = 0, active = n_tiles, which = 0;
     const uint32_t* list = nullptr;
     for (uint32_t k = 0; active > 0; ++k) {
         const uint32_t n = adaptive_samples_after(ad->initial_samples, ad->max_samples, k);
         p.samples = n - n_prev; p.sample_offset = prm->sample_offset + n_prev;
-        const AdaptivePass pass{list, active, k == 0 ? scr->d_fix : scr->d_pass, ad->max_samples};
-        if (int rc = launch_render(sc, cam, &p, reinterpret_cast<float*>(scr->d_accum), stream, scr, &pass)) return rc;
-        launches += scr->launches;
         uint32_t next = active;
-        if (k > 0) {
+        const int rc = run_pass(sc, cam, &p, g, {list, active, k == 0 ? scr->d_fix : scr->d_pass, ad->max_samples}, scr, sum, [&] {
+            if (k == 0) return B200RT_OK;
             MergeArgs m{};
             m.list = list; m.n_active = active; m.F = scr->d_fix; m.P = scr->d_pass; m.accum = scr->d_accum; m.tile_error = d_err; m.keep = keep;
             m.n = n_prev; m.s = n - n_prev; m.last = n == ad->max_samples ? 1u : 0u; m.threshold = ad->threshold;
-            m.W = W; m.row_begin = row_begin; m.row_end = row_end; m.tiles_x = tiles_x; m.tile_row0 = tile_row0;
+            m.W = W; m.row_begin = g.row_begin; m.row_end = g.row_end; m.tiles_x = g.tiles_x; m.tile_row0 = g.tile_row0;
             adaptive_merge_kernel<<<(active + 7) / 8, 256, 0, stream>>>(m);
             CU(cudaGetLastError());
             adaptive_compact_kernel<<<1, COMPACT_THREADS, 0, stream>>>(list, keep, active, lists[which], d_count);
             CU(cudaGetLastError());
-            launches += 2;
+            sum.launches += 2;
             CU(cudaMemcpyAsync(&next, d_count, sizeof next, cudaMemcpyDeviceToHost, stream));
-        }
-        CU(cudaStreamSynchronize(stream));
-        const Counters& c = *scr->h_counters;
-        sum.rays += c.rays; sum.paths += c.paths; sum.node_visits += c.nodes; sum.prim_tests += c.prims; sum.depth_exhausted += c.exhausted;
-        for (int d = 0; d < 8; ++d) sum.diag[d] += c.diag[d];
-        float ms = 0.f;
-        CU(cudaEventElapsedTime(&ms, scr->ev1, scr->ev2)); sum.kernel_ms += ms;
+            return B200RT_OK;
+        });
+        if (rc) return rc;
         if (k > 0) { list = lists[which]; which ^= 1u; }
         active = next; n_prev = n;
     }
-    if (out_rgb8) {
-        if (int rc = b200rt_resolve_rgb8_device(reinterpret_cast<float*>(scr->d_accum), W, H, 0, scr->d_rgb, stream)) return rc;
-        launches += 1;
-        e = cudaMemcpyAsync(out_rgb8, scr->d_rgb, px * 3, cudaMemcpyDeviceToHost, stream);
-    }
-    if (e == cudaSuccess && accum) e = cudaMemcpyAsync(accum, scr->d_accum, px * sizeof(float4), cudaMemcpyDeviceToHost, stream);
-    if (e == cudaSuccess && tile_error) {
-        // tiles with no selected pixel: -1; the others sit in one contiguous block of tile rows
-        std::fill(tile_error, tile_error + (size_t)tiles_x * ((H + TILE_H - 1) / TILE_H), -1.0f);
-        if (n_tiles) e = cudaMemcpyAsync(tile_error + (size_t)tile_row0 * tiles_x, d_err, n_tiles * sizeof(float), cudaMemcpyDeviceToHost, stream);
-    }
-    if (e == cudaSuccess) e = cudaEventRecord(scr->ev0, stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
-    if (e != cudaSuccess) return fail(B200RT_ECUDA, "adaptive sampling copy-back: %s", cudaGetErrorString(e));
-    if (stats) {
-        float ms = 0.f;
-        CU(cudaEventElapsedTime(&ms, scr->ev3, scr->ev0));
-        sum.total_ms = ms;
-        sum.launches = launches;
-        *stats = sum;
-    }
+    // tiles with no selected pixel: -1; the others sit in one contiguous block of tile rows
+    if (tile_error) std::fill(tile_error, tile_error + (size_t)g.tiles_x * ((H + TILE_H - 1) / TILE_H), -1.0f);
+    if (int rc = finish_frame(scr, cam, scr->d_accum, 0, out_rgb8,
+                              {{accum, scr->d_accum, px * sizeof(float4)},
+                               {tile_error ? tile_error + (size_t)g.tile_row0 * g.tiles_x : nullptr, d_err, n_tiles * sizeof(float)}},
+                              "adaptive sampling copy-back", sum))
+        return rc;
+    if (stats) *stats = sum;
     return B200RT_OK;
 }
 
@@ -1038,88 +1076,48 @@ int b200rt_render_adaptive(const B200rtScene* csc, const B200rtCamera* cam, cons
     if (ad->max_samples <= ad->initial_samples) return fail(B200RT_EINVAL, "adaptive max_samples %u must exceed initial_samples %u", ad->max_samples, ad->initial_samples);
     if (!(ad->threshold >= 0.0f) || !std::isfinite(ad->threshold)) return fail(B200RT_EINVAL, "adaptive threshold %g must be finite and >= 0", (double)ad->threshold);
     B200rtScene* sc = const_cast<B200rtScene*>(csc);
-    if (prm->device >= 0 && prm->device != sc->device) return fail(B200RT_EINVAL, "params.device %d != scene device %d", prm->device, sc->device);
-    const uint32_t W = cam->image_width, H = cam->image_height;
-    if (W == 0 || H == 0) return fail(B200RT_EINVAL, "camera image dimensions are zero");
-    if ((uint64_t)W * H > 0xFFFFFFFFull) return fail(B200RT_EINVAL, "image too large");
-    const uint32_t row_end = prm->row_begin == 0 && prm->row_end == 0 ? H : prm->row_end;
-    if (row_end > H || prm->row_begin > row_end) return fail(B200RT_EINVAL, "row range [%u,%u) outside image height %u", prm->row_begin, row_end, H);
-
-    DeviceGuard guard(sc->device);
-    int key_local; void* key = &key_local;   // private key: concurrent host threads never collide
-    Scratch* scr; int rc = get_scratch(sc, key, &scr); if (rc) return rc;
-    rc = render_adaptive_impl(sc, cam, prm, ad, accum, out_rgb8, tile_error, stats, scr);
-    if (rc) cudaStreamSynchronize(scr->own_stream);   // nothing of a failed call may still run when its scratch is reused
-    scr->launched = false;
-    put_scratch(sc, key);
-    return rc;
+    TileGrid g;
+    if (int rc = check_frame(sc, cam, prm, &g)) return rc;
+    return with_private_scratch(sc, [&](Scratch* scr) { return render_adaptive_impl(sc, cam, prm, ad, g, accum, out_rgb8, tile_error, stats, scr); });
 }
 
-// Denoised render (b200rt_render_denoised): the two halves [0, h) and [h, n) as two K2 launches into the fixed-point buffers
-// F and P (the adaptive pass mechanism over all tiles, clamp taken for n), their float4 forms and the whole render's, the
-// feature pass, the filter, the optional resolve and the copies.
+// Denoised render (b200rt_render_denoised): the two halves [0, h) and [h, n) as two K2 passes into the fixed-point buffers
+// F and P (over all tiles, clamp taken for n), their float4 forms and the whole render's, the feature pass, the filter, the
+// optional resolve and the copies.
 static int render_denoised_impl(B200rtScene* sc, const B200rtCamera* cam, const B200rtRenderParams* prm, const B200rtDenoiseParams* dn,
-                                float* accum, float* denoised, float* features, uint8_t* out_rgb8, B200rtStats* stats, Scratch* scr) {
+                                const TileGrid& g, float* accum, float* denoised, float* features, uint8_t* out_rgb8, B200rtStats* stats, Scratch* scr) {
     const uint32_t W = cam->image_width, H = cam->image_height;
     const uint32_t n = prm->samples, h = n / 2;
-    const uint32_t n_tiles = ((W + TILE_W - 1) / TILE_W) * ((H + TILE_H - 1) / TILE_H);
     const size_t px = (size_t)W * H;
     cudaError_t e = grow(scr->d_accum, scr->accum_bytes, px * sizeof(float4));
     if (e == cudaSuccess) e = grow(scr->d_fix, scr->fix_bytes, px * 3 * sizeof(long long));
     if (e == cudaSuccess) e = grow(scr->d_pass, scr->pass_bytes, px * 3 * sizeof(long long));
-    if (e == cudaSuccess) e = grow(scr->d_denoise, scr->denoise_bytes, px * 6 * sizeof(float4));
+    if (e == cudaSuccess) e = grow(scr->d_denoise, scr->denoise_bytes, px * DN_PLANES * sizeof(float4));
     if (e == cudaSuccess && out_rgb8) e = grow(scr->d_rgb, scr->rgb_bytes, px * 3);
     if (e != cudaSuccess) return fail(B200RT_ENOMEM, "denoising buffers (%zu px): %s", px, cudaGetErrorString(e));
-    float4* d_a = scr->d_denoise;
-    float4* d_b = d_a + px;
-    float4* d_feat = d_b + px;          // two planes
-    float4* x0 = d_feat + 2 * px;
-    float4* x1 = x0 + px;
+    const DenoiseBufs d = carve_denoise(scr->d_denoise, px);
     cudaStream_t stream = scr->own_stream;
-    // ev3 marks the start of the call; launch_render records ev0..ev2 per half, and ev0 is recorded again to mark the end
-    CU(cudaEventRecord(scr->ev3, stream));
+    CU(cudaEventRecord(scr->call_begin, stream));
     CU(cudaMemsetAsync(scr->d_fix, 0, px * 3 * sizeof(long long), stream));
     CU(cudaMemsetAsync(scr->d_pass, 0, px * 3 * sizeof(long long), stream));
     B200rtRenderParams p = *prm;
-    p.flags &= B200RT_FLAG_COUNT_TRAVERSAL; p.shard_count = 1; p.shard_index = 0; p.row_begin = 0; p.row_end = H;
+    p.flags &= B200RT_FLAG_COUNT_TRAVERSAL; p.shard_count = 1; p.shard_index = 0;
     B200rtStats sum{};
-    uint32_t launches = 0;
     for (uint32_t half = 0; half < 2; ++half) {
         p.samples = half ? n - h : h; p.sample_offset = prm->sample_offset + (half ? h : 0u);
-        const AdaptivePass pass{nullptr, n_tiles, half ? scr->d_pass : scr->d_fix, n};
-        if (int rc = launch_render(sc, cam, &p, reinterpret_cast<float*>(scr->d_accum), stream, scr, &pass)) return rc;
-        launches += scr->launches;
-        CU(cudaStreamSynchronize(stream));   // the counters and events of this half
-        const Counters& c = *scr->h_counters;
-        sum.rays += c.rays; sum.paths += c.paths; sum.node_visits += c.nodes; sum.prim_tests += c.prims; sum.depth_exhausted += c.exhausted;
-        for (int d = 0; d < 8; ++d) sum.diag[d] += c.diag[d];
-        float ms = 0.f;
-        CU(cudaEventElapsedTime(&ms, scr->ev1, scr->ev2)); sum.kernel_ms += ms;
+        if (int rc = run_pass(sc, cam, &p, g, {nullptr, g.n_tiles, half ? scr->d_pass : scr->d_fix, n}, scr, sum, [] { return B200RT_OK; })) return rc;
     }
-    denoise_halves_kernel<<<(unsigned)((px + 255) / 256), 256, 0, stream>>>(scr->d_fix, scr->d_pass, (uint32_t)px, h, n - h, d_a, d_b, scr->d_accum);
+    denoise_halves_kernel<<<(unsigned)((px + 255) / 256), 256, 0, stream>>>(scr->d_fix, scr->d_pass, (uint32_t)px, h, n - h, d.a, d.b, scr->d_accum);
     CU(cudaGetLastError());
-    launches += 1;
-    if (int rc = launch_features(sc, cam, prm->seed, prm->sample_offset, dn->feature_samples, d_feat, stream, &launches)) return rc;
+    sum.launches += 1;
+    if (int rc = launch_features(sc, cam, prm->seed, prm->sample_offset, dn->feature_samples, d.feat, stream, &sum.launches)) return rc;
     float4* d_out = nullptr;
-    if (int rc = launch_filter(d_a, d_b, d_feat, W, H, dn->iterations, x0, x1, stream, &d_out, &launches)) return rc;
-    if (out_rgb8) {
-        if (int rc = b200rt_resolve_rgb8_device(reinterpret_cast<float*>(d_out), W, H, 0, scr->d_rgb, stream)) return rc;
-        launches += 1;
-        e = cudaMemcpyAsync(out_rgb8, scr->d_rgb, px * 3, cudaMemcpyDeviceToHost, stream);
-    }
-    if (e == cudaSuccess && accum) e = cudaMemcpyAsync(accum, scr->d_accum, px * sizeof(float4), cudaMemcpyDeviceToHost, stream);
-    if (e == cudaSuccess && denoised) e = cudaMemcpyAsync(denoised, d_out, px * sizeof(float4), cudaMemcpyDeviceToHost, stream);
-    if (e == cudaSuccess && features) e = cudaMemcpyAsync(features, d_feat, 2 * px * sizeof(float4), cudaMemcpyDeviceToHost, stream);
-    if (e == cudaSuccess) e = cudaEventRecord(scr->ev0, stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
-    if (e != cudaSuccess) return fail(B200RT_ECUDA, "denoised render: %s", cudaGetErrorString(e));
-    if (stats) {
-        float ms = 0.f;
-        CU(cudaEventElapsedTime(&ms, scr->ev3, scr->ev0));
-        sum.total_ms = ms;
-        sum.launches = launches;
-        *stats = sum;
-    }
+    if (int rc = launch_filter(d, W, H, dn->iterations, stream, &d_out, &sum.launches)) return rc;
+    if (int rc = finish_frame(scr, cam, d_out, 0, out_rgb8,
+                              {{accum, scr->d_accum, px * sizeof(float4)}, {denoised, d_out, px * sizeof(float4)}, {features, d.feat, 2 * px * sizeof(float4)}},
+                              "denoised render", sum))
+        return rc;
+    if (stats) *stats = sum;
     return B200RT_OK;
 }
 
@@ -1134,21 +1132,14 @@ int b200rt_render_denoised(const B200rtScene* csc, const B200rtCamera* cam, cons
     if (prm->flags & B200RT_FLAG_ACCUMULATE) return fail(B200RT_EINVAL, "a denoised render cannot add to an earlier result (B200RT_FLAG_ACCUMULATE)");
     if (prm->shard_count > 1) return fail(B200RT_EINVAL, "the denoiser needs every neighbour: shard_count %u is not supported", prm->shard_count);
     B200rtScene* sc = const_cast<B200rtScene*>(csc);
-    if (prm->device >= 0 && prm->device != sc->device) return fail(B200RT_EINVAL, "params.device %d != scene device %d", prm->device, sc->device);
-    const uint32_t W = cam->image_width, H = cam->image_height;
-    if (W == 0 || H == 0) return fail(B200RT_EINVAL, "camera image dimensions are zero");
-    if ((uint64_t)W * H > 0xFFFFFFFFull) return fail(B200RT_EINVAL, "image too large");
-    if (!(prm->row_begin == 0 && (prm->row_end == 0 || prm->row_end == H)))
-        return fail(B200RT_EINVAL, "the denoiser needs every neighbour: row range [%u,%u) is not the whole frame of %u rows", prm->row_begin, prm->row_end, H);
-
-    DeviceGuard guard(sc->device);
-    int key_local; void* key = &key_local;   // private key: concurrent host threads never collide
-    Scratch* scr; int rc = get_scratch(sc, key, &scr); if (rc) return rc;
-    rc = render_denoised_impl(sc, cam, prm, dn, accum, denoised, features, out_rgb8, stats, scr);
-    if (rc) cudaStreamSynchronize(scr->own_stream);   // nothing of a failed call may still run when its scratch is reused
-    scr->launched = false;
-    put_scratch(sc, key);
-    return rc;
+    // the frame is checked as the whole frame it renders; the row range of the call must say the same
+    B200rtRenderParams whole = *prm;
+    whole.row_begin = whole.row_end = 0;
+    TileGrid g;
+    if (int rc = check_frame(sc, cam, &whole, &g)) return rc;
+    if (!(prm->row_begin == 0 && (prm->row_end == 0 || prm->row_end == cam->image_height)))
+        return fail(B200RT_EINVAL, "the denoiser needs every neighbour: row range [%u,%u) is not the whole frame of %u rows", prm->row_begin, prm->row_end, cam->image_height);
+    return with_private_scratch(sc, [&](Scratch* scr) { return render_denoised_impl(sc, cam, prm, dn, g, accum, denoised, features, out_rgb8, stats, scr); });
 }
 
 int b200rt_denoise(const float* accum_a, const float* accum_b, const float* features, uint32_t W, uint32_t H, uint32_t iterations,
@@ -1161,20 +1152,16 @@ int b200rt_denoise(const float* accum_a, const float* accum_b, const float* feat
     DeviceGuard guard(device);
     const size_t px = (size_t)W * H;
     DevBuf buf;
-    if ((rc = buf.alloc(px * 6 * sizeof(float4)))) return rc;
-    float4* d_a = buf.as<float4>();
-    float4* d_b = d_a + px;
-    float4* d_feat = d_b + px;
-    float4* x0 = d_feat + 2 * px;
-    float4* x1 = x0 + px;
+    if ((rc = buf.alloc(px * DN_PLANES * sizeof(float4)))) return rc;
+    const DenoiseBufs d = carve_denoise(buf.as<float4>(), px);
     cudaStream_t stream = nullptr;
     CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-    cudaError_t e = cudaMemcpyAsync(d_a, accum_a, px * sizeof(float4), cudaMemcpyHostToDevice, stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_b, accum_b, px * sizeof(float4), cudaMemcpyHostToDevice, stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_feat, features, 2 * px * sizeof(float4), cudaMemcpyHostToDevice, stream);
+    cudaError_t e = cudaMemcpyAsync(d.a, accum_a, px * sizeof(float4), cudaMemcpyHostToDevice, stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d.b, accum_b, px * sizeof(float4), cudaMemcpyHostToDevice, stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d.feat, features, 2 * px * sizeof(float4), cudaMemcpyHostToDevice, stream);
     float4* d_out = nullptr;
     uint32_t launches = 0;
-    if (e == cudaSuccess) rc = launch_filter(d_a, d_b, d_feat, W, H, iterations, x0, x1, stream, &d_out, &launches);
+    if (e == cudaSuccess) rc = launch_filter(d, W, H, iterations, stream, &d_out, &launches);
     if (e == cudaSuccess && rc == B200RT_OK) e = cudaMemcpyAsync(out, d_out, px * sizeof(float4), cudaMemcpyDeviceToHost, stream);
     const cudaError_t es = cudaStreamSynchronize(stream);
     cudaStreamDestroy(stream);
@@ -1535,10 +1522,8 @@ int b200rt_closest_hit(const B200rtScene* csc, const B200rtRay* rays, size_t n, 
     // traversal counters ride along with the full hit records (parity runs); ids-only calls — the BVH microbenchmark
     // shape of benches/my_benchmark.rs — run the kernel without them
     HitKernel kernel = hit_kernel(plan.all_in_smem, use_fast_slab(sc, max_origin, min_dir_inf), stats != nullptr && hits != nullptr);
-    if ((rc = set_smem(kernel, sc, plan.bytes))) return rc;
     int bps = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kernel, BLOCK, plan.bytes));
-    if (bps < 1) return fail(B200RT_ECUDA, "closest_hit_kernel does not fit on an SM");
+    if ((rc = fit_kernel(kernel, "closest_hit_kernel", sc, BLOCK, plan.bytes, &bps))) return rc;
     size_t want = (n + BLOCK - 1) / BLOCK;
     uint32_t grid = (uint32_t)std::min<size_t>(want, (size_t)sc->sm_count * bps);      // persistent: one wave of CTAs
     cudaEvent_t e0, e1; CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));

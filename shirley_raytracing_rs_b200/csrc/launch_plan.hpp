@@ -19,6 +19,21 @@ constexpr uint32_t RAYQ_SLOTS = 32, RAYQ_FIELDS = 9;   // v2: o, d, RNG state + 
 // way measured 3 % slower).
 constexpr int SMEM_NODE_QUADS = 5;
 
+// The 8x4 tiles that cover rows [row_begin, row_end) of a W x H frame, (0, 0) meaning the whole frame.  `ok` is false for a
+// range outside the image; an empty range covers no tile.
+struct TileGrid { bool ok; uint32_t row_begin, row_end, tiles_x, tile_row0, n_tiles; };
+
+inline TileGrid tile_grid(uint32_t W, uint32_t H, uint32_t row_begin, uint32_t row_end) {
+    TileGrid g{};
+    g.row_begin = row_begin;
+    g.row_end = row_begin == 0 && row_end == 0 ? H : row_end;
+    g.ok = g.row_end <= H && g.row_begin <= g.row_end;
+    g.tiles_x = (W + TILE_W - 1) / TILE_W;
+    g.tile_row0 = g.row_begin / TILE_H;
+    g.n_tiles = g.ok && g.row_end > g.row_begin ? g.tiles_x * ((g.row_end + TILE_H - 1) / TILE_H - g.tile_row0) : 0u;
+    return g;
+}
+
 struct SmemPlan {
     uint32_t all_in_smem;           // 1: nodes + geom + mats + tex all staged (SmemAcc)
     uint32_t n_top;                 // nodes staged when !all_in_smem

@@ -105,5 +105,37 @@ int main() {
         CHECK(render_grid(148, 0, 1, 24) == 1);
         report("render grid", before);
     }
+    {
+        int before = failures;
+        TileGrid g = tile_grid(1200, 800, 0, 0);                      // (0, 0): the whole frame
+        CHECK(g.ok && g.row_begin == 0 && g.row_end == 800 && g.tiles_x == 150 && g.tile_row0 == 0 && g.n_tiles == weekend);
+        g = tile_grid(97, 61, 0, 0);                                  // ragged: partial tiles on the right and at the bottom
+        CHECK(g.ok && g.row_end == 61 && g.tiles_x == 13 && g.n_tiles == 13 * 16);
+        g = tile_grid(7, 3, 0, 3);
+        CHECK(g.ok && g.tiles_x == 1 && g.n_tiles == 1);
+        for (uint32_t r : {1u, 8u, 9u, 61u}) {                        // empty ranges cover no tile
+            g = tile_grid(97, 61, r, r);
+            CHECK(g.ok && g.n_tiles == 0 && g.row_begin == r && g.row_end == r);
+        }
+        g = tile_grid(97, 61, 5, 10);                                 // [5, 10) ends mid-tile: tile rows 1 and 2
+        CHECK(g.ok && g.tile_row0 == 1 && g.n_tiles == 13 * 2);
+        g = tile_grid(97, 61, 0, 62);                                 // outside the image
+        CHECK(!g.ok && g.row_end == 62 && g.n_tiles == 0);
+        g = tile_grid(97, 61, 10, 5);
+        CHECK(!g.ok && g.n_tiles == 0);
+        g = tile_grid(97, 61, 62, 0);
+        CHECK(!g.ok && g.row_end == 0);
+        // every non-empty range: the grid the render launch computed before it took it from tile_grid
+        for (uint32_t W : {1u, 7u, 8u, 9u, 97u})
+            for (uint32_t H : {1u, 3u, 4u, 5u, 61u})
+                for (uint32_t r0 = 0; r0 < H; ++r0)
+                    for (uint32_t r1 = r0 + 1; r1 <= H; ++r1) {
+                        g = tile_grid(W, H, r0, r1);
+                        const uint32_t tiles_x = (W + TILE_W - 1) / TILE_W, tile_row0 = r0 / TILE_H, tile_row1 = (r1 + TILE_H - 1) / TILE_H;
+                        CHECK(g.ok && g.row_begin == r0 && g.row_end == r1 && g.tiles_x == tiles_x && g.tile_row0 == tile_row0 &&
+                              g.n_tiles == tiles_x * (tile_row1 - tile_row0));
+                    }
+        report("tile grid", before);
+    }
     return failures ? 1 : 0;
 }
