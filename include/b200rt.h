@@ -432,16 +432,24 @@ int  b200rt_closest_hit(const B200rtScene* scene, const B200rtRay* rays, size_t 
 int  b200rt_aabb_hit(const float* boxes6, const B200rtRay* rays, size_t n,
                      float t_min, float t_max, uint8_t* out, int device);
 
+/* Random streams of the scatter and camera hooks.  `stream` NULL: record i draws from the stream
+ * b200rt_rng(seed, i, 0) (see b200rt_rng_uniforms).  Otherwise stream[3*i .. 3*i+2] = (a, b, skip):
+ * record i draws from b200rt_rng(seed, a, b) after discarding its first `skip` draws.  With
+ * a = pixel and b = sample index, that continues the render's own stream of that path (draws 0 and 1
+ * jitter the pixel, the lens draws follow, then each bounce's scatter draws). */
+
 /* K4: Material::scatter + ::emitted (material_type.rs:50-79) for hit records `hits`
- * produced by incoming rays `rays`; the material is materials[hits[i].id]. Record i draws
- * its random numbers from the stream b200rt_rng(seed, i, 0) (see below). */
+ * produced by incoming rays `rays`; the material is materials[hits[i].id]; `stream` may be NULL
+ * (see above).  A record with hits[i].id == -1 is a miss: emitted = Skybox::background(rays[i].d)
+ * exactly as the render kernel computes it, scattered = 0, draws = 0, attenuation = 0. */
 int  b200rt_scatter(const B200rtScene* scene, const B200rtRay* rays, const B200rtHit* hits,
-                    size_t n, uint64_t seed, B200rtScatter* out);
+                    size_t n, uint64_t seed, const uint32_t* stream, B200rtScatter* out);
 
 /* Camera::pixel_ray (camera/mod.rs:98-131) for pixel coordinates xy[2*i], xy[2*i+1]
- * (already jittered); record i draws the lens sample from stream b200rt_rng(seed, i, 0). */
+ * (already jittered); record i draws the lens sample from its stream (see above; may be NULL).
+ * `draws` (may be NULL): the number of lens draws record i took (0 without a lens). */
 int  b200rt_camera_rays(const B200rtCamera* camera, const float* xy, size_t n, uint64_t seed,
-                        B200rtRay* out, int device);
+                        const uint32_t* stream, B200rtRay* out, uint32_t* draws, int device);
 
 /* Texture::value (material/texture/mod.rs:8-10) of textures[tex] at (u, v, p). */
 int  b200rt_texture_value(const B200rtScene* scene, int32_t tex, const float* uvp5, size_t n,

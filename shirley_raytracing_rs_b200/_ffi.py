@@ -159,8 +159,8 @@ SIGNATURES = {
     "b200rt_free": (None, [C.c_void_p]),
     "b200rt_closest_hit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_float, C.c_float, C.c_void_p, C.c_void_p, _P(Stats)]),
     "b200rt_aabb_hit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_float, C.c_float, C.c_void_p, C.c_int]),
-    "b200rt_scatter": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint64, C.c_void_p]),
-    "b200rt_camera_rays": (C.c_int, [_P(Camera), C.c_void_p, C.c_size_t, C.c_uint64, C.c_void_p, C.c_int]),
+    "b200rt_scatter": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint64, C.c_void_p, C.c_void_p]),
+    "b200rt_camera_rays": (C.c_int, [_P(Camera), C.c_void_p, C.c_size_t, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "b200rt_texture_value": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]),
     "b200rt_rng_uniforms": (C.c_int, [C.c_uint64, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p, C.c_int]),
     "b200rt_fp32_peak": (C.c_int, [C.c_int, _P(C.c_double)]),

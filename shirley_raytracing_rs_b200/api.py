@@ -475,19 +475,38 @@ def aabb_hit(boxes6, rays, t_min=0.0, t_max=float("inf"), device: int = -1) -> n
     return out.astype(bool)
 
 
-def scatter(scene: Scene, rays, hits: np.ndarray, seed: int = 0, device: int = -1) -> np.ndarray:
+def _as_stream(stream, n: int):
+    """None, or (n, 3) uint32 stream positions (a, b, skip): record i draws from stream (seed, a, b) after `skip` draws."""
+    if stream is None:
+        return None
+    s = np.ascontiguousarray(stream, dtype=np.uint32)
+    if s.shape != (n, 3):
+        raise ValueError(f"stream must have shape ({n}, 3)")
+    return s
+
+
+def scatter(scene: Scene, rays, hits: np.ndarray, seed: int = 0, device: int = -1, *, stream=None) -> np.ndarray:
+    """Material::scatter + ::emitted per record (b200rt_scatter); a record with id -1 is a miss and returns the
+    background of its direction as `emitted`.  `stream`: see _as_stream (None: record i draws from (seed, i, 0))."""
     r = as_rays(rays)
     h = np.ascontiguousarray(hits, dtype=HIT_DTYPE)
+    s = _as_stream(stream, r.shape[0])
     out = np.zeros(r.shape[0], dtype=SCATTER_DTYPE)
-    F.check(lib.b200rt_scatter(scene.device(device), r.ctypes.data, h.ctypes.data, r.shape[0], seed, out.ctypes.data))
+    F.check(lib.b200rt_scatter(scene.device(device), r.ctypes.data, h.ctypes.data, r.shape[0], seed,
+                               None if s is None else s.ctypes.data, out.ctypes.data))
     return out
 
 
-def camera_rays(cam: F.Camera, xy, seed: int = 0, device: int = -1) -> np.ndarray:
+def camera_rays(cam: F.Camera, xy, seed: int = 0, device: int = -1, *, stream=None, with_draws: bool = False):
+    """Camera::pixel_ray for jittered pixel coordinates (b200rt_camera_rays): rays float32[n, 6], and with `with_draws`
+    also the lens draws each record took (uint32[n]).  `stream`: see _as_stream (None: record i draws from (seed, i, 0))."""
     xy = np.ascontiguousarray(xy, dtype=np.float32)
+    s = _as_stream(stream, xy.shape[0])
     out = np.empty((xy.shape[0], 6), dtype=np.float32)
-    F.check(lib.b200rt_camera_rays(C.byref(cam), xy.ctypes.data, xy.shape[0], seed, out.ctypes.data, device))
-    return out
+    draws = np.empty(xy.shape[0], dtype=np.uint32) if with_draws else None
+    F.check(lib.b200rt_camera_rays(C.byref(cam), xy.ctypes.data, xy.shape[0], seed, None if s is None else s.ctypes.data,
+                                   out.ctypes.data, None if draws is None else draws.ctypes.data, device))
+    return (out, draws) if with_draws else out
 
 
 def texture_value(scene: Scene, tex: int, uvp, device: int = -1) -> np.ndarray:

@@ -222,7 +222,23 @@ __global__ void aabb_hit_kernel(const float* __restrict__ boxes6, const B200rtRa
     out[i] = aabb_hit2(ray, b[0], b[1], b[2], b[3], b[4], b[5], t_min, t_max, &e) ? 1 : 0;
 }
 
-struct ScatterArgs { DeviceScene scene; const B200rtRay* rays; const B200rtHit* hits; size_t n; RngKeys keys; B200rtScatter* out; };
+// The hooks' random stream of record i: b200rt_rng(seed, i, 0), or with `stream` (three words per record) b200rt_rng(seed, a, b)
+// after `skip` draws, which continues a render's path stream (pixel, sample) where the render is.
+__device__ __forceinline__ Rng hook_rng(RngKeys keys, const uint32_t* stream, size_t i) {
+    Rng rng;
+    if (!stream) { rng.init(keys, (uint32_t)i, 0u); return rng; }
+    rng.init(keys, stream[3 * i], stream[3 * i + 1]);
+    for (uint32_t k = stream[3 * i + 2]; k != 0u; --k) rng.state = rng.state * 747796405u + rng.inc;
+    return rng;
+}
+// draws taken since the state was s0 = LCG steps from s0 to rng.state, recounted by stepping
+__device__ __forceinline__ uint32_t draws_since(uint32_t s0, const Rng& rng) {
+    uint32_t st = s0, k = 0;
+    while (st != rng.state && k < 4096) { st = st * 747796405u + rng.inc; ++k; }
+    return k;
+}
+
+struct ScatterArgs { DeviceScene scene; const B200rtRay* rays; const B200rtHit* hits; size_t n; RngKeys keys; const uint32_t* stream; B200rtScatter* out; };
 __global__ void scatter_kernel(const __grid_constant__ ScatterArgs a) {
     // The render kernel's own shading sequence: shade_prepare -> warp-cooperative Perlin -> shade_finish.
     // No early return: coop_turbulence is a warp collective (the grid is rounded up to whole warps).
@@ -249,7 +265,7 @@ __global__ void scatter_kernel(const __grid_constant__ ScatterArgs a) {
     float turb = 0.0f;
     if (a.scene.perlin != nullptr && __any_sync(0xffffffffu, need)) turb = coop_turbulence(a.scene.perlin, need, h.p, sp.tex.perlin_idx);
     if (valid) {
-        Rng rng; rng.init(a.keys, (uint32_t)i, 0u);
+        Rng rng = hook_rng(a.keys, a.stream, i);
         uint32_t s0 = rng.state;
         float3 atten = f3(1, 1, 1), emit = f3(0, 0, 0);
         float3 albedo = sp.tex.need_perlin ? marble(sp.tex.perlin_scale, h.p, turb) : sp.tex.rgb;
@@ -261,22 +277,25 @@ __global__ void scatter_kernel(const __grid_constant__ ScatterArgs a) {
         out.attenuation[0] = atten.x; out.attenuation[1] = atten.y; out.attenuation[2] = atten.z;
         out.emitted[0] = emit.x; out.emitted[1] = emit.y; out.emitted[2] = emit.z;
         out.scattered = so.scattered ? 1 : 0;
-        // draws consumed = LCG steps between s0 and rng.state: recount by stepping
-        uint32_t st = s0, k = 0;
-        while (st != rng.state && k < 4096) { st = st * 747796405u + rng.inc; ++k; }
-        out.draws = k;
+        out.draws = draws_since(s0, rng);
+    } else if (in_range && hi.id == -1) {        // a miss: the render kernel's background for the ray's direction
+        const float3 bg = background(a.scene, ray.d);
+        out.emitted[0] = bg.x; out.emitted[1] = bg.y; out.emitted[2] = bg.z;
     }
     if (in_range) a.out[i] = out;
 }
 
-__global__ void camera_rays_kernel(DeviceCamera cam, const float* __restrict__ xy, size_t n, RngKeys keys, B200rtRay* out) {
+__global__ void camera_rays_kernel(DeviceCamera cam, const float* __restrict__ xy, size_t n, RngKeys keys, const uint32_t* stream,
+                                   B200rtRay* out, uint32_t* draws) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    Rng rng; rng.init(keys, (uint32_t)i, 0u);
+    Rng rng = hook_rng(keys, stream, i);
+    const uint32_t s0 = rng.state;
     float3 o, d;
     pixel_ray(cam, rng, xy[2 * i], xy[2 * i + 1], &o, &d);
     B200rtRay r; r.ox = o.x; r.oy = o.y; r.oz = o.z; r.dx = d.x; r.dy = d.y; r.dz = d.z;
     out[i] = r;
+    if (draws) draws[i] = draws_since(s0, rng);
 }
 
 struct TexArgs { DeviceScene scene; int32_t tex; const float* uvp5; size_t n; float* out; };

@@ -1562,33 +1562,43 @@ int b200rt_aabb_hit(const float* boxes6, const B200rtRay* rays, size_t n, float 
     return B200RT_OK;
 }
 
-int b200rt_scatter(const B200rtScene* csc, const B200rtRay* rays, const B200rtHit* hits, size_t n, uint64_t seed, B200rtScatter* out) {
+int b200rt_scatter(const B200rtScene* csc, const B200rtRay* rays, const B200rtHit* hits, size_t n, uint64_t seed, const uint32_t* stream,
+                   B200rtScatter* out) {
     if (!csc || (n && (!rays || !hits || !out))) return fail(B200RT_EINVAL, "NULL argument");
     B200rtScene* sc = const_cast<B200rtScene*>(csc);
     DeviceGuard guard(sc->device);
     if (n == 0) return B200RT_OK;
-    DevBuf r, h, o; int rc;
+    DevBuf r, h, o, s; int rc;
     if ((rc = r.alloc(n * sizeof(B200rtRay))) || (rc = h.alloc(n * sizeof(B200rtHit))) || (rc = o.alloc(n * sizeof(B200rtScatter)))) return rc;
+    if (stream && (rc = s.alloc(n * 12))) return rc;
     CU(cudaMemcpy(r.p, rays, n * sizeof(B200rtRay), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(h.p, hits, n * sizeof(B200rtHit), cudaMemcpyHostToDevice));
-    ScatterArgs a{}; a.scene = sc->ds; a.rays = r.as<B200rtRay>(); a.hits = h.as<B200rtHit>(); a.n = n; a.keys = rng_keys(seed); a.out = o.as<B200rtScatter>();
+    if (stream) CU(cudaMemcpy(s.p, stream, n * 12, cudaMemcpyHostToDevice));
+    ScatterArgs a{}; a.scene = sc->ds; a.rays = r.as<B200rtRay>(); a.hits = h.as<B200rtHit>(); a.n = n; a.keys = rng_keys(seed);
+    a.stream = stream ? s.as<uint32_t>() : nullptr; a.out = o.as<B200rtScatter>();
     scatter_kernel<<<(unsigned)((n + 127) / 128), 128>>>(a);
     CU(cudaGetLastError());
     CU(cudaMemcpy(out, o.p, n * sizeof(B200rtScatter), cudaMemcpyDeviceToHost));
     return B200RT_OK;
 }
 
-int b200rt_camera_rays(const B200rtCamera* cam, const float* xy, size_t n, uint64_t seed, B200rtRay* out, int device) {
+int b200rt_camera_rays(const B200rtCamera* cam, const float* xy, size_t n, uint64_t seed, const uint32_t* stream, B200rtRay* out,
+                       uint32_t* draws, int device) {
     if (!cam || (n && (!xy || !out))) return fail(B200RT_EINVAL, "NULL argument");
     int rc = resolve_device(device, &device); if (rc) return rc;
     DeviceGuard guard(device);
     if (n == 0) return B200RT_OK;
-    DevBuf x, o;
+    DevBuf x, o, s, k;
     if ((rc = x.alloc(n * 8)) || (rc = o.alloc(n * sizeof(B200rtRay)))) return rc;
+    if ((stream && (rc = s.alloc(n * 12))) || (draws && (rc = k.alloc(n * 4)))) return rc;
     CU(cudaMemcpy(x.p, xy, n * 8, cudaMemcpyHostToDevice));
-    camera_rays_kernel<<<(unsigned)((n + 255) / 256), 256>>>(make_camera(*cam), x.as<float>(), n, rng_keys(seed), o.as<B200rtRay>());
+    if (stream) CU(cudaMemcpy(s.p, stream, n * 12, cudaMemcpyHostToDevice));
+    camera_rays_kernel<<<(unsigned)((n + 255) / 256), 256>>>(make_camera(*cam), x.as<float>(), n, rng_keys(seed),
+                                                             stream ? s.as<uint32_t>() : nullptr, o.as<B200rtRay>(),
+                                                             draws ? k.as<uint32_t>() : nullptr);
     CU(cudaGetLastError());
     CU(cudaMemcpy(out, o.p, n * sizeof(B200rtRay), cudaMemcpyDeviceToHost));
+    if (draws) CU(cudaMemcpy(draws, k.p, n * 4, cudaMemcpyDeviceToHost));
     return B200RT_OK;
 }
 

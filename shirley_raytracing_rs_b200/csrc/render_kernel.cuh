@@ -225,7 +225,9 @@ __global__ void __launch_bounds__(BLK, 1) path_trace_kernel_v2(const __grid_cons
             float3 radiance = f3(0.f, 0.f, 0.f);         // what the path adds to its pixel when it ends in this iteration
             if (fin && !hit) {                           // render.rs:44-45: emitted + attenuation * background
                 const float3 bg = background(a.scene, ray.d);
-                radiance = has_emitters ? ps_ld3(PS_EMIT) + ps_ld3(PS_ATTEN) * bg : ps_ld3(PS_ATTEN) * bg;
+                // (`emitted` is loaded before `attenuation` in both updates, the order of the code before the explicit fmaf)
+                if (has_emitters) { const float3 e = ps_ld3(PS_EMIT); radiance = fma_f3(ps_ld3(PS_ATTEN), bg, e); }
+                else radiance = mul_rn3(ps_ld3(PS_ATTEN), bg);
                 done = true;
             }
             if (hit) {
@@ -238,13 +240,16 @@ __global__ void __launch_bounds__(BLK, 1) path_trace_kernel_v2(const __grid_cons
             if (hit) {
                 float3 albedo = sp_.tex.need_perlin ? marble(sp_.tex.perlin_scale, h.p, turb) : sp_.tex.rgb;
                 ShadeOut so = shade_finish(ray, h, sp_.m, albedo, rng);
-                if (so.has_emission) ps_st3(PS_EMIT, ps_ld3(PS_EMIT) + ps_ld3(PS_ATTEN) * so.emission);     // only scenes with emitters get here
+                if (so.has_emission) {                   // only scenes with emitters get here
+                    const float3 e = ps_ld3(PS_EMIT);
+                    ps_st3(PS_EMIT, fma_f3(ps_ld3(PS_ATTEN), so.emission, e));
+                }
                 done = !so.scattered;
                 if (!done) {
                     if (--depth == 0) { done = true; ++nexh; }
                     else {
                         ray.o = so.o; ray.d = so.d; setup = true;
-                        if (so.has_mul) ps_st3(PS_ATTEN, ps_ld3(PS_ATTEN) * so.mul);
+                        if (so.has_mul) ps_st3(PS_ATTEN, mul_rn3(ps_ld3(PS_ATTEN), so.mul));
                     }
                 }
             }

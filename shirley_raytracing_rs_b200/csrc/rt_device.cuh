@@ -145,6 +145,10 @@ __device__ __forceinline__ float3 operator*(float3 a, float s) { return f3(a.x *
 __device__ __forceinline__ float3 operator-(float3 a) { return f3(-a.x, -a.y, -a.z); }
 __device__ __forceinline__ float dot(float3 a, float3 b) { return a.x * b.x + a.y * b.y + a.z * b.z; }
 __device__ __forceinline__ float3 fma3(float s, float3 a, float3 b) { return f3(fmaf(s, a.x, b.x), fmaf(s, a.y, b.y), fmaf(s, a.z, b.z)); }
+// a * b + c and a * b per component, each rounded once: ray_color's accumulators (render kernel), which the render replay
+// restates on the host (tests/test_render_replay.py)
+__device__ __forceinline__ float3 fma_f3(float3 a, float3 b, float3 c) { return f3(fmaf(a.x, b.x, c.x), fmaf(a.y, b.y, c.y), fmaf(a.z, b.z, c.z)); }
+__device__ __forceinline__ float3 mul_rn3(float3 a, float3 b) { return f3(__fmul_rn(a.x, b.x), __fmul_rn(a.y, b.y), __fmul_rn(a.z, b.z)); }
 __device__ __forceinline__ float comp(float3 a, int i) { return i == 0 ? a.x : (i == 1 ? a.y : a.z); }
 
 // ------------------------------------------------------------------------------------------
@@ -812,9 +816,13 @@ __device__ __forceinline__ ShadeOut shade_finish(const RayF& r, const HitRec& h,
         return out;
     }
     if (m.kind == B200RT_MAT_FAIRY_LIGHT) {                             // lighting.rs:59-66 then :43-57
-        float scale = -dot(h.n, r.d) * rsqrtf(fmaf(r.d.z, r.d.z, fmaf(r.d.y, r.d.y, __fmul_rn(r.d.x, r.d.x))));
-        out.emission = a * scale; out.has_emission = true;
-        a = unit(a);
+        // every rounding spelled out: these are the ones nvcc chose for the render kernel from plain operators, but it
+        // contracted the scatter hook's copy differently, and the hook must give the render kernel's bits
+        const float nd = fmaf(h.n.z, r.d.z, fmaf(h.n.y, r.d.y, __fmul_rn(h.n.x, r.d.x)));
+        const float scale = __fmul_rn(-nd, rsqrtf(fmaf(r.d.z, r.d.z, fmaf(r.d.y, r.d.y, __fmul_rn(r.d.x, r.d.x)))));
+        out.emission = f3(__fmul_rn(a.x, scale), __fmul_rn(a.y, scale), __fmul_rn(a.z, scale)); out.has_emission = true;
+        const float inv = rsqrtf(fmaf(a.z, a.z, fmaf(a.y, a.y, __fmul_rn(a.x, a.x))));
+        a = f3(__fmul_rn(a.x, inv), __fmul_rn(a.y, inv), __fmul_rn(a.z, inv));
     }
     float3 dir = h.n + unit(rs);                                        // lambertian.rs:23, math.rs:62-68
     if (fabsf(dir.x) < 1e-8f && fabsf(dir.y) < 1e-8f && fabsf(dir.z) < 1e-8f) dir = h.n;   // vec3.rs:130

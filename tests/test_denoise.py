@@ -165,7 +165,6 @@ def expected_features(rt, scene, cam, seed, k, sample_offset=0):
     desc = scene.desc.contents
     nz = np.zeros((H * W, 4), np.float32)
     al = np.zeros((H * W, 3), np.float32)
-    all_hit = np.ones(H * W, bool)
     kinds = np.array([desc.materials[i].kind for i in range(desc.n_prims)])
     texs = np.array([desc.materials[i].texture for i in range(desc.n_prims)])
     pix = np.arange(H * W)
@@ -176,7 +175,6 @@ def expected_features(rt, scene, cam, seed, k, sample_offset=0):
         rays = rt.camera_rays(cam, xy)
         ids, hits, _ = rt.closest_hit(scene, rays, 0.001, float("inf"))
         hit = ids >= 0
-        all_hit &= hit
         d = rays[:, 3:6]
         depth = hits["t"] * np.sqrt((d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1]) + d[:, 2] * d[:, 2])
         f = np.zeros((H * W, 4), np.float32)
@@ -192,8 +190,11 @@ def expected_features(rt, scene, cam, seed, k, sample_offset=0):
             sel = texd & (tex == t)
             h = hits[sel]
             a[sel] = rt.texture_value(scene, t, np.column_stack([h["u"], h["v"], h["p"]]))
+        if (~hit).any():                                       # a miss record returns the device's background(d)
+            sky = np.zeros((~hit).sum(), rt.HIT_DTYPE)
+            sky["id"] = -1
+            a[~hit] = rt.scatter(scene, rays[~hit], sky)["emitted"]
         nz, al = nz + f, al + a
-    al[~all_hit] = np.nan                                     # some ray met the sky: background(d) uses rsqrt, checked apart
     kf = np.float32(k)
     return (nz / kf).reshape(H, W, 4), (al / kf).reshape(H, W, 3)
 
@@ -206,12 +207,10 @@ def test_features_are_the_first_hits_of_the_primary_rays(rt, weekend, lensless, 
     _, _, feat, _ = rt.render_denoised(weekend, cam, 8, feature_samples=k, seed=seed)
     nz, al = expected_features(rt, weekend, cam, seed, k)
     assert np.array_equal(feat[0], nz)
-    geo = np.isfinite(al).all(-1)
-    assert geo.mean() > 0.5 and (~geo).any()
-    assert np.array_equal(feat[1][geo][:, :3], al[geo]) and np.all(feat[1][..., 3] == 0)
-    # pixels with a missed feature ray: the sky colour of background(d) (rsqrt on the device)
+    assert np.array_equal(feat[1][..., :3], al) and np.all(feat[1][..., 3] == 0)
+    # pixels with feature rays on geometry and pixels whose feature rays all met the sky are both there
     sky = feat[0, ..., 3] == 0
-    assert sky.any() and np.all((feat[1][sky][:, :3] > 0.4) & (feat[1][sky][:, :3] <= 1.0))
+    assert (~sky).mean() > 0.5 and sky.any() and np.all((feat[1][sky][:, :3] > 0.4) & (feat[1][sky][:, :3] <= 1.0))
 
 
 @pytest.mark.gpu
